@@ -11,6 +11,7 @@ convergence.  correspondences = sum over pairs of N_src * outer iterations execu
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this engine
     python bench.py --impl reference [...]                          # the CPU arm (oracle port)
+    python bench.py --dump-outputs DIR [...]                        # + the last timed step's results as DIR/*.npy
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for every field.
 """
@@ -46,7 +47,15 @@ def parse():
                     help="config4 (default): the batch of independent pairs the metric is quoted on; config5: ONE 3-D pair of "
                          "16.7 M points per side, source sharded over the ranks with an NCCL all-reduce per outer iteration")
     ap.add_argument("--config5-points", type=int, default=0, help="points per side of the config5 pair (0 = 16 777 216)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last timed step's results (T, n_outer, converged_at of "
+                         "every pair) as DIR/<name>.npy, so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the GPU path computed; it does not apply to --impl reference")
+    return args
 
 
 def workload_config(args):
@@ -237,6 +246,8 @@ def run_b200(args):
     e1.record()
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res, world, gather=True)
     launches = eng.launch_count - l0
     ms = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
     tot = torch.tensor([float(corr_per_step), float(my_pairs), float(launches)], dtype=torch.float64, device=dev)
@@ -431,6 +442,8 @@ def run_config5(args):
     e1.record()
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res, world, gather=False)   # every rank solves the same pair
     launches = eng.launch_count - l0
     ms = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
     if world > 1:
@@ -539,6 +552,35 @@ def claim_stdout():
 def emit(line):
     _REAL_STDOUT.write(json.dumps(line) + "\n")
     _REAL_STDOUT.flush()
+
+
+DUMP_MAX_BYTES = 60 * 10**6     # keeps a dump, .npy headers included, under 64 MB
+
+
+def dump_outputs(out_dir, res, world, gather):
+    """Writes what register() returned in the last timed step: T (P, 4, 4) f64, n_outer (P,) and converged_at (P,)
+    as f64, pairs in job order (gather: the ranks' shares are concatenated on rank 0).  Beyond DUMP_MAX_BYTES a fixed
+    seeded sample of pairs is written, with the sampled pair indices in pair_index.npy."""
+    import numpy as np
+    import torch.distributed as dist
+    part = {"T": res.T.cpu().numpy(), "n_outer": res.n_outer.cpu().numpy().astype(np.float64),
+            "converged_at": res.converged_at.cpu().numpy().astype(np.float64)}
+    parts = [part]
+    if gather and world > 1:
+        parts = [None] * world
+        dist.all_gather_object(parts, part)
+    if int(os.environ.get("RANK", "0")) != 0:
+        return
+    out = {k: np.concatenate([p[k] for p in parts]) for k in part}
+    n_pairs = len(out["T"])
+    per_pair = sum(v[0].nbytes for v in out.values())
+    if n_pairs * per_pair > DUMP_MAX_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(n_pairs, DUMP_MAX_BYTES // (per_pair + 8), replace=False))
+        out = {k: v[keep] for k, v in out.items()}
+        out["pair_index"] = keep.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 def main():

@@ -1,9 +1,9 @@
-"""SURVEY 8b / appendix C: the reference's two demos run UNMODIFIED under scripts/run_demo.py (module resolution
-controlled by the launcher, headless pygame, scripted QUIT).  The demo sources exist only in the dev container
-(/root/reference does not travel to the GPU box) and the dev container has no GPU, so what is checked HERE is the
-launcher's mechanics with the demos' real bytes: a stand-in gicp module backed by the CPU oracle takes the engine's
-place (same 7-tuple).  The engine itself in the demos' process layout - first gicp() call inside a forked worker,
-lists of tuples in, pickled numpy out - is checked on the GPU by tests/test_gpu_fork.py."""
+"""SURVEY 8b / appendix C: demo scripts run UNMODIFIED under scripts/run_demo.py (module resolution controlled by the
+launcher, headless pygame, scripted QUIT).  The scripts are tests/demos/, stand-ins with the structure of the
+reference's two demos (the reference itself is not part of this repository).  What is checked here is the launcher's
+mechanics: a stand-in gicp module backed by the CPU oracle takes the engine's place (same 7-tuple).  The engine itself
+in the demos' process layout - first gicp() call inside a forked worker, lists of tuples in, pickled numpy out - is
+checked on the GPU by tests/test_gpu_fork.py."""
 import os
 import sys
 import types
@@ -12,8 +12,7 @@ import pytest
 
 from conftest import ROOT
 
-REF = "/root/reference/python-implementation"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference demos are only present in the dev container")
+REF = os.path.join(ROOT, "tests", "demos")
 
 
 def _oracle_backed_module():
@@ -43,7 +42,7 @@ def _launcher():
 
 
 def test_static_viewer_runs_unmodified(capsys):
-    """visualization.py:169-198: builds its pair, calls gicp(source, target) once, steps through the result."""
+    """The static viewer builds its pair, calls gicp(source, target) once, steps through the result."""
     before = open(os.path.join(REF, "visualization.py"), "rb").read()
     r = _launcher().run(os.path.join(REF, "visualization.py"), frames=25, headless=True,
                         gicp_module=_oracle_backed_module(), seed=0, tick=0.0)
@@ -54,8 +53,8 @@ def test_static_viewer_runs_unmodified(capsys):
 
 
 def test_robot_demo_runs_unmodified_with_forked_worker():
-    """robot-visualization.py:168-352: UI loop at 10 fps, GICP worker in a forked process fed through queues, each
-    call padded to 0.5 s (lines 163-165).  40 frames of 0.1 s leave time for several results."""
+    """The robot demo: UI loop at 10 fps, GICP worker in a forked process fed through queues, each call padded to
+    0.5 s.  40 frames of 0.1 s leave time for several results."""
     r = _launcher().run(os.path.join(REF, "robot-visualization.py"), frames=40, headless=True,
                         gicp_module=_oracle_backed_module(), seed=1, tick=0.1)
     assert r["exit"] == 0
@@ -65,8 +64,8 @@ def test_robot_demo_runs_unmodified_with_forked_worker():
 
 def test_launcher_registers_the_repo_module_by_default():
     """Without a stand-in the launcher binds the demos to THIS repo's drop-in (which needs a GPU at call time):
-    in the GPU-less dev container the static viewer must fail loudly inside gicp(), not fall back to the reference's
-    gicp.py lying beside the script."""
+    without a GPU the static viewer must fail loudly inside gicp(), not fall back to a gicp.py lying beside the
+    script."""
     import torch
     if torch.cuda.is_available():
         pytest.skip("GPU present")
