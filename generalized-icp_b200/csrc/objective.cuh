@@ -63,6 +63,28 @@ template <typename Real> struct ObjArgs {
     const int* n_list;
 };
 
+// ---- the two fp32 bounds of the exact search (host-callable: tests/host_harness/bounds_host.cu checks them) ----
+// Filter: for a candidate c, a query p' (fp64) and its fp32 rounding f, d2_32 = |c - f|^2 in fp32 satisfies
+// |d2_32 - d2| <= 2 sqrt(3) d u P + 6 u d2  (u = 2^-24, P >= max|f_i|).  c1 is the coefficient of d in that bound.
+__host__ __device__ __forceinline__ float filter_c1(float Pf) { return 5e-7f * Pf * 1.0001f; }
+// Threshold on d2_32 that every candidate with exact d2 <= bd passes: b = bd rounded up to fp32, rs ~ 1/sqrt(max(b,
+// 1e-30)).  The device passes rsqrtf (2 ulp of error, covered by the 1.0001 in c1).
+__host__ __device__ __forceinline__ float filter_thr_of(float b, float rs, float c1) {
+    const float sq = fmaxf(b, 1e-30f) * rs;           // sqrt(max(b, 1e-30)) >= sqrt(b): never under the bound
+    return fmaf(b, 1.000002f, c1 * sq) + 1e-30f;
+}
+// Slack of a tracked, matched point: how far it may move before its match can change.  d1 = its match distance
+// rounded up, m2 = second smallest fp32 squared distance seen (INFINITY: none), rad32 = lower bound of the distance
+// to every target point outside the examined cell box.  Never more than half the gap to the true runner-up.
+__host__ __device__ __forceinline__ float match_slack(float d1, float m2, float rad32, float c1, float Pf) {
+    // runner-up: at least lb2 away (fp32 error bound of the filter), or outside the examined ball
+    const float lb2 = m2 * 0.999999f - c1 * sqrtf(m2);
+    const float d2e = fminf(sqrtf(fmaxf(lb2, 0.f)) * 0.999999f, rad32);
+    float sl = fmaxf(0.f, 0.5f * (d2e - d1) * 0.99999f - 1e-6f * (Pf + d1));
+    if (!(m2 < INFINITY)) sl = fmaxf(0.f, 0.5f * (fminf(rad32, 1e30f) - d1) * 0.99999f - 1e-6f * (Pf + d1));
+    return sl;
+}
+
 template <typename Real>
 __device__ __forceinline__ int obj_pair_of_block(const ObjArgs<Real>& a) {
     if (!a.active_list) return (int)blockIdx.y;
@@ -186,15 +208,12 @@ __device__ __forceinline__ void correspond_block(const ObjArgs<Real>& a, const i
         }
         const float fx = (float)pp[0], fy = (float)pp[1], fz = (float)pp[2];
         const float Pf = fmaxf(fabsf(fx), fmaxf(fabsf(fy), fabsf(fz))) * 1.0000002f;
-        // conservative fp32 filter threshold: |d2_32 - d2| <= 2 sqrt(3) d u P + 6 u d2  (u = 2^-24)
-        const float c1 = 5e-7f * Pf * 1.0001f;
+        const float c1 = filter_c1(Pf);
         auto filter_thr = [&](double bd) {
             const float b = __double2float_ru(bd);
             // sqrt(b) through the reciprocal-square-root unit (2 instructions instead of the IEEE sequence; it is
-            // re-evaluated on every improvement of the best distance): 2 ulp of error, covered by the 1.0001 in c1
-            const float bb = fmaxf(b, 1e-30f);
-            const float sq = bb * rsqrtf(bb);               // sqrt(max(b, 1e-30)) >= sqrt(b): never under the bound
-            return fmaf(b, 1.000002f, c1 * sq) + 1e-30f;
+            // re-evaluated on every improvement of the best distance)
+            return filter_thr_of(b, rsqrtf(fmaxf(b, 1e-30f)), c1);
         };
         float thr32 = filter_thr(bestd);
         float m1 = INFINITY, m2 = INFINITY;   // two smallest fp32 squared distances seen (slack of the next iterations)
@@ -361,14 +380,7 @@ __device__ __forceinline__ void correspond_block(const ObjArgs<Real>& a, const i
         a.match[s] = bestpos;
         if (a.slack) {
             float sl = 0.f;
-            if (tracked && matched) {
-                // runner-up: at least lb2 away (fp32 error bound of the filter), or outside the examined ball
-                const float d1 = __double2float_ru(dist);
-                const float lb2 = m2 * 0.999999f - c1 * sqrtf(m2);
-                const float d2e = fminf(sqrtf(fmaxf(lb2, 0.f)) * 0.999999f, rad32);
-                sl = fmaxf(0.f, 0.5f * (d2e - d1) * 0.99999f - 1e-6f * (Pf + d1));
-                if (!(m2 < INFINITY)) sl = fmaxf(0.f, 0.5f * (fminf(rad32, 1e30f) - d1) * 0.99999f - 1e-6f * (Pf + d1));
-            }
+            if (tracked && matched) sl = match_slack(__double2float_ru(dist), m2, rad32, c1, Pf);
             a.slack[s] = sl;
         }
         if (a.out_idx || a.out_dist) {

@@ -131,9 +131,9 @@ def test_reduced_form_reproduces_loss_and_grad_loss(name, golden):
 
 @pytest.fixture(scope="module")
 def solve_host(tmp_path_factory):
-    """tests/host_harness/*.cu: the 2-D inner solver and the damped linear solve of csrc/solve.cuh and the covariance
-    tail of csrc/knn_cov.cuh (__host__ __device__ functions) compiled for the host with nvcc - product source, run here
-    as the thing under test."""
+    """tests/host_harness/*.cu: the 2-D inner solver and the damped linear solve of csrc/solve.cuh, the covariance
+    tail of csrc/knn_cov.cuh and the fp32 search bounds of csrc/objective.cuh (__host__ __device__ functions) compiled
+    for the host with nvcc - product source, run here as the thing under test."""
     import ctypes
     import shutil
     import subprocess
@@ -143,17 +143,23 @@ def solve_host(tmp_path_factory):
     tmp = tmp_path_factory.mktemp("host_harness")
     here = os.path.join(os.path.dirname(os.path.abspath(__file__)), "host_harness")
     libs = []
-    for name in ("solve_host", "cov_host"):
+    for name in ("solve_host", "cov_host", "bounds_host"):
         out = str(tmp / (name + ".so"))
         subprocess.run([nvcc, "-gencode", "arch=compute_100a,code=sm_100a", "-std=c++17", "-O2", "-Xcompiler", "-fPIC",
                         "-shared", "-o", out, os.path.join(here, name + ".cu")], check=True)
         libs.append(ctypes.CDLL(out))
-    lib, cov = libs
+    lib, cov, bounds = libs
     dp = ctypes.POINTER(ctypes.c_double)
+    ip = ctypes.POINTER(ctypes.c_int)
     lib.gicp_test_solve2d.argtypes = [dp, ctypes.c_int, dp]
     lib.gicp_test_spd_solve6.argtypes = [dp, dp]
     cov.gicp_test_regularised_cov.argtypes = [ctypes.c_int, dp, ctypes.c_double, ctypes.c_double, dp]
     lib.regularised_cov = cov.gicp_test_regularised_cov
+    bounds.gicp_test_filter.argtypes = [ctypes.c_longlong, dp, dp, dp, ctypes.c_int, ip]
+    bounds.gicp_test_filter.restype = ctypes.c_longlong
+    bounds.gicp_test_slack.argtypes = [ctypes.c_longlong, dp, dp, dp, ctypes.c_int, dp, dp]
+    bounds.gicp_test_slack.restype = ctypes.c_longlong
+    lib.bounds = bounds
     return lib
 
 
@@ -256,3 +262,90 @@ def test_covariance_tail_host(solve_host):
             assert np.abs(got(S, dim) - want(S, dim)).max() <= max(tol, 1e-9), (dim, case, ev)
         bad = np.full((dim, dim), np.nan)
         assert np.array_equal(got(bad, dim), np.eye(dim))
+
+
+def _queries(rng, n):
+    """Transformed source points p' (fp64) with |p'| spread log-uniformly over 1 .. 1e5 m (one axis dominant or all
+    comparable); half of them are fp32 values (an fp64 query rounded to fp32)."""
+    u = rng.normal(size=(n, 3)) * 10.0 ** rng.uniform(-3, 0, size=(n, 3))
+    p = u / np.abs(u).max(1, keepdims=True) * 10.0 ** rng.uniform(0, 5, size=(n, 1))
+    f = rng.random(n) < 0.5
+    p[f] = p[f].astype(np.float32)
+    return p
+
+
+def _unit(rng, n):
+    v = rng.normal(size=(n, 3))
+    return v / np.linalg.norm(v, axis=1, keepdims=True)
+
+
+def _key(c, p):
+    d = c - p
+    return (d[:, 0] * d[:, 0] + d[:, 1] * d[:, 1]) + d[:, 2] * d[:, 2]
+
+
+def test_search_filter_threshold_is_sound(solve_host):
+    """K3a's fp32 candidate filter (csrc/objective.cuh filter_c1 / filter_thr_of, compiled for the host): a target
+    point whose exact squared distance - the fp64 key or the __float128 value - is <= the best distance so far always
+    passes, for 1.2e6 cases: fp32 targets, |p'| from 1 to 1e5 m (where the filter's Pf term dominates), distances from
+    1e-6 m to d_max, best distance equal to the candidate's own key or one ulp below it, and the device's approximate
+    rsqrtf modelled by +-2 ulp around the exact reciprocal square root."""
+    import ctypes
+    dp = ctypes.POINTER(ctypes.c_double)
+    rng = np.random.default_rng(2024)
+    n = 1_200_000
+    p = _queries(rng, n)
+    d_max = 10.0 ** rng.uniform(0, np.log10(150.0), n)
+    d = 10.0 ** rng.uniform(-6, 0, n) * d_max
+    c = (p + d[:, None] * _unit(rng, n)).astype(np.float32).astype(np.float64)
+    # a third: the worst alignment the bound covers.  p' sits just past the midpoint between two fp32 values on
+    # every axis (fp32(p') is half an ulp away), the candidate is m whole ulps beyond the other neighbour, so its fp32
+    # distance exceeds the exact one by the full 2 sqrt(3) u P d
+    w = np.arange(n) % 3 == 0
+    x = p[w].astype(np.float32)
+    ulp = np.nextafter(np.abs(x), np.float32(np.inf)) - np.abs(x)
+    sgn = np.where(x < 0, -1.0, 1.0)
+    p[w] = x + sgn * ulp * (0.5 + 1e-3)                # rounds to the neighbour one ulp out
+    m = np.minimum(10.0 ** rng.uniform(0, 6, w.sum()), 0.5 * d_max[w] / ulp.max(1))
+    m = np.maximum(np.floor(m), 0.0)[:, None]
+    c[w] = (x - sgn * ulp * m).astype(np.float32)
+    bd = _key(c, p)
+    below = rng.random(n) < 0.3
+    bd[below] = np.nextafter(bd[below], 0.0)          # must pass only if the exact value is still <= bd
+    p, c, bd = (np.ascontiguousarray(a) for a in (p, c, bd))
+    out = np.zeros(n, dtype=np.int32)
+    bad = solve_host.bounds.gicp_test_filter(n, p.ctypes.data_as(dp), c.ctypes.data_as(dp), bd.ctypes.data_as(dp), 2,
+                                             out.ctypes.data_as(ctypes.POINTER(ctypes.c_int)))
+    assert bad == 0, (p[out == 1][:5], c[out == 1][:5], bd[out == 1][:5])
+
+
+@pytest.mark.parametrize("f32", [1, 0])
+def test_search_slack_is_sound(f32, solve_host):
+    """The slack K3a stores for a tracked match (csrc/objective.cuh match_slack: how far the point may move before
+    its match could change, which lets the next iterations skip its search) never exceeds half the exact gap between
+    the nearest and the runner-up target point (__float128 distances), for 6e5 near-ties per storage type: runner-up
+    1 + 1e-7 ... 1 + 1e-3 times as far as the nearest, |p'| from 1 to 1e5 m, distances from 1e-6 m to d_max.  Also
+    checks that the bound is not vacuous: well separated pairs get a positive slack."""
+    import ctypes
+    dp = ctypes.POINTER(ctypes.c_double)
+    rng = np.random.default_rng(7 + f32)
+    n = 600_000
+    p = _queries(rng, n)
+    d_max = 10.0 ** rng.uniform(0, np.log10(150.0), n)
+    d = 10.0 ** rng.uniform(-6, 0, n) * d_max
+    gap = 10.0 ** rng.uniform(-7, -3, n)
+    a = p + d[:, None] * _unit(rng, n)
+    b = p + (d * (1.0 + gap))[:, None] * _unit(rng, n)
+    if f32:
+        a, b = a.astype(np.float32).astype(np.float64), b.astype(np.float32).astype(np.float64)
+    swap = rng.random(n) < 0.5
+    a[swap], b[swap] = b[swap].copy(), a[swap].copy()
+    p, a, b = (np.ascontiguousarray(x) for x in (p, a, b))
+    sl, hg = np.zeros(n), np.zeros(n)
+    bad = solve_host.bounds.gicp_test_slack(n, p.ctypes.data_as(dp), a.ctypes.data_as(dp), b.ctypes.data_as(dp), f32,
+                                            sl.ctypes.data_as(dp), hg.ctypes.data_as(dp))
+    worst = np.argmax(sl - hg)
+    assert bad == 0, (p[worst], a[worst], b[worst], sl[worst], hg[worst])
+    # not vacuous: where the gap is wide compared with the fp32 resolution at |p'|, the slack is a fair share of it
+    wide = hg > 1e-4 * (np.abs(p).max(1) + d)
+    assert wide.sum() > 1000 and (sl[wide] > 0.2 * hg[wide]).mean() > 0.9
