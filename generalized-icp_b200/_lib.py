@@ -12,7 +12,7 @@ SYMBOLS = [
     "gicpCreate", "gicpDestroy", "gicpGetLastError", "gicpVersion", "gicpDefaultParams", "gicpSetParams",
     "gicpSetTarget", "gicpSetSource", "gicpSetPair", "gicpPromoteTargetToSource", "gicpRegister", "gicpKnn", "gicpCovariances", "gicpCorrespond",
     "gicpNormalEquations", "gicpSourceCovariancesAt", "gicpCommGetUniqueId", "gicpCommInit", "gicpCommDestroy",
-    "gicpLaunchCount", "gicpProfile", "gicpProfileRead", "gicpRayCast",
+    "gicpLaunchCount", "gicpProfile", "gicpProfileRead", "gicpRayCast", "gicpVoxelDownsample",
 ]
 
 
@@ -68,6 +68,7 @@ def load():
     lib.gicpLaunchCount.argtypes = [vp]
     lib.gicpLaunchCount.restype = i64
     lib.gicpRayCast.argtypes = [C.c_int, vp, i32, i32, vp, i32, vp, i32, C.c_double, vp, vp, vp, vp]
+    lib.gicpVoxelDownsample.argtypes = [vp, vp, C.POINTER(i64), i32, C.c_double, i32, vp, C.POINTER(i64), vp, vp, vp]
     lib.gicpProfile.argtypes = [vp, C.c_int]
     lib.gicpProfileRead.argtypes = [vp, dp, C.POINTER(i64)]
     _lib = lib

@@ -34,13 +34,30 @@ def _engine(dim, storage, tag="main"):
     return eng
 
 
+def _downsample(eng, cloud, voxel_size, min_points):
+    pts, _ = eng.voxel_downsample(np.ascontiguousarray(cloud), voxel_size=voxel_size, min_points=min_points)
+    return pts.cpu().numpy().astype(np.float64)
+
+
+def voxel_downsample(cloud, voxel_size, min_points=1):
+    """PCL-style voxel-grid filter of one (N, 2) or (N, 3) cloud on the GPU: the centroid of every voxel of edge
+    ``voxel_size`` holding >= ``min_points`` finite points, in the order of each voxel's lowest row (semantics in
+    include/gicp_b200.h).  float64 numpy in and out."""
+    cloud = np.asarray(cloud, dtype=np.float64)
+    if cloud.ndim != 2 or cloud.shape[1] not in (2, 3):
+        raise ValueError(f"expected an (N, 2) or (N, 3) cloud, got {cloud.shape}")
+    return _downsample(_engine(int(cloud.shape[1]), "f64"), cloud, voxel_size, min_points)
+
+
 def gicp_extended(source_points, target_points, max_iterations=100, tolerance=1e-6,
                   max_distance_correspondence=150, max_distance_nearest_neighbors=50, k=6,
                   lambda_tangent=100.0, lambda_normal=10.0, storage="f64", full_history=True, covariance_model=0,
-                  **engine_params):
+                  voxel_size=None, **engine_params):
     """The registration with everything the engine knows (SURVEY.md discrepancy 3: the reference
     computes ``min_loss`` and drops it; here the loss history, inlier counts and the fitness-like
-    final loss are returned as well).  Returns a dict."""
+    final loss are returned as well).  Returns a dict.  With ``voxel_size`` both clouds are first
+    voxel-grid downsampled on the GPU (in ``storage``); the dict then holds them as ``source_points`` /
+    ``target_points`` (float64) and every per-point output refers to them."""
     import torch
 
     src = np.asarray(source_points)
@@ -51,6 +68,9 @@ def gicp_extended(source_points, target_points, max_iterations=100, tolerance=1e
     if dim not in (2, 3) or tgt.shape[1] != dim:
         raise ValueError(f"expected (N, 2) or (N, 3) clouds of equal dimension, got {src.shape} and {tgt.shape}")
     eng = _engine(dim, storage)
+    if voxel_size is not None:
+        src = _downsample(eng, src[:, :dim], voxel_size, 1)
+        tgt = _downsample(eng, tgt[:, :dim], voxel_size, 1)
     eng.set_params(k=k, max_iterations=int(max_iterations), tolerance=float(tolerance),
                    max_distance_correspondence=float(max_distance_correspondence),
                    max_distance_nearest_neighbors=float(max_distance_nearest_neighbors),
@@ -63,6 +83,8 @@ def gicp_extended(source_points, target_points, max_iterations=100, tolerance=1e
     out = dict(T=T_hist[-1].copy(), all_T=[T_hist[i].copy() for i in range(n_T)], n_outer=n_outer,
                converged_at=conv, loss_hist=r["loss_hist"].copy(), inliers=r["inliers"].copy(), dim=dim,
                tgt_cov=r["tgt_cov"], src_cov0=r["src_cov0"])
+    if voxel_size is not None:
+        out["source_points"], out["target_points"] = src, tgt
     if full_history:
         covs = eng.source_covariances_at(T_hist[:n_outer].reshape(n_outer, 1, dim + 1, dim + 1)).cpu().numpy()
         out["all_src_cov"] = [covs[i] for i in range(n_outer)]

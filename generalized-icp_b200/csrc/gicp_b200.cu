@@ -2,6 +2,7 @@
 // Orchestrates the kernels K1 (grid.cuh), K2 (knn_cov.cuh), K3 (objective.cuh), K4 (solve.cuh).
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
+#include <cub/device/device_segmented_sort.cuh>
 #include <dlfcn.h>
 #include <nvtx3/nvToolsExt.h>   // header-only NVTX: ranges per stage for nsys / ncu timelines
 
@@ -9,6 +10,7 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
+#include <cmath>
 #include <cstring>
 #include <string>
 #include <vector>
@@ -20,6 +22,7 @@
 #include "raycast.cuh"
 #include "solve.cuh"
 #include "fused.cuh"
+#include "voxel.cuh"
 
 using namespace gicp;
 
@@ -140,12 +143,31 @@ struct SetupScratch {
     }
 };
 
+// scratch of gicpVoxelDownsample: its own, so a downsample between gicpSetPair and gicpRegister leaves both sides alone
+struct VoxelScratch {
+    DevBuf offsets, part, vb, keys, keys_alt, vals, vals_alt, rid, orow, out_off, big, cub_tmp;
+    double* h_vb = nullptr;     // pinned: per-cloud voxel bounds
+    int* h_out_off = nullptr;   // pinned: output offsets
+    int h_cap = 0;              // clouds the pinned buffers hold
+    std::vector<int> off32;
+    void release() {
+        for (DevBuf* b : {&offsets, &part, &vb, &keys, &keys_alt, &vals, &vals_alt, &rid, &orow, &out_off, &big, &cub_tmp})
+            b->release();
+        if (h_vb) cudaFreeHost(h_vb);
+        if (h_out_off) cudaFreeHost(h_out_off);
+        h_vb = nullptr;
+        h_out_off = nullptr;
+        h_cap = 0;
+    }
+};
+
 struct gicpContext {
     int device = 0, dim = 2, storage = GICP_STORAGE_F64;
     gicpParams prm;
     CloudSet src, tgt;
     // [0]: every call on the caller's stream; [1]: the source side of gicpSetPair while it runs on the internal stream
     SetupScratch scr[2];
+    VoxelScratch vox;
     DevBuf state, partial, partial2, red, T_dev, n_active, prev_match, slack, active_list;
     static constexpr int NPOLL = 8;
     int* h_poll = nullptr;  // pinned [NPOLL]: progress polls in flight
@@ -898,7 +920,178 @@ int do_rotcov(gicpContext* h, const double* h_T, int n_T, double* d_out, cudaStr
     return 0;
 }
 
-#define DISPATCH(h, FN, ...)                                                                  \
+int bit_length(unsigned long long v) {
+    int b = 0;
+    while (b < 64 && (v >> b)) ++b;
+    return b;
+}
+
+// gicpVoxelDownsample (voxel.cuh).  Two host synchronisations: the per-cloud voxel bounds (they size the key fields and
+// are checked against the limits) and the output offsets.
+template <int D, typename Real>
+int do_voxel(gicpContext* h, const void* d_points, const int64_t* h_off, int nc, double leaf, int min_points,
+             void* d_out, int64_t* h_out_off, int* d_voxel_of, int* d_counts, cudaStream_t st) {
+    VoxelScratch& v = h->vox;
+    if (nc <= 0 || nc > 65535) return fail("n_clouds must be in [1, 65535] (got %d)", nc);
+    if (h_off[0] != 0) return fail("offsets[0] must be 0");
+    int max_n = 0;
+    for (int i = 1; i <= nc; ++i) {
+        if (h_off[i] < h_off[i - 1]) return fail("offsets must be non-decreasing");
+        if (h_off[i] >= (1LL << 31) - 1024) return fail("more than 2^31 points in one batch");
+        max_n = std::max<int>(max_n, (int)(h_off[i] - h_off[i - 1]));
+    }
+    const int n = (int)h_off[nc];
+    if (n == 0) {
+        for (int i = 0; i <= nc; ++i) h_out_off[i] = 0;
+        return 0;
+    }
+    if (!d_points || !d_out) return fail("null point or output array");
+    const Real* pts = static_cast<const Real*>(d_points);
+    v.off32.assign(h_off, h_off + nc + 1);
+    if (nc + 1 > v.h_cap) {
+        if (v.h_vb) cudaFreeHost(v.h_vb);
+        if (v.h_out_off) cudaFreeHost(v.h_out_off);
+        v.h_vb = nullptr;
+        v.h_out_off = nullptr;
+        v.h_cap = 0;
+        CU(cudaMallocHost(&v.h_vb, (size_t)(nc + 1) * 6 * sizeof(double)));
+        CU(cudaMallocHost(&v.h_out_off, (size_t)(nc + 1) * sizeof(int)));
+        v.h_cap = nc + 1;
+    }
+    const int chunks = (max_n + VOX_THREADS * VOX_ITEMS - 1) / (VOX_THREADS * VOX_ITEMS);
+    CU(v.offsets.ensure((size_t)(nc + 1) * sizeof(int)));
+    CU(v.part.ensure((size_t)nc * std::max(chunks, 1) * 6 * sizeof(double)));
+    CU(v.vb.ensure((size_t)nc * 6 * sizeof(double)));
+    const int* offs = v.offsets.as<int>();
+    CU(cudaMemcpyAsync(v.offsets.p, v.off32.data(), (size_t)(nc + 1) * sizeof(int), cudaMemcpyHostToDevice, st));
+    // 1. voxel bounds of every cloud's finite rows -> host
+    voxel_bounds_partial_kernel<D, Real><<<dim3(chunks, nc), VOX_THREADS, 0, st>>>(pts, offs, v.part.as<double>(), chunks);
+    voxel_bounds_kernel<<<(nc + 3) / 4, 128, 0, st>>>(v.part.as<double>(), chunks, nc, leaf, v.vb.as<double>());
+    CU(cudaMemcpyAsync(v.h_vb, v.vb.p, (size_t)nc * 6 * sizeof(double), cudaMemcpyDeviceToHost, st));
+    h->launches += 2;
+    CU(cudaStreamSynchronize(st));
+    CU(cudaGetLastError());
+    // every voxel index an int64, every cloud-relative index below the per-axis limit; then the narrowest key fields
+    const double two63 = 9223372036854775808.0;
+    const int limit_bits = D == 3 ? 21 : 31;
+    long long max_ext[3] = {0, 0, 0};
+    for (int c = 0; c < nc; ++c) {
+        const double* b = v.h_vb + (size_t)c * 6;
+        if (!(b[0] <= b[3])) continue;   // no finite row
+        for (int a = 0; a < D; ++a) {
+            for (double q : {b[a], b[3 + a]})
+                if (!(q >= -two63 && q < two63))
+                    return fail("voxel_size %g: cloud %d has voxel index %g along axis %c, outside int64; use a larger "
+                                "voxel_size", leaf, c, q, "xyz"[a]);
+            const __int128 ext = (__int128)(long long)b[3 + a] - (__int128)(long long)b[a];
+            if (ext >= ((__int128)1 << limit_bits))
+                return fail("voxel_size %g: cloud %d spans %.0f voxels along axis %c, the limit is 2^%d per axis in %d-D; "
+                            "use a larger voxel_size", leaf, c, (double)ext + 1.0, "xyz"[a], limit_bits, D);
+            max_ext[a] = std::max<long long>(max_ext[a], (long long)ext);
+        }
+    }
+    VoxKeyGeom geo;
+    int coord_bits = 0;
+    for (int a = 2; a >= 0; --a) {
+        geo.shift[a] = coord_bits;
+        if (a < D) coord_bits += bit_length((unsigned long long)max_ext[a]);
+    }
+    // the cloud index above the coordinates, sized so that the all-ones sentinel exceeds every finite row's key; when
+    // it does not fit 64 bits the clouds are sorted as segments on the coordinates alone
+    const int end_bit = coord_bits + bit_length((unsigned long long)nc);
+    const bool segmented = end_bit > 64;
+    geo.cloud_shift = segmented ? -1 : coord_bits;
+
+    // 2. keys, stable sort
+    CU(v.keys.ensure((size_t)n * 8));
+    CU(v.keys_alt.ensure((size_t)n * 8));
+    CU(v.vals.ensure((size_t)(n + 1) * 4));
+    CU(v.vals_alt.ensure((size_t)(n + 1) * 4));
+    CU(v.rid.ensure((size_t)(n + 1) * 4));
+    CU(v.orow.ensure((size_t)(n + 1) * 4));
+    CU(v.out_off.ensure((size_t)(nc + 1) * 4));
+    CU(v.big.ensure((size_t)(n / (VOX_SEQ_MAX + 1) + 2) * 4));
+    voxel_key_kernel<D, Real><<<dim3((max_n + 255) / 256, nc), 256, 0, st>>>(pts, offs, v.vb.as<double>(), leaf, geo,
+                                                                             v.keys.as<unsigned long long>(), v.vals.as<int>());
+    h->launches += 1;
+    const unsigned long long* K;
+    const int* R;
+    int* free_vals;
+    unsigned long long* free_keys;
+    if (!segmented) {
+        cub::DoubleBuffer<unsigned long long> dk(v.keys.as<unsigned long long>(), v.keys_alt.as<unsigned long long>());
+        cub::DoubleBuffer<int> dv(v.vals.as<int>(), v.vals_alt.as<int>());
+        size_t tmp = 0;
+        CU(cub::DeviceRadixSort::SortPairs(nullptr, tmp, dk, dv, n, 0, end_bit, st));
+        CU(v.cub_tmp.ensure(tmp));
+        CU(cub::DeviceRadixSort::SortPairs(v.cub_tmp.p, tmp, dk, dv, n, 0, end_bit, st));
+        h->launches += (end_bit + 7) / 8 + 2;
+        K = dk.Current();
+        R = dv.Current();
+        free_keys = dk.Alternate();
+        free_vals = dv.Alternate();
+    } else {
+        size_t tmp = 0;
+        CU(cub::DeviceSegmentedSort::StableSortPairs(nullptr, tmp, v.keys.as<unsigned long long>(),
+                                                     v.keys_alt.as<unsigned long long>(), v.vals.as<int>(),
+                                                     v.vals_alt.as<int>(), n, nc, offs, offs + 1, st));
+        CU(v.cub_tmp.ensure(tmp));
+        CU(cub::DeviceSegmentedSort::StableSortPairs(v.cub_tmp.p, tmp, v.keys.as<unsigned long long>(),
+                                                     v.keys_alt.as<unsigned long long>(), v.vals.as<int>(),
+                                                     v.vals_alt.as<int>(), n, nc, offs, offs + 1, st));
+        h->launches += 3;
+        K = v.keys_alt.as<unsigned long long>();
+        R = v.vals_alt.as<int>();
+        free_keys = v.keys.as<unsigned long long>();
+        free_vals = v.vals.as<int>();
+    }
+    // 3. voxels as runs of the sorted keys: run id by a scan of the head flags, begin / end per run
+    int* rid = v.rid.as<int>();
+    int* run_begin = reinterpret_cast<int*>(free_keys);   // the sort's other key buffer holds 2n ints
+    int* run_end = run_begin + n;
+    voxel_head_kernel<<<(n + 1 + 255) / 256, 256, 0, st>>>(K, n, rid);
+    h->launches += 1;
+    if (segmented) {
+        voxel_segment_heads_kernel<<<(nc + 255) / 256, 256, 0, st>>>(K, offs, nc, rid);
+        h->launches += 1;
+    }
+    auto excl_scan = [&](int* a, int len) -> int {
+        size_t tmp = 0;
+        CU(cub::DeviceScan::ExclusiveSum(nullptr, tmp, a, a, len, st));
+        CU(v.cub_tmp.ensure(tmp));
+        CU(cub::DeviceScan::ExclusiveSum(v.cub_tmp.p, tmp, a, a, len, st));
+        h->launches += 2;
+        return 0;
+    };
+    if (excl_scan(rid, n + 1)) return 1;
+    const int nb = (n + 255) / 256;
+    voxel_runs_kernel<<<nb, 256, 0, st>>>(K, rid, n, run_begin, run_end);
+    // 4. keep flag at each kept voxel's lowest row; its scan in input order is the output row
+    int* orow = v.orow.as<int>();
+    CU(cudaMemsetAsync(orow, 0, (size_t)(n + 1) * 4, st));
+    voxel_keep_kernel<<<nb, 256, 0, st>>>(rid, n, run_begin, run_end, R, min_points, orow);
+    h->launches += 2;
+    if (excl_scan(orow, n + 1)) return 1;
+    voxel_out_offsets_kernel<<<(nc + 1 + 255) / 256, 256, 0, st>>>(orow, offs, nc, v.out_off.as<int>());
+    h->launches += 1;
+    // 5. centroids, counts and the row -> output map
+    if (d_voxel_of) CU(cudaMemsetAsync(d_voxel_of, 0xFF, (size_t)n * 4, st));
+    int* big_count = free_vals + n;    // the sort's other value buffer: n + 1 ints, the list lives in v.big
+    CU(cudaMemsetAsync(big_count, 0, sizeof(int), st));
+    VoxOutArgs oa{rid, n, run_begin, run_end, R, orow, v.out_off.as<int>(), nc, min_points, d_voxel_of, d_counts,
+                  v.big.as<int>(), big_count};
+    voxel_centroid_kernel<D, Real><<<nb, 256, 0, st>>>(oa, pts, static_cast<Real*>(d_out));
+    const int big_blocks = std::max(1, std::min(n / (VOX_SEQ_MAX + 1), 148 * 8));
+    voxel_centroid_block_kernel<D, Real><<<big_blocks, VOX_THREADS, 0, st>>>(oa, pts, static_cast<Real*>(d_out));
+    h->launches += 2;
+    CU(cudaMemcpyAsync(v.h_out_off, v.out_off.p, (size_t)(nc + 1) * sizeof(int), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    CU(cudaGetLastError());
+    for (int i = 0; i <= nc; ++i) h_out_off[i] = v.h_out_off[i];
+    return 0;
+}
+
+#define DISPATCH(h, FN, ...)                                                               \
     ((h)->dim == 2 ? ((h)->storage == GICP_STORAGE_F32 ? FN<2, float>(__VA_ARGS__) : FN<2, double>(__VA_ARGS__)) \
                    : ((h)->storage == GICP_STORAGE_F32 ? FN<3, float>(__VA_ARGS__) : FN<3, double>(__VA_ARGS__)))
 
@@ -914,7 +1107,7 @@ int check(gicpHandle h) {
 extern "C" {
 
 const char* gicpGetLastError(void) { return g_last_error.c_str(); }
-int gicpVersion(void) { return 100; }
+int gicpVersion(void) { return 101; }
 
 int gicpDefaultParams(gicpParams* p) {
     if (!p) return fail("null params");
@@ -962,6 +1155,7 @@ int gicpDestroy(gicpHandle h) {
     h->src.release();
     h->tgt.release();
     for (SetupScratch& sc : h->scr) sc.release();
+    h->vox.release();
     DevBuf* bufs[] = {&h->state, &h->partial, &h->partial2, &h->red, &h->T_dev, &h->n_active, &h->prev_match, &h->slack,
                       &h->active_list};
     for (DevBuf* b : bufs) b->release();
@@ -1080,6 +1274,18 @@ int gicpSourceCovariancesAt(gicpHandle h, const double* h_T, int32_t n_T, double
     if (check(h)) return 1;
     if (!h_T || !d_out) return fail("h_T and d_out are required");
     return DISPATCH(h, do_rotcov, h, h_T, n_T, d_out, (cudaStream_t)stream);
+}
+
+int gicpVoxelDownsample(gicpHandle h, const void* d_points, const int64_t* h_offsets, int32_t n_clouds,
+                        double voxel_size, int32_t min_points, void* d_out, int64_t* h_out_offsets,
+                        int32_t* d_voxel_of, int32_t* d_counts, void* stream) {
+    if (check(h)) return 1;
+    if (!h_offsets || !h_out_offsets) return fail("null offsets");
+    if (d_points && d_out == d_points) return fail("d_out must not alias d_points");
+    if (!(std::isfinite(voxel_size) && voxel_size > 0)) return fail("voxel_size must be finite and > 0 (got %g)", voxel_size);
+    if (min_points < 1) return fail("min_points must be >= 1 (got %d)", min_points);
+    return DISPATCH(h, do_voxel, h, d_points, h_offsets, n_clouds, voxel_size, min_points, d_out, h_out_offsets,
+                    d_voxel_of, d_counts, (cudaStream_t)stream);
 }
 
 int gicpCommGetUniqueId(char id[128]) {

@@ -306,6 +306,31 @@ class GicpEngine:
         torch.cuda.synchronize(self.device)
         return T_out, n_out, c_out
 
+    # ---- voxel-grid downsampling ----
+    def voxel_downsample(self, points, offsets=None, *, voxel_size, min_points=1, with_index=False):
+        """Voxel-grid filter of a batch on the device (gicpVoxelDownsample; semantics in include/gicp_b200.h): every
+        voxel of edge ``voxel_size`` with >= ``min_points`` finite points becomes their centroid, in the order of each
+        voxel's lowest input row.  Returns ``(pts, out_offsets)`` - pts (M, d) on the engine's device in its dtype, a
+        tensor of its own (safe to pass to set_source / set_target: no later call writes it), out_offsets (P+1,)
+        int64 numpy, usable as the offsets of set_*.  With ``with_index`` also ``(voxel_of (N,) i32, counts (M,) i32)``:
+        each input row's cloud-local output row (-1 when dropped) and the points behind each output row.  Leaves the
+        engine's source and target as they are."""
+        points, off = self._prep(points, offsets)
+        n, nc = points.shape[0], len(off) - 1
+        out = torch.empty((n, self.dim), dtype=self.dtype, device=self.device)
+        out_off = np.zeros(nc + 1, dtype=np.int64)
+        vox = torch.empty((n,), dtype=torch.int32, device=self.device) if with_index else None
+        cnt = torch.empty((n,), dtype=torch.int32, device=self.device) if with_index else None
+        i64p = C.POINTER(C.c_int64)
+        _lib.check(self.lib.gicpVoxelDownsample(self._h, _ptr(points), off.ctypes.data_as(i64p), nc, float(voxel_size),
+                                                int(min_points), _ptr(out), out_off.ctypes.data_as(i64p), _ptr(vox),
+                                                _ptr(cnt), self._stream()))
+        m = int(out_off[-1])
+        pts = out[:m].clone() if m < n else out
+        if with_index:
+            return pts, out_off, vox, cnt[:m].clone()
+        return pts, out_off
+
     # ---- stage entry points ----
     def knn(self, which, with_dist=True):
         n = self._n[which][0]

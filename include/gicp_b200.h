@@ -136,6 +136,28 @@ int gicpNormalEquations(gicpHandle h, const double* h_T, double* h_out, void* st
  * d_out (n_T, n_src_total, dim, dim) f64 in input order.  all_source_cov_matrices, gicp.py:121. */
 int gicpSourceCovariancesAt(gicpHandle h, const double* h_T, int32_t n_T, double* d_out, void* stream);
 
+/* ---- voxel-grid downsampling (PCL's VoxelGrid filter), for clouds too dense to register raw ----------------
+ * A batch in the layout of gicpSet*, in the handle's dim and storage.  For every cloud, with leaf L:
+ *  - the voxel of a point is v_a = floor((double)p_a / L) per axis (IEEE float64 division, lattice anchored at the
+ *    origin, so clouds share one lattice); rows with a non-finite coordinate are dropped;
+ *  - a voxel with fewer than min_points points is dropped (1 keeps every voxel);
+ *  - the output point of a voxel is the centroid of its points: a float64 sum in a fixed order, started from the
+ *    first point, divided by the count, rounded to the storage type; bit-identical from run to run;
+ *  - a cloud's output rows are ordered by each voxel's lowest input row, so with every point alone in its voxel the
+ *    output is the finite input rows, bit for bit;
+ *  - per cloud, floor(hi / L) - floor(lo / L) over its finite rows must be < 2^21 along each axis in 3-D (< 2^31 in
+ *    2-D) and every voxel index must fit int64; otherwise the call fails naming the cloud and the axis.
+ *  d_out         (n_total, dim) caller-allocated, same dtype as d_points, not d_points itself; the first
+ *                h_out_offsets[n_clouds] rows are written
+ *  h_out_offsets (n_clouds+1) host: row range of each cloud's output - directly usable as the offsets of gicpSet*
+ *  d_voxel_of    optional (n_total) i32: cloud-local output row of each input point, -1 when dropped
+ *  d_counts      optional (n_total) i32: points per output row
+ * Synchronises the stream.  Uses scratch of its own: the handle's source / target (grids, covariances, loop state)
+ * are untouched, so it may be called between gicpSetPair and gicpRegister.                                      */
+int gicpVoxelDownsample(gicpHandle h, const void* d_points, const int64_t* h_offsets, int32_t n_clouds,
+                        double voxel_size, int32_t min_points, void* d_out, int64_t* h_out_offsets,
+                        int32_t* d_voxel_of, int32_t* d_counts, void* stream);
+
 /* ---- multi-GPU: one large pair with the source sharded over ranks (BASELINE config 5) ----
  * Every rank holds both full clouds; rank r computes covariances for its slice of the
  * target (all-gathered once) and runs the per-iteration reduction on its slice of the
