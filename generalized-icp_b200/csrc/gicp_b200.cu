@@ -13,6 +13,7 @@
 #include <cmath>
 #include <cstring>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/gicp_b200.h"
@@ -23,6 +24,7 @@
 #include "solve.cuh"
 #include "fused.cuh"
 #include "voxel.cuh"
+#include "plan.h"
 
 using namespace gicp;
 
@@ -69,32 +71,24 @@ struct DevBuf {
 
 struct Grid {
     DevBuf meta, cell_start, spts, inv_perm, bbox, lut;
-    long long budget = 0;
-    long long total_cells = 0;
-    double h_target = 0;
     bool built = false;
     void release() { meta.release(); cell_start.release(); spts.release(); inv_perm.release(); bbox.release(); lut.release(); }
 };
 
 struct CloudSet {
     const void* raw = nullptr;
-    std::vector<int64_t> offsets;
+    SetupPlan plan;           // sizes, grids and kernels of this cloud set, fixed by its set-up
     std::vector<int> off32;   // staging copy of the offsets for the asynchronous upload (must outlive the call)
-    int n_clouds = 0;
-    int64_t n_total = 0;
-    int max_n = 0;
-    DevBuf d_offsets;   // int32 [n_clouds+1]
-    int inline_n = -1;  // >= 0: one small cloud of that many points, its offsets travel as a kernel argument (no upload)
+    DevBuf d_offsets;   // int32 [n_clouds+1]; not uploaded when plan.inline_n >= 0
     Grid knn;           // grid of the covariance neighbourhoods (cell ~ knn radius / 4)
     Grid nn;            // grid of the correspondence search (cell ~ d_max / 2): the target is searched in it,
                         // the source is only ORDERED by it (compact warps in K3).  Built only when the k-NN
-                        // grid's cells do not suit the search (`shared` = false)
+                        // grid's cells do not suit the search (plan.shared = false)
     DevBuf cov_knn;     // covariances in knn-grid order (written by K2)
     DevBuf cov_nn;      // the same covariances in nn-grid order (read by K3); unused when shared
-    bool shared = true; // one grid serves both stages: half the grid builds, no covariance re-ordering
     bool ready = false;
-    Grid& nng() { return shared ? knn : nn; }
-    DevBuf& covnn() { return shared ? cov_knn : cov_nn; }
+    Grid& nng() { return plan.shared ? knn : nn; }
+    DevBuf& covnn() { return plan.shared ? cov_knn : cov_nn; }
     void release() { d_offsets.release(); knn.release(); nn.release(); cov_knn.release(); cov_nn.release(); }
 };
 
@@ -223,33 +217,16 @@ struct ProfScope {
 
 template <int D, typename Real>
 int build_grid(gicpContext* h, CloudSet& cs, Grid& g, double h_target, cudaStream_t st, SetupScratch& sc) {
-    const int nc = cs.n_clouds;
-    const int64_t n = cs.n_total;
-    long long budget = h->prm.max_cells_per_cloud;
-    if (budget <= 0) {
-        budget = 4096;  // Morton padding can cost up to 8x the occupied box
-        while (budget < 8LL * cs.max_n) budget <<= 1;
-    }
-    // Large batches: the table (memset + scan + 4 B per cell, per cloud set) is sized for one cell per point instead
-    // of eight - grid_meta_kernel then enlarges the cell edge by the few per cent that save the Morton bits (a 40 m
-    // cloud at 1.25 m cells needs 33-36 cells per axis = 2^18 padded; at 1.3-1.4 m it fits 2^15)
-    if (h->prm.max_cells_per_cloud <= 0) {
-        long long cap_total = 1LL << 30;   // default: no shrinking (measured: the larger cells cost K2 more than K1 gains)
-        if (getenv("GICP_CELL_TABLE_LOG2") && atoi(getenv("GICP_CELL_TABLE_LOG2")) > 0) cap_total = 1LL << atoi(getenv("GICP_CELL_TABLE_LOG2"));
-        while (budget * (long long)nc > cap_total && budget > 4096 && budget / 2 >= cs.max_n) budget >>= 1;
-    }
-    if (budget * (long long)nc > (1LL << 30)) {
-        budget = (1LL << 30) / nc;
-        if (budget < 64) return fail("too many clouds for the cell table (%d)", nc);
-    }
-    g.budget = budget;
-    g.total_cells = budget * nc;
-    g.h_target = h_target;
-    const int chunks = std::max(1, (cs.max_n + BBOX_THREADS * BBOX_ITEMS - 1) / (BBOX_THREADS * BBOX_ITEMS));
+    const SetupPlan& p = cs.plan;
+    const int nc = p.n_clouds;
+    const int64_t n = p.n_total;
+    const long long budget = p.budget;
+    const long long total_cells = budget * nc;
+    const int chunks = std::max(1, (p.max_n + BBOX_THREADS * BBOX_ITEMS - 1) / (BBOX_THREADS * BBOX_ITEMS));
     CU(sc.bbox_part.ensure((size_t)nc * chunks * 6 * sizeof(double)));
     CU(g.meta.ensure((size_t)nc * sizeof(CloudMeta)));
     CU(g.bbox.ensure((size_t)nc * 6 * sizeof(double)));
-    CU(g.cell_start.ensure((size_t)(g.total_cells + 1) * sizeof(int)));
+    CU(g.cell_start.ensure((size_t)(total_cells + 1) * sizeof(int)));
     CU(g.spts.ensure((size_t)std::max<int64_t>(n, 1) * sizeof(PRec<Real>)));
     CU(g.inv_perm.ensure((size_t)std::max<int64_t>(n, 1) * sizeof(int)));
     CU(sc.keys.ensure((size_t)std::max<int64_t>(n, 1) * 4));
@@ -260,14 +237,12 @@ int build_grid(gicpContext* h, CloudSet& cs, Grid& g, double h_target, cudaStrea
     const int* offs = cs.d_offsets.as<int>();
     ProfScope prof(h, GICP_STAGE_GRID, st);
 
-    // small clouds (the reference's own workloads): the whole build of a cloud in one block, one launch
-    if (cs.max_n <= SMALL_GRID_MAX && budget <= (1LL << 20) && n > 0 &&
-        !(getenv("GICP_SMALL_GRID") && atoi(getenv("GICP_SMALL_GRID")) == 0)) {
+    if (p.single_block) {   // the whole build of a cloud in one block, one launch
         CU(g.lut.ensure((size_t)nc * 3 * GICP_LUT_N * sizeof(int)));
         small_grid_kernel<D, Real><<<nc, SMALL_GRID_THREADS, 0, st>>>(pts, offs, h_target, budget, g.meta.as<CloudMeta>(),
                                                                       g.bbox.as<double>(), g.lut.as<int>(),
                                                                       g.cell_start.as<int>(), g.spts.as<PRec<Real>>(),
-                                                                      g.inv_perm.as<int>(), 1, cs.inline_n);
+                                                                      g.inv_perm.as<int>(), 1, p.inline_n);
         h->launches += 1;
         CU(cudaGetLastError());
         g.built = true;
@@ -280,10 +255,10 @@ int build_grid(gicpContext* h, CloudSet& cs, Grid& g, double h_target, cudaStrea
     CU(g.lut.ensure((size_t)nc * 3 * GICP_LUT_N * sizeof(int)));
     morton_lut_kernel<<<dim3(3 * GICP_LUT_N / 256, nc), 256, 0, st>>>(g.meta.as<CloudMeta>(), g.lut.as<int>());
     // the cell histogram is built in the table itself and scanned in place (no second 4-byte-per-cell buffer)
-    CU(cudaMemsetAsync(g.cell_start.p, 0, (size_t)(g.total_cells + 1) * sizeof(int), st));
+    CU(cudaMemsetAsync(g.cell_start.p, 0, (size_t)(total_cells + 1) * sizeof(int), st));
     h->launches += 3;
     if (n > 0) {
-        const int bx = (cs.max_n + 255) / 256;
+        const int bx = (p.max_n + 255) / 256;
         cell_key_kernel<D, Real><<<dim3(bx, nc), 256, 0, st>>>(pts, g.meta.as<CloudMeta>(), sc.keys.as<unsigned>(),
                                                                sc.vals.as<int>(), g.cell_start.as<int>());
         h->launches += 1;
@@ -291,15 +266,15 @@ int build_grid(gicpContext* h, CloudSet& cs, Grid& g, double h_target, cudaStrea
     {   // cell_start = exclusive scan of the histogram
         size_t tmp = 0;
         CU(cub::DeviceScan::ExclusiveSum(nullptr, tmp, g.cell_start.as<int>(), g.cell_start.as<int>(),
-                                         (int)(g.total_cells + 1), st));
+                                         (int)(total_cells + 1), st));
         CU(sc.cub_tmp.ensure(tmp));
         CU(cub::DeviceScan::ExclusiveSum(sc.cub_tmp.p, tmp, g.cell_start.as<int>(), g.cell_start.as<int>(),
-                                         (int)(g.total_cells + 1), st));
+                                         (int)(total_cells + 1), st));
         h->launches += 2;
     }
     if (n > 0) {
         int bits = 1;
-        while ((1LL << bits) < g.total_cells) ++bits;
+        while ((1LL << bits) < total_cells) ++bits;
         cub::DoubleBuffer<unsigned> dk(sc.keys.as<unsigned>(), sc.keys_alt.as<unsigned>());
         cub::DoubleBuffer<int> dv(sc.vals.as<int>(), sc.vals_alt.as<int>());
         size_t tmp = 0;
@@ -307,7 +282,7 @@ int build_grid(gicpContext* h, CloudSet& cs, Grid& g, double h_target, cudaStrea
         CU(sc.cub_tmp.ensure(tmp));
         CU(cub::DeviceRadixSort::SortPairs(sc.cub_tmp.p, tmp, dk, dv, (int)n, 0, bits, st));
         h->launches += (bits + 7) / 8 + 2;
-        const int bx = (cs.max_n + 255) / 256;
+        const int bx = (p.max_n + 255) / 256;
         gather_sorted_kernel<D, Real><<<dim3(bx, nc), 256, 0, st>>>(pts, g.meta.as<CloudMeta>(), dv.Current(),
                                                                     g.spts.as<PRec<Real>>(), g.inv_perm.as<int>());
         h->launches += 1;
@@ -383,9 +358,11 @@ __global__ void rotated_cov_kernel(const CloudMeta* __restrict__ meta, const PRe
         }
 }
 
+// K2 along `path` (pick_knn), over the slice [slice_b, slice_e) of a single cloud or, with slice_b < 0, every cloud
 template <int D, typename Real>
-int launch_knn(gicpContext* h, CloudSet& cs, int* d_idx, double* d_dist, cudaStream_t st, int slice_b, int slice_e,
-               SetupScratch& sc) {
+int launch_knn(gicpContext* h, CloudSet& cs, KnnPath path, int* d_idx, double* d_dist, cudaStream_t st, int slice_b,
+               int slice_e, SetupScratch& sc) {
+    const SetupPlan& p = cs.plan;
     KnnArgs<Real> a;
     a.meta = cs.knn.meta.as<CloudMeta>();
     a.cell_start = cs.knn.cell_start.as<int>();
@@ -401,22 +378,18 @@ int launch_knn(gicpContext* h, CloudSet& cs, int* d_idx, double* d_dist, cudaStr
     a.lam_n = h->prm.lambda_normal;
     a.slice_begin = slice_b;
     a.slice_end = slice_e;
-    if (cs.n_total == 0) return 0;
-    const int span = (slice_b >= 0) ? (slice_e - slice_b) : cs.max_n;
+    if (p.n_total == 0) return 0;
+    const int span = (slice_b >= 0) ? (slice_e - slice_b) : p.max_n;
     if (span <= 0) return 0;
     const int bx = (span + KNN_THREADS - 1) / KNN_THREADS;
-    dim3 grid(bx, cs.n_clouds);
+    dim3 grid(bx, p.n_clouds);
     // fast path's overflow hand-over: worst case every warp
-    const long long n_chunks = (long long)bx * KNN_WARPS * cs.n_clouds;
+    const long long n_chunks = (long long)bx * KNN_WARPS * p.n_clouds;
     CU(sc.ovf_count.ensure(sizeof(int)));
     CU(sc.ovf_list.ensure((size_t)n_chunks * sizeof(int2)));
     a.overflow_count = sc.ovf_count.as<int>();
     a.overflow_list = sc.ovf_list.as<int2>();
     a.overflow_cap = (int)std::min<long long>(n_chunks, INT_MAX);
-    // latency mode (a few small clouds): the general kernel alone - one launch, no overflow hand-over
-    const bool latency_mode = cs.max_n <= SMALL_GRID_MAX && cs.n_total <= 65536 &&
-                              !(getenv("GICP_SMALL_GRID") && atoi(getenv("GICP_SMALL_GRID")) == 0);
-    const bool fast = a.k + 8 <= knn_list_cap<Real>() && !latency_mode;
     const size_t smem_g = 128 + (size_t)KNN_WARPS * KNN_WARP_SMEM;
     const size_t smem_h = 128 + (size_t)KNN_WARPS * KNN_HIST_WARP_SMEM;
     ProfScope prof(h, GICP_STAGE_KNN_COV, st);
@@ -426,40 +399,26 @@ int launch_knn(gicpContext* h, CloudSet& cs, int* d_idx, double* d_dist, cudaStr
                                 (int)smem_g));                                                               \
         knn_general_kernel<D, Real, KC><<<GRID, KNN_THREADS, smem_g, st>>>(a, FROM_LIST);                    \
     } while (0)
-    if (latency_mode && cs.max_n <= KNN_BRUTE_MAX && slice_b < 0 &&
-        !(getenv("GICP_KNN_BRUTE") && atoi(getenv("GICP_KNN_BRUTE")) == 0)) {
+    if (path == KnnPath::Brute) {
         // tiny clouds: brute force from shared memory, one block per cloud, one launch
-        const size_t smem_b = (size_t)cs.max_n * sizeof(PRec<Real>);
-        if (a.k <= 6) knn_brute_kernel<D, Real, 6><<<cs.n_clouds, KNN_BRUTE_THREADS, smem_b, st>>>(a);
-        else if (a.k <= 20) knn_brute_kernel<D, Real, 20><<<cs.n_clouds, KNN_BRUTE_THREADS, smem_b, st>>>(a);
-        else knn_brute_kernel<D, Real, 32><<<cs.n_clouds, KNN_BRUTE_THREADS, smem_b, st>>>(a);
+        const size_t smem_b = (size_t)p.max_n * sizeof(PRec<Real>);
+        if (p.kc == 6) knn_brute_kernel<D, Real, 6><<<p.n_clouds, KNN_BRUTE_THREADS, smem_b, st>>>(a);
+        else if (p.kc == 20) knn_brute_kernel<D, Real, 20><<<p.n_clouds, KNN_BRUTE_THREADS, smem_b, st>>>(a);
+        else knn_brute_kernel<D, Real, 32><<<p.n_clouds, KNN_BRUTE_THREADS, smem_b, st>>>(a);
         h->launches += 1;
-        CU(cudaGetLastError());
-        return 0;
-    }
-    if (fast) {
+    } else if (path == KnnPath::HistGeneral) {
         CU(cudaMemsetAsync(sc.ovf_count.p, 0, sizeof(int), st));
         CU(cudaFuncSetAttribute(knn_hist_kernel<D, Real>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_h));
         CU(cudaFuncSetAttribute(knn_hist_kernel<D, Real>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-        const size_t smem_l = (size_t)KNN_WARPS * KNN_LANE_WARP_SMEM;
-        // two equally fast variants (measured): warp-cooperative with TMA-staged cell blocks (default) and
-        // per-lane cell walks from L1 (GICP_KNN_LANE=1)
-        const bool per_lane = getenv("GICP_KNN_LANE") && atoi(getenv("GICP_KNN_LANE")) != 0;
-        if (per_lane) {
-            CU(cudaFuncSetAttribute(knn_lane_kernel<D, Real>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_l));
-            CU(cudaFuncSetAttribute(knn_lane_kernel<D, Real>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-            knn_lane_kernel<D, Real><<<grid, KNN_THREADS, smem_l, st>>>(a);
-        } else {
-            knn_hist_kernel<D, Real><<<grid, KNN_THREADS, smem_h, st>>>(a);
-        }
+        knn_hist_kernel<D, Real><<<grid, KNN_THREADS, smem_h, st>>>(a);
         const dim3 lgrid(296, 1);
-        if (a.k <= 6) KNN_LAUNCH(6, lgrid, 1);
-        else if (a.k <= 20) KNN_LAUNCH(20, lgrid, 1);
+        if (p.kc == 6) KNN_LAUNCH(6, lgrid, 1);
+        else if (p.kc == 20) KNN_LAUNCH(20, lgrid, 1);
         else KNN_LAUNCH(32, lgrid, 1);
         h->launches += 2;
     } else {
-        if (a.k <= 6) KNN_LAUNCH(6, grid, 0);
-        else if (a.k <= 20) KNN_LAUNCH(20, grid, 0);
+        if (p.kc == 6) KNN_LAUNCH(6, grid, 0);
+        else if (p.kc == 20) KNN_LAUNCH(20, grid, 0);
         else KNN_LAUNCH(32, grid, 0);
         h->launches += 1;
     }
@@ -473,110 +432,49 @@ inline size_t obj_smem(int ppt) {
     return 128 + (size_t)(OBJ_THREADS / 32) * OBJ_STAGE_BYTES + (size_t)OBJ_THREADS * ppt * sizeof(int);
 }
 
-// cell edges; never smaller than (search radius)/8 so that a lane's ball spans <= 17 cells per axis
-double auto_knn_cell(const gicpContext* h) {
-    const double r = h->prm.max_distance_nearest_neighbors;
-    if (getenv("GICP_KNN_CELL") && atof(getenv("GICP_KNN_CELL")) > 0) return std::max(atof(getenv("GICP_KNN_CELL")), r / 8.0);   // A/B timing
-    if (h->prm.knn_cell > 0) return std::max(h->prm.knn_cell, r / 8.0);
-    return 0.25 * r;   // measured optimum of the cooperative fast path on the bench workload (r = 5 m -> 1.25 m cells)
-}
-double auto_nn_cell(const gicpContext* h) {
-    const double r = h->prm.max_distance_correspondence;
-    if (getenv("GICP_NN_CELL") && atof(getenv("GICP_NN_CELL")) > 0) return std::max(atof(getenv("GICP_NN_CELL")), r / 8.0);   // A/B timing
-    if (h->prm.nn_cell > 0) return std::max(h->prm.nn_cell, r / 8.0);
-    return 0.5 * r;
-}
-
-// true when set_cloud takes the latency path for these clouds (small_grid_kernel + one k-NN launch): that path
-// touches only the side's own buffers, none of the handle's shared scratch (same conditions as build_grid / launch_knn)
-bool latency_path(const gicpContext* h, const int64_t* off, int n_clouds) {
-    if (getenv("GICP_SMALL_GRID") && atoi(getenv("GICP_SMALL_GRID")) == 0) return false;
-    if (n_clouds <= 0 || off[0] != 0 || h->prm.max_cells_per_cloud > (1LL << 20)) return false;
-    int64_t max_n = 0;
-    for (int i = 1; i <= n_clouds; ++i) {
-        if (off[i] < off[i - 1]) return false;
-        max_n = std::max<int64_t>(max_n, off[i] - off[i - 1]);
-    }
-    return max_n <= SMALL_GRID_MAX && off[n_clouds] > 0 && off[n_clouds] <= 65536;
-}
-
 template <int D, typename Real>
-int set_cloud(gicpContext* h, int which, const void* d_points, const int64_t* h_offsets, int n_clouds,
-              cudaStream_t st, int scratch_slot) {
+int set_cloud(gicpContext* h, const Switches& sw, int which, const void* d_points, const int64_t* h_offsets,
+              int n_clouds, cudaStream_t st, int scratch_slot) {
     SetupScratch& sc = h->scr[scratch_slot];
     CloudSet& cs = which == GICP_TARGET ? h->tgt : h->src;
     cs.ready = false;
     h->last_stream = st;
-    if (n_clouds <= 0) return fail("n_clouds must be positive");
-    if (n_clouds > 65535) return fail("at most 65535 clouds per batch (got %d)", n_clouds);
+    cs.plan = plan_setup(h->prm, sw, h_offsets, n_clouds, which, std::is_same<Real, float>::value,
+                         Ranks{h->comm != nullptr, h->n_ranks, h->rank});
+    const SetupPlan& p = cs.plan;
+    if (p.error) return fail("%s (%d clouds)", p.error, n_clouds);
+    if (p.n_total > 0 && !d_points) return fail("null point array");
     cs.raw = d_points;
-    cs.n_clouds = n_clouds;
-    cs.offsets.assign(h_offsets, h_offsets + n_clouds + 1);
-    cs.n_total = h_offsets[n_clouds] - h_offsets[0];
-    if (h_offsets[0] != 0) return fail("offsets[0] must be 0");
-    if (cs.n_total >= (1LL << 31) - 1024) return fail("more than 2^31 points in one batch");
-    cs.max_n = 0;
-    std::vector<int>& off32 = cs.off32;
-    off32.resize(n_clouds + 1);
-    for (int i = 0; i <= n_clouds; ++i) {
-        off32[i] = (int)h_offsets[i];
-        if (i && h_offsets[i] < h_offsets[i - 1]) return fail("offsets must be non-decreasing");
-        if (i) cs.max_n = std::max<int>(cs.max_n, (int)(h_offsets[i] - h_offsets[i - 1]));
-    }
-    if (cs.n_total > 0 && !d_points) return fail("null point array");
-    CU(cs.d_offsets.ensure(off32.size() * sizeof(int)));
-    // one small cloud (the reference's own calls): the single-block grid build takes the point count as an argument
-    // and the 12-byte upload with its copy-engine hop disappears from the latency path
-    cs.inline_n = (n_clouds == 1 && latency_path(h, h_offsets, 1)) ? (int)cs.n_total : -1;
+    CU(cs.d_offsets.ensure((size_t)(n_clouds + 1) * sizeof(int)));
     // no stream synchronisation here: a copy from pageable memory is staged by the driver before the call returns,
     // and the staging vector lives in the handle
-    if (cs.inline_n < 0)
-        CU(cudaMemcpyAsync(cs.d_offsets.p, off32.data(), off32.size() * sizeof(int), cudaMemcpyHostToDevice, st));
-
-    const double h_knn = auto_knn_cell(h);
-    const double h_nn = auto_nn_cell(h);
-    // one grid for both stages when the k-NN cell suits the correspondence search: not larger than twice the search's
-    // own choice (d_max / 2) and not smaller than d_max / 8 (a lane's ball then spans <= 17 cells per axis).  Measured
-    // on the bench workload (k-NN cell 1.25 m, search cell 1.0 m): K3a 14.97 vs 15.16 ms per 512 pairs - no loss.
-    cs.shared = h_knn <= 2.0 * h_nn && h_knn >= h->prm.max_distance_correspondence / 8.0 &&
-                !(getenv("GICP_SHARED_GRID") && atoi(getenv("GICP_SHARED_GRID")) == 0);
-    if (build_grid<D, Real>(h, cs, cs.knn, h_knn, st, sc)) return 1;
-    CU(cs.cov_knn.ensure((size_t)std::max<int64_t>(cs.n_total, 1) * ns_of(D) * sizeof(Real)));
-
-    // covariances; in sharded mode every rank computes an equal slice (k-NN grid order) of BOTH clouds
-    // and the slices are all-gathered: the correspondence stage walks the clouds in a different
-    // (1-NN grid) order, so every rank needs every covariance
-    int slice_b = -1, slice_e = -1;
-    const bool sharded = h->comm && n_clouds == 1;
-    int64_t per = 0;
-    if (sharded) {
-        const int64_t n = cs.n_total;
-        per = (n + h->n_ranks - 1) / h->n_ranks;   // equal-sized slices are required by ncclAllGather
-        slice_b = (int)std::min<int64_t>(n, per * h->rank);
-        slice_e = (int)std::min<int64_t>(n, per * (h->rank + 1));
-        CU(cs.cov_knn.ensure((size_t)per * h->n_ranks * ns_of(D) * sizeof(Real)));
+    if (p.inline_n < 0) {
+        cs.off32.assign(h_offsets, h_offsets + n_clouds + 1);
+        CU(cudaMemcpyAsync(cs.d_offsets.p, cs.off32.data(), cs.off32.size() * sizeof(int), cudaMemcpyHostToDevice, st));
     }
-    // covariance model (ICP family): GICP estimates both sides; point-to-point uses C_src = 0, C_tgt = I;
-    // point-to-plane uses C_src = 0 and the estimated target covariances
-    const int model = h->prm.covariance_model;
-    const bool constant = (model == GICP_POINT_TO_POINT) || (model == GICP_POINT_TO_PLANE && which == GICP_SOURCE);
-    if (constant) {
-        const Real diag = (model == GICP_POINT_TO_POINT && which == GICP_TARGET) ? Real(1) : Real(0);
-        const size_t n = (size_t)std::max<int64_t>(cs.n_total, 1);
+
+    if (build_grid<D, Real>(h, cs, cs.knn, p.knn_cell, st, sc)) return 1;
+    const size_t n_cov = (size_t)std::max<int64_t>(p.sharded ? p.slice_len * h->n_ranks : p.n_total, 1);
+    CU(cs.cov_knn.ensure(n_cov * ns_of(D) * sizeof(Real)));
+    if (p.cov != CovSource::Knn) {
+        const size_t n = (size_t)std::max<int64_t>(p.n_total, 1);
+        const Real diag = p.cov == CovSource::Identity ? Real(1) : Real(0);
         fill_cov_kernel<D, Real><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(cs.cov_knn.as<Real>(), n, diag);
         h->launches += 1;
-    } else if (launch_knn<D, Real>(h, cs, nullptr, nullptr, st, slice_b, slice_e, sc)) return 1;
-    if (sharded && !constant) {
-        const size_t bytes = (size_t)per * ns_of(D) * sizeof(Real);
-        char* basep = cs.cov_knn.as<char>();
-        int rc = g_nccl.AllGather(basep + bytes * h->rank, basep, bytes, NCCL_INT8, h->comm, st);
-        if (rc) return fail("ncclAllGather failed: %s", g_nccl.GetErrorString ? g_nccl.GetErrorString(rc) : "?");
+    } else {
+        if (launch_knn<D, Real>(h, cs, p.knn, nullptr, nullptr, st, p.slice_begin, p.slice_end, sc)) return 1;
+        if (p.sharded) {
+            const size_t bytes = (size_t)p.slice_len * ns_of(D) * sizeof(Real);
+            char* basep = cs.cov_knn.as<char>();
+            int rc = g_nccl.AllGather(basep + bytes * h->rank, basep, bytes, NCCL_INT8, h->comm, st);
+            if (rc) return fail("ncclAllGather failed: %s", g_nccl.GetErrorString ? g_nccl.GetErrorString(rc) : "?");
+        }
     }
-    if (!cs.shared) {   // second ordering for the correspondence stage + the covariances carried over to it
-        if (build_grid<D, Real>(h, cs, cs.nn, h_nn, st, sc)) return 1;
-        CU(cs.cov_nn.ensure((size_t)std::max<int64_t>(cs.n_total, 1) * ns_of(D) * sizeof(Real)));
-        if (cs.n_total > 0) {
-            const int bx = (cs.max_n + 255) / 256;
+    if (!p.shared) {   // second ordering for the correspondence stage + the covariances carried over to it
+        if (build_grid<D, Real>(h, cs, cs.nn, p.nn_cell, st, sc)) return 1;
+        CU(cs.cov_nn.ensure((size_t)std::max<int64_t>(p.n_total, 1) * ns_of(D) * sizeof(Real)));
+        if (p.n_total > 0) {
+            const int bx = (p.max_n + 255) / 256;
             regather_cov_kernel<D, Real><<<dim3(bx, n_clouds), 256, 0, st>>>(
                 cs.nn.meta.as<CloudMeta>(), cs.nn.spts.as<PRec<Real>>(), cs.knn.inv_perm.as<int>(), cs.cov_knn.as<Real>(),
                 cs.cov_nn.as<Real>());
@@ -593,19 +491,21 @@ int set_cloud(gicpContext* h, int which, const void* d_points, const int64_t* h_
 template <int D, typename Real>
 int zero_source_cov(gicpContext* h, cudaStream_t st) {
     CloudSet& cs = h->src;
-    const size_t n = (size_t)std::max<int64_t>(cs.n_total, 1);
+    const size_t n = (size_t)std::max<int64_t>(cs.plan.n_total, 1);
     fill_cov_kernel<D, Real><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(cs.cov_knn.as<Real>(), n, Real(0));
-    if (!cs.shared) fill_cov_kernel<D, Real><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(cs.cov_nn.as<Real>(), n, Real(0));
-    h->launches += cs.shared ? 1 : 2;
+    if (!cs.plan.shared) fill_cov_kernel<D, Real><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(cs.cov_nn.as<Real>(), n, Real(0));
+    h->launches += cs.plan.shared ? 1 : 2;
     CU(cudaGetLastError());
     return 0;
 }
 
 template <int D, typename Real>
-int objective_args(gicpContext* h, ObjArgs<Real>& a, int& blocks_per_pair, bool allow_slice) {
+int objective_args(gicpContext* h, const Switches& sw, bool sliced, bool has_T0, ObjArgs<Real>& a, LoopPlan& lp) {
     CloudSet &S = h->src, &T = h->tgt;
     if (!S.ready || !T.ready) return fail("set source and target first");
-    if (S.n_clouds != T.n_clouds) return fail("source has %d clouds, target %d", S.n_clouds, T.n_clouds);
+    const int np = S.plan.n_clouds;
+    if (np != T.plan.n_clouds) return fail("source has %d clouds, target %d", np, T.plan.n_clouds);
+    lp = plan_loop(sw, S.plan, sliced, Ranks{h->comm != nullptr, h->n_ranks, h->rank}, h->prof_on, has_T0);
     a.src_meta = S.nng().meta.as<CloudMeta>();
     a.src_spts = S.nng().spts.as<PRec<Real>>();
     a.src_cov = S.covnn().as<Real>();
@@ -617,59 +517,50 @@ int objective_args(gicpContext* h, ObjArgs<Real>& a, int& blocks_per_pair, bool 
     a.tgt_inv_perm = T.nng().inv_perm.as<int>();
     a.match = nullptr;
     a.use_prev = 0;
-    CU(h->state.ensure((size_t)S.n_clouds * sizeof(PairState)));
+    CU(h->state.ensure((size_t)np * sizeof(PairState)));
     a.state = h->state.as<PairState>();
     a.T_override = nullptr;
     a.d_max = h->prm.max_distance_correspondence;
     a.out_idx = nullptr;
     a.out_dist = nullptr;
     a.out_W = nullptr;
-    a.slice_begin = a.slice_end = -1;
+    a.slice_begin = lp.slice_begin;
+    a.slice_end = lp.slice_end;
     a.ignore_status = 0;
-    a.track_max_cells = getenv("GICP_TRACK_CELLS") ? atoi(getenv("GICP_TRACK_CELLS")) : 1 << 30;
-    a.centre_first = getenv("GICP_CENTRE_FIRST") ? atoi(getenv("GICP_CENTRE_FIRST")) : 1;
-    a.shell_search = getenv("GICP_SHELL_SEARCH") ? atoi(getenv("GICP_SHELL_SEARCH")) : 1;
+    a.track_max_cells = sw.track_max_cells;
+    a.centre_first = sw.centre_first;
+    a.shell_search = sw.shell_search;
     a.active_list = nullptr;
     a.n_list = nullptr;
-    int span = S.max_n;
-    if (allow_slice && h->comm && S.n_clouds == 1) {
-        a.slice_begin = (int)(S.n_total * h->rank / h->n_ranks);
-        a.slice_end = (int)(S.n_total * (h->rank + 1) / h->n_ranks);
-        span = a.slice_end - a.slice_begin;
-    }
-    // enough blocks to fill the machine, as many points per thread as that allows (<= OBJ_MAX_PPT)
-    const long long total_pts = (long long)std::max(span, 1) * S.n_clouds;
-    int ppt = (int)(total_pts / (148LL * 8 * OBJ_THREADS));
-    // the accumulation's software pipeline has a fill bubble per thread (match index -> gathered record): longer
-    // per-thread runs amortise it when the batch is large enough.  Measured per 1024 pairs of the bench workload:
-    // 16 / 32 / 64 points per thread -> 9.66 / 9.16 / 9.31 ms (GICP_ACC_PPT: A/B timing)
-    const int ppt_cap = (getenv("GICP_ACC_PPT") && atoi(getenv("GICP_ACC_PPT")) > 0) ? atoi(getenv("GICP_ACC_PPT")) : 2 * OBJ_MAX_PPT;
-    ppt = std::max(1, std::min(ppt_cap, ppt));
-    a.ppt = ppt;
-    blocks_per_pair = std::max(1, (span + OBJ_THREADS * ppt - 1) / (OBJ_THREADS * ppt));
-    a.blocks_per_pair = blocks_per_pair;
-    CU(h->partial.ensure((size_t)S.n_clouds * blocks_per_pair * Dim<D>::NRED * sizeof(double)));
-    CU(h->red.ensure((size_t)S.n_clouds * Dim<D>::NRED * sizeof(double)));
+    a.ppt = lp.acc_ppt;
+    a.blocks_per_pair = lp.bpp;
+    CU(h->partial.ensure((size_t)np * lp.bpp * Dim<D>::NRED * sizeof(double)));
+    CU(h->red.ensure((size_t)np * Dim<D>::NRED * sizeof(double)));
     a.partial = h->partial.as<double>();
-    CU(h->prev_match.ensure((size_t)std::max<int64_t>(S.n_total, 1) * sizeof(int)));
+    CU(h->prev_match.ensure((size_t)std::max<int64_t>(S.plan.n_total, 1) * sizeof(int)));
     a.match = h->prev_match.as<int>();
-    CU(h->slack.ensure((size_t)std::max<int64_t>(S.n_total, 1) * sizeof(float)));
+    CU(h->slack.ensure((size_t)std::max<int64_t>(S.plan.n_total, 1) * sizeof(float)));
     a.slack = nullptr;
+    return 0;
+}
+
+// the host transforms to T_dev, complete before the call returns (the caller's buffer may go away)
+int upload_T(gicpContext* h, const double* h_T, size_t bytes, cudaStream_t st) {
+    CU(h->T_dev.ensure(bytes));
+    CU(cudaMemcpyAsync(h->T_dev.p, h_T, bytes, cudaMemcpyHostToDevice, st));
+    CU(cudaStreamSynchronize(st));
     return 0;
 }
 
 template <int D, typename Real>
 int ensure_state(gicpContext* h, const double* h_T0, double* d_T, double* d_T_hist, int* d_n_outer,
                  int* d_converged, cudaStream_t st) {
-    const int np = h->src.n_clouds;
+    const int np = h->src.plan.n_clouds;
     CU(h->state.ensure((size_t)np * sizeof(PairState)));
     CU(h->n_active.ensure(sizeof(int)));
     const double* d_T0 = nullptr;
     if (h_T0) {
-        const size_t bytes = (size_t)np * (D + 1) * (D + 1) * sizeof(double);
-        CU(h->T_dev.ensure(bytes));
-        CU(cudaMemcpyAsync(h->T_dev.p, h_T0, bytes, cudaMemcpyHostToDevice, st));
-        CU(cudaStreamSynchronize(st));
+        if (upload_T(h, h_T0, (size_t)np * (D + 1) * (D + 1) * sizeof(double), st)) return 1;
         d_T0 = h->T_dev.as<double>();
     }
     init_state_kernel<D><<<(np + 127) / 128, 128, 0, st>>>(h->state.as<PairState>(), d_T0, h->tgt.knn.bbox.as<double>(), np,
@@ -681,29 +572,24 @@ int ensure_state(gicpContext* h, const double* h_T0, double* d_T, double* d_T_hi
 }
 
 template <int D, typename Real>
-int do_register(gicpContext* h, const double* h_T0, double* d_T, int* d_n_outer, int* d_converged,
+int do_register(gicpContext* h, const Switches& sw, const double* h_T0, double* d_T, int* d_n_outer, int* d_converged,
                 double* d_loss_hist, double* d_T_hist, int* d_inliers, cudaStream_t st) {
     ObjArgs<Real> oa;
-    int bpp = 1;
-    if (objective_args<D, Real>(h, oa, bpp, true)) return 1;
-    const int np = h->src.n_clouds;
+    LoopPlan lp;
+    if (objective_args<D, Real>(h, sw, true, h_T0 != nullptr, oa, lp)) return 1;
+    const int np = h->src.plan.n_clouds;
+    const int bpp = lp.bpp;
     h->last_stream = st;
-    // Small pairs (every source cloud fits one block): the whole outer loop in one launch (fused.cuh).  Not with a
-    // communicator (the all-reduce sits between the stages) and not while per-stage timing is on.
-    const bool fused = !(h->comm && np == 1) && !h->prof_on && h->src.max_n <= OBJ_THREADS * OBJ_MAX_PPT &&
-                       !(getenv("GICP_FUSED_LOOP") && atoi(getenv("GICP_FUSED_LOOP")) == 0);
-    // without a start transform the fused loop initialises its pair itself (state, match and slack arrays)
-    const bool self_init = fused && !h_T0;
-    if (self_init) {
+    if (lp.self_init) {
         CU(h->state.ensure((size_t)np * sizeof(PairState)));
     } else {
         if (ensure_state<D, Real>(h, h_T0, d_T, d_T_hist, d_n_outer, d_converged, st)) return 1;
         // last iteration's match per source point (bounds the next search); -1 = none yet
-        CU(cudaMemsetAsync(h->prev_match.p, 0xFF, (size_t)std::max<int64_t>(h->src.n_total, 1) * sizeof(int), st));
-        CU(cudaMemsetAsync(h->slack.p, 0, (size_t)std::max<int64_t>(h->src.n_total, 1) * sizeof(float), st));
+        CU(cudaMemsetAsync(h->prev_match.p, 0xFF, (size_t)std::max<int64_t>(h->src.plan.n_total, 1) * sizeof(int), st));
+        CU(cudaMemsetAsync(h->slack.p, 0, (size_t)std::max<int64_t>(h->src.plan.n_total, 1) * sizeof(float), st));
     }
     oa.use_prev = 1;
-    oa.slack = (getenv("GICP_NO_SKIP") && atoi(getenv("GICP_NO_SKIP"))) ? nullptr : h->slack.as<float>();
+    oa.slack = sw.no_skip ? nullptr : h->slack.as<float>();
     SolveArgs sa;
     sa.partial = h->partial.as<double>();
     sa.blocks_per_pair = bpp;
@@ -722,8 +608,8 @@ int do_register(gicpContext* h, const double* h_T0, double* d_T, int* d_n_outer,
     sa.n_active = h->n_active.as<int>();
     sa.active_list = nullptr;
     sa.n_list = nullptr;
-    if (fused) {
-        oa.ppt = std::max(1, (h->src.max_n + OBJ_THREADS - 1) / OBJ_THREADS);
+    if (lp.fused) {
+        oa.ppt = lp.fused_ppt;
         oa.blocks_per_pair = 1;
         sa.blocks_per_pair = 1;
         sa.n_active = nullptr;   // nobody polls
@@ -731,32 +617,21 @@ int do_register(gicpContext* h, const double* h_T0, double* d_T, int* d_n_outer,
         CU(cudaFuncSetAttribute(register_loop_kernel<D, Real>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         ProfScope prof(h, GICP_STAGE_CORRESPOND, st);
         register_loop_kernel<D, Real><<<np, OBJ_THREADS, smem, st>>>(oa, sa,
-                                                                     self_init ? h->tgt.knn.bbox.as<double>() : nullptr);
+                                                                     lp.self_init ? h->tgt.knn.bbox.as<double>() : nullptr);
         h->launches += 1;
         CU(cudaGetLastError());
         return 0;
     }
-    const dim3 ogrid(bpp, np);
-    // thousands of block partials per pair (one large pair): fold them 64 to 1 before the one-warp sum of K4
-    const bool presum = bpp > 2 * PRESUM_SPAN;
-    const int bpp2 = (bpp + PRESUM_SPAN - 1) / PRESUM_SPAN;
-    if (presum) {
+    const int bpp2 = lp.bpp2;
+    if (lp.presum) {
         CU(h->partial2.ensure((size_t)np * bpp2 * Dim<D>::NRED * sizeof(double)));
         sa.partial = h->partial2.as<double>();
         sa.blocks_per_pair = bpp2;
     }
-    // the search runs on smaller blocks than the accumulation (its work per point is uneven: better balance and
-    // a shorter tail), the accumulation keeps the longer per-thread pipeline
     ObjArgs<Real> oc = oa;
-    {
-        int split = getenv("GICP_CORR_SPLIT") ? atoi(getenv("GICP_CORR_SPLIT")) : 2;
-        while (oa.ppt / split > OBJ_MAX_PPT / 2) split *= 2;   // the search keeps blocks of <= 8 points per thread
-        while (split > 1 && oa.ppt % split) --split;
-        oc.ppt = oa.ppt / std::max(split, 1);
-    }
-    const dim3 cgrid(bpp * (oa.ppt / oc.ppt), np);
+    oc.ppt = lp.search_ppt;
     const int sgrid = (np + SOLVE_WARPS - 1) / SOLVE_WARPS;
-    const bool sharded = h->comm && np == 1;
+    const bool sharded = lp.sharded;
     // Progress polls (4 bytes each, the only host<->device traffic inside the loop).  A single-process registration
     // does not wait for them: the count of still-active pairs is copied to pinned memory after every iteration and
     // looked at (cudaEventQuery) before later iterations are launched, so the host runs a few iterations ahead and the
@@ -765,11 +640,9 @@ int do_register(gicpContext* h, const double* h_T0, double* d_T, int* d_n_outer,
     // mode keeps a blocking poll on a fixed schedule (all ranks see the same count: they solve bit-identical forms).
     constexpr int LOOK = 3;
     int issued = 0, checked = 0;
-    // Large batches: after every iteration the still-active pairs are compacted into a list (one small block), and
-    // the next launches cover only `known_active` slots of it - the latest polled count, an upper bound of the list's
-    // length since the count only falls.  Without it every launch of the convergence tail starts tens of thousands
-    // of blocks that return at once (4096 pairs: 131 k blocks per search launch).
-    const bool use_list = !sharded && np >= 64 && !(getenv("GICP_ACTIVE_LIST") && atoi(getenv("GICP_ACTIVE_LIST")) == 0);
+    // with the active-pair list the launches cover `known_active` slots of it: the latest polled count, an upper
+    // bound of the list's length since the count only falls
+    const bool use_list = lp.active_list;
     int known_active = np;
     if (use_list) {
         CU(h->active_list.ensure((size_t)(np + 1) * sizeof(int)));
@@ -795,15 +668,15 @@ int do_register(gicpContext* h, const double* h_T0, double* d_T, int* d_n_outer,
         const int gy = use_list ? known_active : np;
         {
             ProfScope prof(h, GICP_STAGE_CORRESPOND, st);
-            correspond_kernel<D, Real><<<dim3(cgrid.x, gy), OBJ_THREADS, obj_smem(oc.ppt), st>>>(oc);
+            correspond_kernel<D, Real><<<dim3(lp.search_bpp, gy), OBJ_THREADS, obj_smem(oc.ppt), st>>>(oc);
         }
         {
             ProfScope prof(h, GICP_STAGE_ACCUMULATE, st);
-            accumulate_kernel<D, Real><<<dim3(ogrid.x, gy), OBJ_THREADS, 0, st>>>(oa);
+            accumulate_kernel<D, Real><<<dim3(bpp, gy), OBJ_THREADS, 0, st>>>(oa);
         }
         {
             ProfScope prof(h, GICP_STAGE_SOLVE, st);
-            if (presum) {
+            if (lp.presum) {
                 presum_kernel<D><<<dim3(bpp2, np), Dim<D>::NRED, 0, st>>>(h->partial.as<double>(), bpp, h->partial2.as<double>(),
                                                                         bpp2, h->state.as<PairState>());
                 h->launches += 1;
@@ -829,7 +702,7 @@ int do_register(gicpContext* h, const double* h_T0, double* d_T, int* d_n_outer,
                 }
             }
         }
-        if (!sharded || (it + 1) % 2 == 0) {
+        if ((it + 1) % lp.poll_every == 0) {
             const int slot = issued % gicpContext::NPOLL;
             CU(cudaMemcpyAsync(h->h_poll + slot, h->n_active.p, sizeof(int), cudaMemcpyDeviceToHost, st));
             CU(cudaEventRecord(h->poll_ev[slot], st));
@@ -841,24 +714,22 @@ int do_register(gicpContext* h, const double* h_T0, double* d_T, int* d_n_outer,
 }
 
 template <int D, typename Real>
-int do_stage(gicpContext* h, const double* h_T, int* d_idx, double* d_dist, double* d_W, double* h_out,
-             cudaStream_t st) {
+int do_stage(gicpContext* h, const Switches& sw, const double* h_T, int* d_idx, double* d_dist, double* d_W,
+             double* h_out, cudaStream_t st) {
     ObjArgs<Real> oa;
-    int bpp = 1;
-    if (objective_args<D, Real>(h, oa, bpp, false)) return 1;
-    const int np = h->src.n_clouds;
+    LoopPlan lp;
+    // stage entry points always cover the whole source (no slicing), so their outputs are complete
+    if (objective_args<D, Real>(h, sw, false, true, oa, lp)) return 1;
+    const int np = h->src.plan.n_clouds;
+    const int bpp = lp.bpp;
     if (!h_T) return fail("h_T is required");
     if (ensure_state<D, Real>(h, nullptr, nullptr, nullptr, nullptr, nullptr, st)) return 1;
-    const size_t bytes = (size_t)np * (D + 1) * (D + 1) * sizeof(double);
-    CU(h->T_dev.ensure(bytes));
-    CU(cudaMemcpyAsync(h->T_dev.p, h_T, bytes, cudaMemcpyHostToDevice, st));
-    CU(cudaStreamSynchronize(st));
+    if (upload_T(h, h_T, (size_t)np * (D + 1) * (D + 1) * sizeof(double), st)) return 1;
     oa.T_override = h->T_dev.as<double>();
     oa.out_idx = d_idx;
     oa.out_dist = d_dist;
     oa.out_W = d_W;
     oa.ignore_status = 1;
-    // stage entry points always cover the whole source (no slicing), so their outputs are complete
     correspond_kernel<D, Real><<<dim3(bpp, np), OBJ_THREADS, obj_smem(oa.ppt), st>>>(oa);
     if (d_W || h_out) accumulate_kernel<D, Real><<<dim3(bpp, np), OBJ_THREADS, 0, st>>>(oa);
     h->launches += 2;
@@ -883,17 +754,19 @@ template <int D, typename Real>
 int do_knn(gicpContext* h, int which, int* d_idx, double* d_dist, cudaStream_t st) {
     CloudSet& cs = which == GICP_TARGET ? h->tgt : h->src;
     if (!cs.ready) return fail("cloud not set");
-    // re-runs K2 with the index outputs enabled (covariances are rewritten with identical values)
-    return launch_knn<D, Real>(h, cs, d_idx, d_dist, st, -1, -1, h->scr[0]);
+    // re-runs K2 over the whole cloud set with the index outputs enabled; the covariances are rewritten with the
+    // values of that run (the set-up's own values unless the set-up ran a constant model or a sharded slice)
+    return launch_knn<D, Real>(h, cs, cs.plan.knn_whole, d_idx, d_dist, st, -1, -1, h->scr[0]);
 }
 
 template <int D, typename Real>
 int do_cov(gicpContext* h, int which, double* d_cov, cudaStream_t st) {
     CloudSet& cs = which == GICP_TARGET ? h->tgt : h->src;
     if (!cs.ready) return fail("cloud not set");
-    if (cs.n_total == 0) return 0;
-    const int bx = (cs.max_n + 255) / 256;
-    export_cov_kernel<D, Real><<<dim3(bx, cs.n_clouds), 256, 0, st>>>(cs.knn.meta.as<CloudMeta>(),
+    const SetupPlan& p = cs.plan;
+    if (p.n_total == 0) return 0;
+    const int bx = (p.max_n + 255) / 256;
+    export_cov_kernel<D, Real><<<dim3(bx, p.n_clouds), 256, 0, st>>>(cs.knn.meta.as<CloudMeta>(),
                                                                       cs.knn.spts.as<PRec<Real>>(),
                                                                       cs.cov_knn.as<Real>(), d_cov);
     h->launches += 1;
@@ -905,16 +778,14 @@ template <int D, typename Real>
 int do_rotcov(gicpContext* h, const double* h_T, int n_T, double* d_out, cudaStream_t st) {
     CloudSet& cs = h->src;
     if (!cs.ready) return fail("source not set");
-    if (n_T <= 0 || cs.n_total == 0) return 0;
+    const SetupPlan& p = cs.plan;
+    if (n_T <= 0 || p.n_total == 0) return 0;
     if (n_T > 65535) return fail("n_T too large");
-    const size_t bytes = (size_t)n_T * cs.n_clouds * (D + 1) * (D + 1) * sizeof(double);
-    CU(h->T_dev.ensure(bytes));
-    CU(cudaMemcpyAsync(h->T_dev.p, h_T, bytes, cudaMemcpyHostToDevice, st));
-    CU(cudaStreamSynchronize(st));
-    const int bx = (cs.max_n + 255) / 256;
-    rotated_cov_kernel<D, Real><<<dim3(bx, cs.n_clouds, n_T), 256, 0, st>>>(
+    if (upload_T(h, h_T, (size_t)n_T * p.n_clouds * (D + 1) * (D + 1) * sizeof(double), st)) return 1;
+    const int bx = (p.max_n + 255) / 256;
+    rotated_cov_kernel<D, Real><<<dim3(bx, p.n_clouds, n_T), 256, 0, st>>>(
         cs.knn.meta.as<CloudMeta>(), cs.knn.spts.as<PRec<Real>>(), cs.cov_knn.as<Real>(), h->T_dev.as<double>(),
-        cs.n_clouds, (size_t)cs.n_total, d_out);
+        p.n_clouds, (size_t)p.n_total, d_out);
     h->launches += 1;
     CU(cudaGetLastError());
     return 0;
@@ -932,14 +803,8 @@ template <int D, typename Real>
 int do_voxel(gicpContext* h, const void* d_points, const int64_t* h_off, int nc, double leaf, int min_points,
              void* d_out, int64_t* h_out_off, int* d_voxel_of, int* d_counts, cudaStream_t st) {
     VoxelScratch& v = h->vox;
-    if (nc <= 0 || nc > 65535) return fail("n_clouds must be in [1, 65535] (got %d)", nc);
-    if (h_off[0] != 0) return fail("offsets[0] must be 0");
     int max_n = 0;
-    for (int i = 1; i <= nc; ++i) {
-        if (h_off[i] < h_off[i - 1]) return fail("offsets must be non-decreasing");
-        if (h_off[i] >= (1LL << 31) - 1024) return fail("more than 2^31 points in one batch");
-        max_n = std::max<int>(max_n, (int)(h_off[i] - h_off[i - 1]));
-    }
+    if (const char* e = check_offsets(h_off, nc, &max_n)) return fail("%s (%d clouds)", e, nc);
     const int n = (int)h_off[nc];
     if (n == 0) {
         for (int i = 0; i <= nc; ++i) h_out_off[i] = 0;
@@ -1187,13 +1052,13 @@ int gicpSetParams(gicpHandle h, const gicpParams* p) {
 int gicpSetTarget(gicpHandle h, const void* d_points, const int64_t* h_offsets, int32_t n_clouds, void* stream) {
     if (check(h)) return 1;
     if (!h_offsets) return fail("null offsets");
-    return DISPATCH(h, set_cloud, h, GICP_TARGET, d_points, h_offsets, n_clouds, (cudaStream_t)stream, 0);
+    return DISPATCH(h, set_cloud, h, read_switches(), GICP_TARGET, d_points, h_offsets, n_clouds, (cudaStream_t)stream, 0);
 }
 
 int gicpSetSource(gicpHandle h, const void* d_points, const int64_t* h_offsets, int32_t n_clouds, void* stream) {
     if (check(h)) return 1;
     if (!h_offsets) return fail("null offsets");
-    return DISPATCH(h, set_cloud, h, GICP_SOURCE, d_points, h_offsets, n_clouds, (cudaStream_t)stream, 0);
+    return DISPATCH(h, set_cloud, h, read_switches(), GICP_SOURCE, d_points, h_offsets, n_clouds, (cudaStream_t)stream, 0);
 }
 
 int gicpSetPair(gicpHandle h, const void* d_target, const int64_t* h_target_offsets, const void* d_source,
@@ -1201,16 +1066,13 @@ int gicpSetPair(gicpHandle h, const void* d_target, const int64_t* h_target_offs
     if (check(h)) return 1;
     if (!h_target_offsets || !h_source_offsets) return fail("null offsets");
     cudaStream_t st = (cudaStream_t)stream;
-    // Side by side while one side alone cannot fill the GPU: the single-block set-ups of small clouds, and up to ~1 M
-    // points per side (a 100k cloud's k-NN is one partial wave of blocks whose duration is its slowest chunk).  Each
-    // side has its own scratch (scr[0] / scr[1]).  Larger sides saturate the device on their own: sequential.
     if (n_clouds <= 0) return fail("n_clouds must be positive");
-    const int64_t side_max = getenv("GICP_PAIR_OVERLAP_MAX") ? atoll(getenv("GICP_PAIR_OVERLAP_MAX")) : (1LL << 20);
-    const bool concurrent = !h->comm && !h->prof_on && h_target_offsets[n_clouds] <= side_max &&
-                            h_source_offsets[n_clouds] <= side_max;
-    if (!concurrent) {
-        if (DISPATCH(h, set_cloud, h, GICP_TARGET, d_target, h_target_offsets, n_clouds, st, 0)) return 1;
-        return DISPATCH(h, set_cloud, h, GICP_SOURCE, d_source, h_source_offsets, n_clouds, st, 0);
+    const Switches sw = read_switches();
+    // side by side (pair_overlap), each side with its own scratch (scr[0] / scr[1]), or one after the other
+    if (!pair_overlap(sw, Ranks{h->comm != nullptr, h->n_ranks, h->rank}, h->prof_on, h_target_offsets[n_clouds],
+                      h_source_offsets[n_clouds])) {
+        if (DISPATCH(h, set_cloud, h, sw, GICP_TARGET, d_target, h_target_offsets, n_clouds, st, 0)) return 1;
+        return DISPATCH(h, set_cloud, h, sw, GICP_SOURCE, d_source, h_source_offsets, n_clouds, st, 0);
     }
     if (!h->side_stream) {
         CU(cudaStreamCreateWithFlags(&h->side_stream, cudaStreamNonBlocking));
@@ -1221,8 +1083,9 @@ int gicpSetPair(gicpHandle h, const void* d_target, const int64_t* h_target_offs
     // join: `stream` continues only after the source side is set up
     CU(cudaEventRecord(h->ev_fork, st));
     CU(cudaStreamWaitEvent(h->side_stream, h->ev_fork, 0));
-    const int rc_t = DISPATCH(h, set_cloud, h, GICP_TARGET, d_target, h_target_offsets, n_clouds, st, 0);
-    const int rc_s = rc_t ? 1 : DISPATCH(h, set_cloud, h, GICP_SOURCE, d_source, h_source_offsets, n_clouds, h->side_stream, 1);
+    const int rc_t = DISPATCH(h, set_cloud, h, sw, GICP_TARGET, d_target, h_target_offsets, n_clouds, st, 0);
+    const int rc_s =
+        rc_t ? 1 : DISPATCH(h, set_cloud, h, sw, GICP_SOURCE, d_source, h_source_offsets, n_clouds, h->side_stream, 1);
     CU(cudaEventRecord(h->ev_join, h->side_stream));
     CU(cudaStreamWaitEvent(st, h->ev_join, 0));
     h->last_stream = st;
@@ -1242,7 +1105,7 @@ int gicpRegister(gicpHandle h, const double* h_T0, double* d_T, int32_t* d_n_out
                  double* d_loss_hist, double* d_T_hist, int32_t* d_inliers, void* stream) {
     if (check(h)) return 1;
     if (!d_T || !d_n_outer || !d_converged) return fail("d_T, d_n_outer and d_converged are required");
-    return DISPATCH(h, do_register, h, h_T0, d_T, d_n_outer, d_converged, d_loss_hist, d_T_hist, d_inliers,
+    return DISPATCH(h, do_register, h, read_switches(), h_T0, d_T, d_n_outer, d_converged, d_loss_hist, d_T_hist, d_inliers,
                     (cudaStream_t)stream);
 }
 
@@ -1260,13 +1123,13 @@ int gicpCovariances(gicpHandle h, int which, double* d_cov, void* stream) {
 
 int gicpCorrespond(gicpHandle h, const double* h_T, int32_t* d_idx, double* d_dist, double* d_W, void* stream) {
     if (check(h)) return 1;
-    return DISPATCH(h, do_stage, h, h_T, d_idx, d_dist, d_W, (double*)nullptr, (cudaStream_t)stream);
+    return DISPATCH(h, do_stage, h, read_switches(), h_T, d_idx, d_dist, d_W, (double*)nullptr, (cudaStream_t)stream);
 }
 
 int gicpNormalEquations(gicpHandle h, const double* h_T, double* h_out, void* stream) {
     if (check(h)) return 1;
     if (!h_out) return fail("h_out is required");
-    return DISPATCH(h, do_stage, h, h_T, (int*)nullptr, (double*)nullptr, (double*)nullptr, h_out,
+    return DISPATCH(h, do_stage, h, read_switches(), h_T, (int*)nullptr, (double*)nullptr, (double*)nullptr, h_out,
                     (cudaStream_t)stream);
 }
 

@@ -428,176 +428,6 @@ __global__ void __launch_bounds__(KNN_THREADS) knn_hist_kernel(const KnnArgs<Rea
     }
 }
 
-// ================================================================================================
-// fast path, per-lane variant: every lane walks the cells around its own query (ring by ring)
-// straight from L1/L2 - 32 lanes of a Morton-compact warp touch the same few cells - instead of
-// scanning the union of all 32 neighbourhoods.  Same three sweeps (histogram bound, list, rank).
-// ================================================================================================
-constexpr int KNN_LANE_WARP_SMEM = KNN_LIST_BYTES;   // the histogram (sweep 1) and the list (sweeps 2-3) share it
-
-template <int D, typename Real>
-__global__ void __launch_bounds__(KNN_THREADS) knn_lane_kernel(const KnnArgs<Real> a) {
-    using KeyT = Real;
-    constexpr int CAP = knn_list_cap<Real>();
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    unsigned char* wbase = smem_raw + warp * KNN_LANE_WARP_SMEM;
-    unsigned char* hist = wbase;                                                   // [KNN_BINS][32] uint8, sweep 1
-    KeyT* lk = reinterpret_cast<KeyT*>(wbase);                                     // [CAP][32], sweeps 2-3 (aliases hist)
-    int* li = reinterpret_cast<int*>(wbase + CAP * 32 * sizeof(KeyT));
-
-    const int cloud = blockIdx.y;
-    const CloudMeta m = a.meta[cloud];
-    int begin = m.pt_begin, end = m.pt_end;
-    if (a.slice_begin >= 0) { begin = max(begin, a.slice_begin); end = min(end, a.slice_end); }
-    const int base = begin + (blockIdx.x * KNN_WARPS + warp) * 32;
-    if (base >= end) return;
-#pragma unroll
-    for (int b = 0; b < KNN_BINS; ++b) hist[b * 32 + lane] = 0;
-
-    const bool valid = base + lane < end;
-    const PRec<Real> me = a.spts[valid ? base + lane : end - 1];
-    const int my_idx = (int)me.idx;
-    const Real mx = me.x, my = me.y, mz = me.z;
-    const int cx = min(max(cell_coord((double)mx, m.origin[0], m.inv_h), 0), m.dims[0] - 1);
-    const int cy = min(max(cell_coord((double)my, m.origin[1], m.inv_h), 0), m.dims[1] - 1);
-    const int cz = (D == 3) ? min(max(cell_coord((double)mz, m.origin[2], m.inv_h), 0), m.dims[2] - 1) : 0;
-    const int* L = a.lut + m.lut_base;
-    const int* CS = a.cell_start + m.cell_base;
-
-    const double r2cap = a.radius * a.radius * (1.0 + 1e-12);
-    const float r2cap32 = __double2float_ru(r2cap * (1.0 + 1e-6));
-    const int ubase = (int)(__float_as_uint(r2cap32) >> 20) - (KNN_BINS - 1);
-    const float pad = cell_box_pad(m);
-    const int rho_max = max(1, (int)ceil(a.radius / (m.h * (1.0 - 1e-9))));
-
-    auto dist32 = [&](const PRec<Real>& c) {
-        if (sizeof(Real) == 4) {
-            const float dx = (float)c.x - (float)mx, dy = (float)c.y - (float)my, dz = (float)c.z - (float)mz;
-            return fmaf(dz, dz, fmaf(dy, dy, dx * dx));
-        } else {
-            return (float)exact_d2((double)c.x - (double)mx, (double)c.y - (double)my, (double)c.z - (double)mz);
-        }
-    };
-    // ---- sweep 1: histogram the distances, nearest cells first ----
-    // Shell 1 is walked as faces, then edges, then corners; between the classes the histogram is
-    // consulted, and a cell whose box lies beyond the current bound on the k-th distance is skipped
-    // (none of its points can be among the k nearest).
-    float bound32 = r2cap32;
-    float edge_lo = 0.0f;
-    int rho_fin = rho_max;
-    int seen = 0;
-    const float qx = (float)mx, qy = (float)my, qz = (float)mz;
-    auto visit = [&](int x, int y, int z) {
-        if (x < 0 || y < 0 || z < 0 || x >= m.dims[0] || y >= m.dims[1] || z >= m.dims[2]) return;
-        if (cell_box_dist2(m, pad, qx, qy, qz, x, y, z, x, y, z) > bound32) return;
-        const int* cs = CS + (__ldg(L + x) | __ldg(L + GICP_LUT_N + y) | __ldg(L + 2 * GICP_LUT_N + z));
-        const int j0 = __ldg(cs), j1 = __ldg(cs + 1);
-        for (int j = j0; j < j1; ++j) {
-            const float d2 = dist32(a.spts[j]);
-            const int g = min(max((int)(__float_as_uint(d2) >> 20) - ubase, 0), KNN_BINS - 1);
-            if (d2 <= r2cap32) { hist[g * 32 + lane] += 1; ++seen; }
-        }
-    };
-    // bin of the k-th candidate so far -> (lower edge, upper edge) of that bin; false if fewer than k
-    auto kth_bin = [&](float& lo_e, float& hi_e) {
-        if (seen < a.k) return false;
-        int cum = 0, kb = KNN_BINS - 1;
-        for (int b = 0; b < KNN_BINS; ++b) {
-            cum += hist[b * 32 + lane];
-            if (cum >= a.k) { kb = b; break; }
-        }
-        // every candidate of bins <= kb has d2 < hi_e (exact: bin edges are float bit patterns)
-        lo_e = (kb > 0) ? __uint_as_float((unsigned)(ubase + kb) << 20) : 0.0f;
-        hi_e = (kb < KNN_BINS - 1) ? __uint_as_float((unsigned)(ubase + kb + 1) << 20) : r2cap32;
-        return true;
-    };
-    auto cover_of = [&](int rho) {
-        // distance from the query to the nearest face of the searched box that has cells behind it
-        double cover = INFINITY;
-        const double q[3] = {(double)mx, (double)my, (double)mz};
-        const int c[3] = {cx, cy, cz};
-#pragma unroll
-        for (int ax = 0; ax < D; ++ax) {
-            if (c[ax] - rho > 0) cover = fmin(cover, q[ax] - (m.origin[ax] + (c[ax] - rho) * m.h));
-            if (c[ax] + rho < m.dims[ax] - 1) cover = fmin(cover, m.origin[ax] + (c[ax] + rho + 1) * m.h - q[ax]);
-        }
-        return cover * (1.0 - 1e-9);
-    };
-    for (int rho = 0; rho <= rho_max; ++rho) {
-        if (rho == 0) {
-            visit(cx, cy, cz);
-        } else if (rho == 1) {
-            for (int cls = 1; cls <= D; ++cls) {
-                for (int dz = (D == 3) ? -1 : 0; dz <= ((D == 3) ? 1 : 0); ++dz)
-                    for (int dy = -1; dy <= 1; ++dy)
-                        for (int dx = -1; dx <= 1; ++dx)
-                            if (abs(dx) + abs(dy) + abs(dz) == cls) visit(cx + dx, cy + dy, cz + dz);
-                float lo_e, hi_e;
-                if (kth_bin(lo_e, hi_e)) bound32 = fminf(bound32, hi_e);
-            }
-        } else {
-            for (int dz = (D == 3) ? -rho : 0; dz <= ((D == 3) ? rho : 0); ++dz)
-                for (int dy = -rho; dy <= rho; ++dy) {
-                    const bool outer = abs(dz) == rho || abs(dy) == rho;
-                    if (outer) {
-                        for (int dx = -rho; dx <= rho; ++dx) visit(cx + dx, cy + dy, cz + dz);
-                    } else {
-                        visit(cx - rho, cy + dy, cz + dz);
-                        visit(cx + rho, cy + dy, cz + dz);
-                    }
-                }
-        }
-        float lo_e = 0.0f, hi_e = r2cap32;
-        const bool have = kth_bin(lo_e, hi_e);
-        if (have) bound32 = fminf(bound32, hi_e);
-        const double cover = cover_of(rho);
-        if ((have && (double)bound32 <= cover * cover) || cover >= a.radius) {
-            edge_lo = have ? lo_e : 0.0f;
-            rho_fin = rho;
-            break;
-        }
-    }
-    // ---- sweep 2: keep the candidates under the bound (cells that reach into the ball only) ----
-    __syncwarp();   // every lane is done with its histogram column before the list overwrites the memory
-    int cnt_l = 0;
-    const float list32 = bound32 * 1.000002f;   // see knn_hist_kernel
-    {
-        const int z0 = (D == 3) ? max(cz - rho_fin, 0) : 0, z1 = (D == 3) ? min(cz + rho_fin, m.dims[2] - 1) : 0;
-        const int y0 = max(cy - rho_fin, 0), y1 = min(cy + rho_fin, m.dims[1] - 1);
-        const int x0 = max(cx - rho_fin, 0), x1 = min(cx + rho_fin, m.dims[0] - 1);
-        for (int z = z0; z <= z1; ++z)
-            for (int y = y0; y <= y1; ++y)
-                for (int x = x0; x <= x1; ++x) {
-                    if (cell_box_dist2(m, pad, (float)mx, (float)my, (float)mz, x, y, z, x, y, z) > list32) continue;
-                    const int* cs = CS + (__ldg(L + x) | __ldg(L + GICP_LUT_N + y) | __ldg(L + 2 * GICP_LUT_N + z));
-                    const int j0 = __ldg(cs), j1 = __ldg(cs + 1);
-                    for (int j = j0; j < j1; ++j) {
-                        const PRec<Real> c = a.spts[j];
-                        KeyT key;
-                        if (sizeof(Real) == 4) key = (KeyT)dist32(c);
-                        else key = (KeyT)exact_d2((double)c.x - (double)mx, (double)c.y - (double)my,
-                                                  (double)c.z - (double)mz);
-                        if ((float)key <= list32) {
-                            if (cnt_l < CAP) { lk[cnt_l * 32 + lane] = key; li[cnt_l * 32 + lane] = (int)c.idx; }
-                            ++cnt_l;
-                        }
-                    }
-                }
-    }
-    const int mcount = min(cnt_l, CAP);
-    // hand the whole warp to the general path if any lane's list overflowed
-    if (__any_sync(0xffffffffu, cnt_l > CAP)) {
-        if (lane == 0) {
-            const int slot = atomicAdd(a.overflow_count, 1);
-            if (slot < a.overflow_cap) a.overflow_list[slot] = make_int2(cloud, base);
-        }
-        return;
-    }
-    if (!valid) return;
-    knn_rank_and_finish<D, Real>(a, m, base + lane, my_idx, mx, my, mz, lk, li, lane, mcount, edge_lo);
-}
-
 // Sorted top-k (slots [KCAP-k, KCAP) live, INT_MAX = empty) -> radius test, optional index / distance outputs,
 // sample covariance about the mean (ddof = 1) and its regularised form, written for sorted position s_pos.
 template <int D, typename Real, int KCAP>

@@ -18,12 +18,14 @@ def pair_range(n_pairs: int, rank: int, world: int) -> tuple[int, int]:
 
 
 def source_slice(n_points: int, rank: int, world: int) -> tuple[int, int]:
-    """Slice of the (Morton-sorted) source handled by `rank`; mirrors gicp_b200.cu objective_args()."""
+    """Slice of the (Morton-sorted) source handled by `rank`: the slice plan_loop (csrc/plan.h) gives the
+    registration loop (checked in tests/test_plan_host.py)."""
     return n_points * rank // world, n_points * (rank + 1) // world
 
 
 def equal_slice(n_points: int, rank: int, world: int) -> tuple[int, int]:
-    """Equal-length slices (the all-gather needs them); the tail slice is clipped.  Mirrors set_cloud()."""
+    """Equal-length slices (the all-gather needs them); the tail slice is clipped.  The slice plan_setup (csrc/plan.h)
+    gives the covariance estimation (checked in tests/test_plan_host.py)."""
     per = (n_points + world - 1) // world
     return min(n_points, per * rank), min(n_points, per * (rank + 1))
 

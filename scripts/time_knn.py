@@ -1,8 +1,7 @@
-"""A/B timing of the K2 variants on the bench workload (one process, the library reads the switches per launch):
-    python scripts/time_knn.py [pairs] [variants...]      variant = LANE:CELL, e.g. 0:0 1:0 0:1.0 0:1.6
-LANE = GICP_KNN_LANE (0 warp-cooperative, 1 per-lane walks), CELL = GICP_KNN_CELL (k-NN grid cell edge, 0 = auto).
+"""Timing of K2 at several k-NN grid cell edges on the bench workload (one process):
+    python scripts/time_knn.py [pairs] [cells...]      cell = k-NN grid cell edge in m (gicpParams.knn_cell), 0 = auto
 Prints the knn_cov stage time (CUDA events inside the library) and the largest covariance difference
-against the first variant."""
+against the first cell edge."""
 import os
 import sys
 
@@ -12,17 +11,14 @@ from generalized_icp_b200 import synthetic  # noqa: E402
 from generalized_icp_b200.engine import GicpEngine  # noqa: E402
 
 pairs = int(sys.argv[1]) if len(sys.argv) > 1 else 256
-variants = sys.argv[2:] or ["0:0", "1:0"]
+cells = sys.argv[2:] or ["0", "1.0", "1.6"]
 cfg = {k: v for k, v in synthetic.CONFIG4.items() if k != "n"}
 src, tgt, off, _ = synthetic.patches3d_batch_device(pairs, n=32768, seed=0, device="cuda", **cfg)
 off = off.cpu().numpy()
 eng = GicpEngine(3, "f32")
-eng.set_params(**synthetic.CONFIG4_PARAMS)
 ref = None
-for v in variants:
-    team, cell = v.split(":")
-    os.environ["GICP_KNN_LANE"] = team
-    os.environ["GICP_KNN_CELL"] = cell
+for cell in cells:
+    eng.set_params(**synthetic.CONFIG4_PARAMS, knn_cell=float(cell))
     for _ in range(2):
         eng.set_target(tgt, off)
     eng.profile(True)
@@ -35,5 +31,5 @@ for v in variants:
         ref = cov
     diff = float((cov - ref).abs().max())
     nbad = int(((cov - ref).abs().amax(dim=(1, 2)) > 1e-3).sum())
-    print(f"lane={team:>2s} cell={cell:>5s}  knn_cov {prof['knn_cov'][0] / 3:8.3f} ms  grid {prof['grid_build'][0] / 3:7.3f} ms"
+    print(f"cell={cell:>5s}  knn_cov {prof['knn_cov'][0] / 3:8.3f} ms  grid {prof['grid_build'][0] / 3:7.3f} ms"
           f"  max|dC| {diff:.2e}  points off by >1e-3: {nbad}", flush=True)
