@@ -13,6 +13,7 @@ SYMBOLS = [
     "gicpSetTarget", "gicpSetSource", "gicpSetPair", "gicpPromoteTargetToSource", "gicpRegister", "gicpKnn", "gicpCovariances", "gicpCorrespond",
     "gicpNormalEquations", "gicpSourceCovariancesAt", "gicpCommGetUniqueId", "gicpCommInit", "gicpCommDestroy",
     "gicpLaunchCount", "gicpProfile", "gicpProfileRead", "gicpRayCast", "gicpVoxelDownsample",
+    "gicpSetRobustKernel",
 ]
 
 
@@ -52,6 +53,7 @@ def load():
     lib.gicpDestroy.argtypes = [vp]
     lib.gicpDefaultParams.argtypes = [C.POINTER(GicpParams)]
     lib.gicpSetParams.argtypes = [vp, C.POINTER(GicpParams)]
+    lib.gicpSetRobustKernel.argtypes = [vp, C.c_int, C.c_double]
     for f in (lib.gicpSetTarget, lib.gicpSetSource):
         f.argtypes = [vp, vp, C.POINTER(i64), i32, vp]
     lib.gicpSetPair.argtypes = [vp, vp, C.POINTER(i64), vp, C.POINTER(i64), i32, vp]

@@ -12,7 +12,8 @@ namespace gicp {
 
 // `init_bbox` != nullptr: the kernel also initialises its pair (identity start, what init_state_kernel and the two
 // memsets of the match / slack arrays do on the multi-launch path) - a small registration is then ONE launch.
-template <int D, typename Real>
+// Robust: the accumulation weights every correspondence by its robust kernel weight (accumulate_block).
+template <int D, typename Real, bool Robust = false>
 __global__ void __launch_bounds__(OBJ_THREADS) register_loop_kernel(const ObjArgs<Real> oa, const SolveArgs sa,
                                                                     const double* init_bbox) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -41,7 +42,7 @@ __global__ void __launch_bounds__(OBJ_THREADS) register_loop_kernel(const ObjArg
     for (int it = 0; it < sa.max_iterations; ++it) {
         correspond_block<D, Real>(oa, pair, 0, ws, smem_raw, &s_state);
         __syncthreads();                                   // this block's matches are visible to the block
-        accumulate_block<D, Real>(oa, pair, 0, &s_state, s_sum);
+        accumulate_block<D, Real, Robust>(oa, pair, 0, &s_state, s_sum);
         __syncthreads();
         if (threadIdx.x < 32) solve_pair<D>(sa, pair, s_state, s_sum, s_sc, &s_state);   // warp 0, all lanes
         __syncthreads();                                   // the new state is visible to the block

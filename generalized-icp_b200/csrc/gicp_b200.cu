@@ -158,6 +158,8 @@ struct VoxelScratch {
 struct gicpContext {
     int device = 0, dim = 2, storage = GICP_STORAGE_F64;
     gicpParams prm;
+    int robust_kind = GICP_ROBUST_NONE;   // gicpSetRobustKernel
+    double robust_scale = 0.0;
     CloudSet src, tgt;
     // [0]: every call on the caller's stream; [1]: the source side of gicpSetPair while it runs on the internal stream
     SetupScratch scr[2];
@@ -505,7 +507,8 @@ int objective_args(gicpContext* h, const Switches& sw, bool sliced, bool has_T0,
     if (!S.ready || !T.ready) return fail("set source and target first");
     const int np = S.plan.n_clouds;
     if (np != T.plan.n_clouds) return fail("source has %d clouds, target %d", np, T.plan.n_clouds);
-    lp = plan_loop(sw, S.plan, sliced, Ranks{h->comm != nullptr, h->n_ranks, h->rank}, h->prof_on, has_T0);
+    lp = plan_loop(sw, S.plan, sliced, Ranks{h->comm != nullptr, h->n_ranks, h->rank}, h->prof_on, has_T0,
+                   h->robust_kind != GICP_ROBUST_NONE);
     a.src_meta = S.nng().meta.as<CloudMeta>();
     a.src_spts = S.nng().spts.as<PRec<Real>>();
     a.src_cov = S.covnn().as<Real>();
@@ -532,6 +535,8 @@ int objective_args(gicpContext* h, const Switches& sw, bool sliced, bool has_T0,
     a.shell_search = sw.shell_search;
     a.active_list = nullptr;
     a.n_list = nullptr;
+    a.robust_kind = h->robust_kind;
+    a.robust_scale = h->robust_scale;
     a.ppt = lp.acc_ppt;
     a.blocks_per_pair = lp.bpp;
     CU(h->partial.ensure((size_t)np * lp.bpp * Dim<D>::NRED * sizeof(double)));
@@ -614,10 +619,10 @@ int do_register(gicpContext* h, const Switches& sw, const double* h_T0, double* 
         sa.blocks_per_pair = 1;
         sa.n_active = nullptr;   // nobody polls
         const size_t smem = obj_smem(oa.ppt);
-        CU(cudaFuncSetAttribute(register_loop_kernel<D, Real>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        auto loop_kernel = lp.robust ? register_loop_kernel<D, Real, true> : register_loop_kernel<D, Real, false>;
+        CU(cudaFuncSetAttribute(loop_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         ProfScope prof(h, GICP_STAGE_CORRESPOND, st);
-        register_loop_kernel<D, Real><<<np, OBJ_THREADS, smem, st>>>(oa, sa,
-                                                                     lp.self_init ? h->tgt.knn.bbox.as<double>() : nullptr);
+        loop_kernel<<<np, OBJ_THREADS, smem, st>>>(oa, sa, lp.self_init ? h->tgt.knn.bbox.as<double>() : nullptr);
         h->launches += 1;
         CU(cudaGetLastError());
         return 0;
@@ -630,6 +635,7 @@ int do_register(gicpContext* h, const Switches& sw, const double* h_T0, double* 
     }
     ObjArgs<Real> oc = oa;
     oc.ppt = lp.search_ppt;
+    auto acc_kernel = lp.robust ? accumulate_kernel<D, Real, true> : accumulate_kernel<D, Real, false>;
     const int sgrid = (np + SOLVE_WARPS - 1) / SOLVE_WARPS;
     const bool sharded = lp.sharded;
     // Progress polls (4 bytes each, the only host<->device traffic inside the loop).  A single-process registration
@@ -672,7 +678,7 @@ int do_register(gicpContext* h, const Switches& sw, const double* h_T0, double* 
         }
         {
             ProfScope prof(h, GICP_STAGE_ACCUMULATE, st);
-            accumulate_kernel<D, Real><<<dim3(bpp, gy), OBJ_THREADS, 0, st>>>(oa);
+            acc_kernel<<<dim3(bpp, gy), OBJ_THREADS, 0, st>>>(oa);
         }
         {
             ProfScope prof(h, GICP_STAGE_SOLVE, st);
@@ -731,7 +737,8 @@ int do_stage(gicpContext* h, const Switches& sw, const double* h_T, int* d_idx, 
     oa.out_W = d_W;
     oa.ignore_status = 1;
     correspond_kernel<D, Real><<<dim3(bpp, np), OBJ_THREADS, obj_smem(oa.ppt), st>>>(oa);
-    if (d_W || h_out) accumulate_kernel<D, Real><<<dim3(bpp, np), OBJ_THREADS, 0, st>>>(oa);
+    auto acc_kernel = lp.robust ? accumulate_kernel<D, Real, true> : accumulate_kernel<D, Real, false>;
+    if (d_W || h_out) acc_kernel<<<dim3(bpp, np), OBJ_THREADS, 0, st>>>(oa);
     h->launches += 2;
     if (h_out) {
         SolveArgs sa;
@@ -972,7 +979,7 @@ int check(gicpHandle h) {
 extern "C" {
 
 const char* gicpGetLastError(void) { return g_last_error.c_str(); }
-int gicpVersion(void) { return 101; }
+int gicpVersion(void) { return 102; }
 
 int gicpDefaultParams(gicpParams* p) {
     if (!p) return fail("null params");
@@ -1046,6 +1053,18 @@ int gicpSetParams(gicpHandle h, const gicpParams* p) {
     if (h->prm.inner_max_iterations <= 0) h->prm.inner_max_iterations = 50;
     h->src.ready = false;
     h->tgt.ready = false;
+    return 0;
+}
+
+int gicpSetRobustKernel(gicpHandle h, int kind, double scale) {
+    if (check(h)) return 1;
+    if (kind < GICP_ROBUST_NONE || kind > GICP_ROBUST_TUKEY)
+        return fail("unknown robust kernel %d (GICP_ROBUST_NONE 0, HUBER 1, CAUCHY 2, TUKEY 3)", kind);
+    if (kind != GICP_ROBUST_NONE && !(std::isfinite(scale) && scale > 0))
+        return fail("robust kernel scale must be finite and > 0 (got %g)", scale);
+    // the set-up source and target stay valid: the weights enter only the accumulation of later calls
+    h->robust_kind = kind;
+    h->robust_scale = kind == GICP_ROBUST_NONE ? 0.0 : scale;
     return 0;
 }
 

@@ -17,6 +17,7 @@
 // reduced with warp shuffles, then across warps and blocks in fp64 in a fixed order (bitwise
 // reproducible, no float atomics).
 #pragma once
+#include "../../include/gicp_b200.h"
 #include "common.cuh"
 #include "stream.cuh"
 
@@ -61,6 +62,9 @@ template <typename Real> struct ObjArgs {
     // otherwise starts (and immediately retires) tens of thousands of blocks of finished pairs
     const int* active_list;
     const int* n_list;
+    // robust kernel (gicpSetRobustKernel): read only by the Robust instantiations of accumulate_block
+    int robust_kind;
+    double robust_scale;
 };
 
 // ---- the two fp32 bounds of the exact search (host-callable: tests/host_harness/bounds_host.cu checks them) ----
@@ -83,6 +87,28 @@ __host__ __device__ __forceinline__ float match_slack(float d1, float m2, float 
     float sl = fmaxf(0.f, 0.5f * (d2e - d1) * 0.99999f - 1e-6f * (Pf + d1));
     if (!(m2 < INFINITY)) sl = fmaxf(0.f, 0.5f * (fminf(rad32, 1e30f) - d1) * 0.99999f - 1e-6f * (Pf + d1));
     return sl;
+}
+
+// ---- robust kernel weight (IRLS; semantics in include/gicp_b200.h), host-callable: tests/host_harness/robust_host.cu
+// checks it bit for bit against the float64 formulas of the oracle.  Every product and sum is rounded on its own (no
+// FMA contraction), so the device, the host and numpy agree, and a huge scale gives w == 1.0 exactly for Huber and
+// Cauchy (u * u underflows to 0). ----
+__host__ __device__ __forceinline__ double robust_mul(double a, double b) {
+#ifdef __CUDA_ARCH__
+    return __dmul_rn(a, b);
+#else
+    return a * b;
+#endif
+}
+__host__ __device__ __forceinline__ double robust_weight(int kind, double d, double c) {
+    const double u = d / c;
+    if (kind == GICP_ROBUST_HUBER) return d <= c ? 1.0 : c / d;
+    if (kind == GICP_ROBUST_CAUCHY) return 1.0 / (1.0 + robust_mul(u, u));
+    if (kind == GICP_ROBUST_TUKEY) {
+        const double a = 1.0 - robust_mul(u, u);
+        return u < 1.0 ? robust_mul(a, a) : 0.0;
+    }
+    return 1.0;
 }
 
 template <typename Real>
@@ -418,8 +444,11 @@ __global__ void __launch_bounds__(OBJ_THREADS, (D == 3 && sizeof(Real) == 4) ? 1
 }
 
 // One block of the accumulation: points [bx * ppt * OBJ_THREADS, ...) of pair `pair` -> out[NRED]
-// (a.partial[pair][bx]; the fused loop passes its shared-memory sum and state instead)
-template <int D, typename Real>
+// (a.partial[pair][bx]; the fused loop passes its shared-memory sum and state instead).
+// Robust: every gated-in correspondence is weighted by robust_weight(kind, d, c) - W, v = W e and e^T W e are scaled by
+// w before they enter the accumulators, so the reduced form is that of sum w_i r_i^T W_i r_i.  A compile-time switch:
+// the Robust = false instantiations are the unweighted kernels, instruction for instruction.
+template <int D, typename Real, bool Robust = false>
 __device__ __forceinline__ void accumulate_block(const ObjArgs<Real>& a, const int pair, const int bx,
                                                  const PairState* stp, double* out) {
     using DD = Dim<D>;
@@ -537,6 +566,7 @@ __device__ __forceinline__ void accumulate_block(const ObjArgs<Real>& a, const i
         }
         // ---- W = inv(C_tgt[j] + R C_src[i] R^T), e = q - p' ----
         const PRec<Real> q = g.q;
+        double w_rob = 1.0;   // robust kernel weight at the current distance (Robust only)
         {   // gicp.py:136: the gate applies to the CURRENT distance (a kept match may have drifted out)
             const double d2 = exact_d2((double)q.x - pp[0], (double)q.y - pp[1], (double)q.z - pp[2]);
             if (sqrt(d2) > a.d_max) {
@@ -545,6 +575,7 @@ __device__ __forceinline__ void accumulate_block(const ObjArgs<Real>& a, const i
                 }
                 continue;
             }
+            if constexpr (Robust) w_rob = robust_weight(a.robust_kind, sqrt(d2), a.robust_scale);
         }
         double Cs[NS], M[NS], W[NS], e[D], v[D];
         {
@@ -588,6 +619,13 @@ __device__ __forceinline__ void accumulate_block(const ObjArgs<Real>& a, const i
         double li = 0.0;
 #pragma unroll
         for (int i = 0; i < D; ++i) li += e[i] * v[i];
+        if constexpr (Robust) {   // w W replaces W: the gated-in count below still counts this point
+            li *= w_rob;
+#pragma unroll
+            for (int i = 0; i < NS; ++i) W[i] *= w_rob;
+#pragma unroll
+            for (int i = 0; i < D; ++i) v[i] *= w_rob;
+        }
         loss_acc += li;
         ++cnt;
         if (a.out_W) {
@@ -647,11 +685,11 @@ __device__ __forceinline__ void accumulate_block(const ObjArgs<Real>& a, const i
 
 // f32 storage: 128 registers, 4 blocks per SM.  f64 storage carries 72 fp64 accumulators per thread: 2 blocks per SM
 // and 255 registers instead of ~1.2 KB of spills per thread under the 128-register cap
-template <int D, typename Real>
+template <int D, typename Real, bool Robust = false>
 __global__ void __launch_bounds__(OBJ_THREADS, (sizeof(Real) == 8 && D == 3) ? 2 : 4) accumulate_kernel(const ObjArgs<Real> a) {
     const int pair = obj_pair_of_block(a);
     if (pair < 0) return;
-    accumulate_block<D, Real>(a, pair, blockIdx.x, a.state + pair,
+    accumulate_block<D, Real, Robust>(a, pair, blockIdx.x, a.state + pair,
                               a.partial + ((size_t)pair * a.blocks_per_pair + blockIdx.x) * Dim<D>::NRED);
 }
 

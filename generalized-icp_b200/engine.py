@@ -15,6 +15,8 @@ from . import _lib
 from ._lib import GicpParams  # noqa: F401
 
 SOURCE, TARGET = 0, 1
+# robust kernels on the correspondence distance (GICP_ROBUST_*, include/gicp_b200.h)
+ROBUST_KINDS = {None: 0, "huber": 1, "cauchy": 2, "tukey": 3}
 _STORAGE = {"f32": (0, torch.float32), "f64": (1, torch.float64)}
 
 
@@ -70,6 +72,17 @@ class GicpEngine:
                 raise TypeError(f"unknown parameter {k!r}")
             setattr(self.params, k, v)
         _lib.check(self.lib.gicpSetParams(self._h, C.byref(self.params)))
+
+    def set_robust_kernel(self, kind, scale=None):
+        """Weight every gated-in correspondence by a robust kernel of its distance d (IRLS, weights frozen at T_k):
+        ``kind`` None (no weighting, the default), "huber", "cauchy" or "tukey"; ``scale`` c > 0 in the units of the
+        points, like max_distance_correspondence.  Semantics in include/gicp_b200.h.  Applies to every later
+        register / correspond / normal_equations; the set-up clouds are kept."""
+        if kind not in ROBUST_KINDS:
+            raise ValueError(f"unknown robust kernel {kind!r}; expected one of None, 'huber', 'cauchy', 'tukey'")
+        if kind is not None and scale is None:
+            raise ValueError(f"the {kind} kernel needs a scale")
+        _lib.check(self.lib.gicpSetRobustKernel(self._h, ROBUST_KINDS[kind], 0.0 if scale is None else float(scale)))
 
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)

@@ -23,11 +23,17 @@ def _rand_rotation(rng, max_deg):
 
 
 def patches3d_pair(n=100_000, n_patches=64, cube=100.0, patch=30.0, sigma=0.02,
-                   max_rot_deg=2.0, max_trans=0.5, seed=0):
+                   max_rot_deg=2.0, max_trans=0.5, seed=0, moved_patches=0, moved_offset=0.0):
     """Source and target drawn independently from the same random planar
     patches; the target surface is moved by a rigid motion about the cube
     centre.  Returned as float32 (N,3) arrays plus the 4x4 ground truth that
-    maps source onto target."""
+    maps source onto target.
+
+    Structured outliers (a moved object): with ``moved_patches`` = m > 0 the
+    target points of patches 0..m-1 are shifted by ``moved_offset`` along their
+    patch's normal before the rigid motion, so those matches are wrong by a
+    fixed distance that can lie inside the correspondence gate.  The defaults
+    draw exactly the same clouds as before (no extra random numbers)."""
     rng = np.random.default_rng(seed)
     centres = rng.uniform(0.25 * cube, 0.75 * cube, size=(n_patches, 3))
     frames = np.stack([np.linalg.qr(rng.normal(size=(3, 3)))[0] for _ in range(n_patches)])
@@ -36,10 +42,13 @@ def patches3d_pair(n=100_000, n_patches=64, cube=100.0, patch=30.0, sigma=0.02,
         which = rng.integers(0, n_patches, size=n)
         ab = rng.uniform(-patch / 2, patch / 2, size=(n, 2))
         p = centres[which] + ab[:, :1] * frames[which, :, 0] + ab[:, 1:] * frames[which, :, 1]
-        return p + rng.normal(0, sigma, size=(n, 3))
+        return p + rng.normal(0, sigma, size=(n, 3)), which
 
-    src = sample()
-    tgt = sample()
+    src, _ = sample()
+    tgt, which_t = sample()
+    if moved_patches:
+        moved = which_t < moved_patches
+        tgt[moved] += moved_offset * frames[which_t[moved], :, 2]
     R = _rand_rotation(rng, max_rot_deg)
     tdir = rng.normal(size=3)
     t = tdir / np.linalg.norm(tdir) * rng.uniform(0, max_trans)

@@ -74,6 +74,27 @@ int gicpVersion(void);
 int gicpDefaultParams(gicpParams* p);
 int gicpSetParams(gicpHandle h, const gicpParams* p);
 
+/* ---- robust kernels (M-estimators) on the correspondence distance ----------------------------------------------
+ * Every gated-in correspondence of outer iteration k gets a weight w_i, computed once at T_k and frozen with the
+ * matches and W_i (iteratively reweighted least squares).  d_i = sqrt(exact_d2(q_j - p'_i)) is the float64 distance
+ * the gate tests, c the scale in the units of the points (those of max_distance_correspondence), and in float64 with
+ * u = d_i / c:
+ *   GICP_ROBUST_NONE    w = 1 (the default: the reference's behaviour)
+ *   GICP_ROBUST_HUBER   w = d_i <= c ? 1 : c / d_i
+ *   GICP_ROBUST_CAUCHY  w = 1 / (1 + u*u)
+ *   GICP_ROBUST_TUKEY   w = u < 1 ? (1 - u*u)^2 : 0
+ * Each product and sum is rounded on its own (no fused multiply-add), so a huge c gives w == 1.0 exactly for Huber
+ * and Cauchy.  The inner problem of iteration k minimises sum w_i r_i^T W_i r_i; min_loss (d_loss_hist and the stop
+ * rule |last - min_loss| < tolerance) is the minimum of that weighted objective.  The gate is unchanged and applied
+ * first; d_inliers and the count slot of gicpNormalEquations still count every gated-in correspondence, so a Tukey
+ * weight of 0 is an inlier that contributes nothing.  The scale is a distance, not a Mahalanobis residual: it means
+ * the same in every covariance_model and is the soft counterpart of max_distance_correspondence.
+ * gicpSetRobustKernel validates kind, and scale (finite and > 0 unless kind is GICP_ROBUST_NONE), and applies to every
+ * later gicpRegister, gicpCorrespond and gicpNormalEquations on the handle.  Unlike gicpSetParams it keeps the set-up
+ * source and target, so one set-up can be registered with and without a kernel.                                  */
+enum { GICP_ROBUST_NONE = 0, GICP_ROBUST_HUBER = 1, GICP_ROBUST_CAUCHY = 2, GICP_ROBUST_TUKEY = 3 };
+int gicpSetRobustKernel(gicpHandle h, int kind, double scale);
+
 /* ---- clouds: grid build (replaces KDTree(points), gicp.py:21,127) and per-point
  *      covariances (replaces compute_covariance_matrix, gicp.py:19-35) ---------------------
  * d_points: (n_total, dim) row-major, float32 or float64 according to `storage`.
@@ -120,7 +141,8 @@ int gicpCovariances(gicpHandle h, int which, double* d_cov, void* stream);
 /* correspondences under the given transforms (gicp.py:119,129-145):
  *   h_T (n_clouds, dim+1, dim+1); d_idx (n_src_total) i32 matched target index or -1 when gated;
  *   d_dist (n_src_total) f64 1-NN distance (inf when nothing within the search bound);
- *   d_W optional (n_src_total, dim, dim) f64 weight matrices, 0 for gated rows.            */
+ *   d_W optional (n_src_total, dim, dim) f64 weight matrices, 0 for gated rows; with a robust kernel the
+ *   matrices the inner problem uses, w_i W_i (w_i at the distance d_dist reports).                               */
 int gicpCorrespond(gicpHandle h, const double* h_T, int32_t* d_idx, double* d_dist, double* d_W, void* stream);
 /* the fused per-iteration reduction at the given transforms: h_out (n_clouds, GICP_NRED_xD).
  * Layout (dim 3; p~ = (1, p' - mu), p' = R p + t, e = q - p', v = W e):
@@ -128,7 +150,8 @@ int gicpCorrespond(gicpHandle h, const double* h_T, int32_t* d_idx, double* d_di
  *   [60..71] sum v_c p~_a  (c slow, a fast)      [72] sum e^T W e      [73] gated-in count
  *   [74..76] mu                                  [77..79] 0
  * dim 2: ab in {00,01,02,11,12,22}, cd in {00,01,11} -> [0..17]; [18..23] v_c p~_a; [24] loss; [25] count;
- *   [26..27] mu.  Synchronises the stream.                                                 */
+ *   [26..27] mu.  With a robust kernel every term is that of w_i W_i (the weighted inner problem); the count is
+ *   still the gated-in count.  Synchronises the stream.                                                          */
 int gicpNormalEquations(gicpHandle h, const double* h_T, double* h_out, void* stream);
 
 /* source covariances as the reference recomputes them on the transformed cloud every outer
