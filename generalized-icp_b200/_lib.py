@@ -13,7 +13,7 @@ SYMBOLS = [
     "gicpSetTarget", "gicpSetSource", "gicpSetPair", "gicpPromoteTargetToSource", "gicpRegister", "gicpKnn", "gicpCovariances", "gicpCorrespond",
     "gicpNormalEquations", "gicpSourceCovariancesAt", "gicpCommGetUniqueId", "gicpCommInit", "gicpCommDestroy",
     "gicpLaunchCount", "gicpProfile", "gicpProfileRead", "gicpRayCast", "gicpVoxelDownsample",
-    "gicpSetRobustKernel",
+    "gicpSetRobustKernel", "gicpSetRobustKernelAdaptive", "gicpRobustScales", "gicpProfileReadStages",
 ]
 
 
@@ -54,6 +54,8 @@ def load():
     lib.gicpDefaultParams.argtypes = [C.POINTER(GicpParams)]
     lib.gicpSetParams.argtypes = [vp, C.POINTER(GicpParams)]
     lib.gicpSetRobustKernel.argtypes = [vp, C.c_int, C.c_double]
+    lib.gicpSetRobustKernelAdaptive.argtypes = [vp, C.c_int, C.c_double, C.c_double]
+    lib.gicpRobustScales.argtypes = [vp, dp, dp, vp]
     for f in (lib.gicpSetTarget, lib.gicpSetSource):
         f.argtypes = [vp, vp, C.POINTER(i64), i32, vp]
     lib.gicpSetPair.argtypes = [vp, vp, C.POINTER(i64), vp, C.POINTER(i64), i32, vp]
@@ -73,6 +75,7 @@ def load():
     lib.gicpVoxelDownsample.argtypes = [vp, vp, C.POINTER(i64), i32, C.c_double, i32, vp, C.POINTER(i64), vp, vp, vp]
     lib.gicpProfile.argtypes = [vp, C.c_int]
     lib.gicpProfileRead.argtypes = [vp, dp, C.POINTER(i64)]
+    lib.gicpProfileReadStages.argtypes = [vp, i32, dp, C.POINTER(i64)]
     _lib = lib
     return lib
 

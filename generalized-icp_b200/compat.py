@@ -52,14 +52,16 @@ def voxel_downsample(cloud, voxel_size, min_points=1):
 def gicp_extended(source_points, target_points, max_iterations=100, tolerance=1e-6,
                   max_distance_correspondence=150, max_distance_nearest_neighbors=50, k=6,
                   lambda_tangent=100.0, lambda_normal=10.0, storage="f64", full_history=True, covariance_model=0,
-                  voxel_size=None, robust_kernel=None, robust_scale=None, **engine_params):
+                  voxel_size=None, robust_kernel=None, robust_scale=None, robust_adaptive=None, robust_min_scale=None,
+                  **engine_params):
     """The registration with everything the engine knows (SURVEY.md discrepancy 3: the reference
     computes ``min_loss`` and drops it; here the loss history, inlier counts and the fitness-like
     final loss are returned as well).  Returns a dict.  With ``voxel_size`` both clouds are first
     voxel-grid downsampled on the GPU (in ``storage``); the dict then holds them as ``source_points`` /
     ``target_points`` (float64) and every per-point output refers to them.  ``robust_kernel`` (None, "huber",
     "cauchy" or "tukey") with ``robust_scale`` weights every correspondence by a robust kernel of its distance
-    (GicpEngine.set_robust_kernel); ``hw_src`` / ``hw_tgt`` then rank the weighted matrices w W."""
+    (GicpEngine.set_robust_kernel); ``hw_src`` / ``hw_tgt`` then rank the weighted matrices w W.  ``robust_adaptive``
+    (kappa) with ``robust_min_scale`` replaces ``robust_scale`` by the adaptive scale of every outer iteration."""
     import torch
 
     src = np.asarray(source_points)
@@ -78,7 +80,7 @@ def gicp_extended(source_points, target_points, max_iterations=100, tolerance=1e
                    max_distance_nearest_neighbors=float(max_distance_nearest_neighbors),
                    lambda_tangent=float(lambda_tangent), lambda_normal=float(lambda_normal),
                    covariance_model=int(covariance_model), **engine_params)
-    eng.set_robust_kernel(robust_kernel, robust_scale)
+    eng.set_robust_kernel(robust_kernel, robust_scale, adaptive=robust_adaptive, min_scale=robust_min_scale)
     r = eng.register_pair_host(src[:, :dim], tgt[:, :dim])  # gicp.py:104, 111, 116-167 in one staged round trip
     n_outer, conv = r["n_outer"], r["converged_at"]
     n_T = n_outer if conv >= 0 else n_outer + 1             # appendix A rule 12
@@ -107,7 +109,7 @@ def gicp_extended(source_points, target_points, max_iterations=100, tolerance=1e
                           max_distance_nearest_neighbors=float(max_distance_nearest_neighbors),
                           lambda_tangent=float(lambda_tangent), lambda_normal=float(lambda_normal),
                           covariance_model=int(covariance_model), **engine_params)
-            eh.set_robust_kernel(robust_kernel, robust_scale)
+            eh.set_robust_kernel(robust_kernel, robust_scale, adaptive=robust_adaptive, min_scale=robust_min_scale)
             n_s, n_t = len(src64), len(tgt64)
             eh.set_target(torch.as_tensor(np.tile(np.ascontiguousarray(tgt[:, :dim], dtype=np_dt), (reps, 1)), device=eh.device),
                           np.arange(reps + 1, dtype=np.int64) * n_t)

@@ -6,14 +6,17 @@
 // registration.  Requires every source cloud to fit one block (<= OBJ_THREADS * OBJ_MAX_PPT points).
 #pragma once
 #include "objective.cuh"
+#include "scale.cuh"
 #include "solve.cuh"
 
 namespace gicp {
 
 // `init_bbox` != nullptr: the kernel also initialises its pair (identity start, what init_state_kernel and the two
 // memsets of the match / slack arrays do on the multi-launch path) - a small registration is then ONE launch.
-// Robust: the accumulation weights every correspondence by its robust kernel weight (accumulate_block).
-template <int D, typename Real, bool Robust = false>
+// Robust: the accumulation weights every correspondence by its robust kernel weight (accumulate_block).  Adaptive
+// (with Robust): the block first selects the pair's scale of the iteration (block_pair_scale, scale.cuh).
+// Adaptive is a template argument of its own, so that the fixed-scale loop keeps its registers.
+template <int D, typename Real, bool Robust = false, bool Adaptive = false>
 __global__ void __launch_bounds__(OBJ_THREADS) register_loop_kernel(const ObjArgs<Real> oa, const SolveArgs sa,
                                                                     const double* init_bbox) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -42,7 +45,16 @@ __global__ void __launch_bounds__(OBJ_THREADS) register_loop_kernel(const ObjArg
     for (int it = 0; it < sa.max_iterations; ++it) {
         correspond_block<D, Real>(oa, pair, 0, ws, smem_raw, &s_state);
         __syncthreads();                                   // this block's matches are visible to the block
-        accumulate_block<D, Real, Robust>(oa, pair, 0, &s_state, s_sum);
+        double c = 0.0;                                    // the robust scale of this iteration
+        if constexpr (Adaptive) {
+            // the keys live behind the search's shared memory (obj_smem(ppt) + 8 B per point)
+            unsigned long long* keys = reinterpret_cast<unsigned long long*>(smem_raw + obj_smem(oa.ppt));
+            if constexpr (D == 2) c = block_pair_scale_call<D, Real>(oa, pair, &s_state, keys);
+            else c = block_pair_scale<D, Real>(oa, pair, &s_state, keys);
+        } else if constexpr (Robust) {
+            c = oa.robust_scale;
+        }
+        accumulate_block<D, Real, Robust>(oa, pair, 0, &s_state, s_sum, c);
         __syncthreads();
         if (threadIdx.x < 32) solve_pair<D>(sa, pair, s_state, s_sum, s_sc, &s_state);   // warp 0, all lanes
         __syncthreads();                                   // the new state is visible to the block

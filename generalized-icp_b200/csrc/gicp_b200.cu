@@ -23,6 +23,7 @@
 #include "raycast.cuh"
 #include "solve.cuh"
 #include "fused.cuh"
+#include "scale.cuh"
 #include "voxel.cuh"
 #include "plan.h"
 
@@ -160,11 +161,14 @@ struct gicpContext {
     gicpParams prm;
     int robust_kind = GICP_ROBUST_NONE;   // gicpSetRobustKernel
     double robust_scale = 0.0;
+    bool robust_adaptive = false;         // gicpSetRobustKernelAdaptive: c = max(robust_min_scale, robust_kappa * median)
+    double robust_kappa = 0.0, robust_min_scale = 0.0;
     CloudSet src, tgt;
     // [0]: every call on the caller's stream; [1]: the source side of gicpSetPair while it runs on the internal stream
     SetupScratch scr[2];
     VoxelScratch vox;
     DevBuf state, partial, partial2, red, T_dev, n_active, prev_match, slack, active_list;
+    DevBuf sel_keys, sel_hist, sel_arrived, sel_state, pair_scale;   // the adaptive scale's select (scale.cuh)
     static constexpr int NPOLL = 8;
     int* h_poll = nullptr;  // pinned [NPOLL]: progress polls in flight
     cudaEvent_t poll_ev[NPOLL] = {};
@@ -196,8 +200,8 @@ namespace {
 
 int ns_of(int dim) { return dim * (dim + 1) / 2; }
 
-const char* const kStageNames[GICP_N_STAGES] = {"gicp:grid_build", "gicp:knn_cov", "gicp:correspond", "gicp:accumulate",
-                                                 "gicp:solve"};
+const char* const kStageNames[GICP_N_STAGES_ALL] = {"gicp:grid_build", "gicp:knn_cov", "gicp:correspond",
+                                                     "gicp:accumulate", "gicp:solve", "gicp:scale_select"};
 
 struct ProfScope {
     gicpContext* h;
@@ -429,11 +433,6 @@ int launch_knn(gicpContext* h, CloudSet& cs, KnnPath path, int* d_idx, double* d
     return 0;
 }
 
-// per-warp TMA stages + the block's work list (one entry per point of the block)
-inline size_t obj_smem(int ppt) {
-    return 128 + (size_t)(OBJ_THREADS / 32) * OBJ_STAGE_BYTES + (size_t)OBJ_THREADS * ppt * sizeof(int);
-}
-
 template <int D, typename Real>
 int set_cloud(gicpContext* h, const Switches& sw, int which, const void* d_points, const int64_t* h_offsets,
               int n_clouds, cudaStream_t st, int scratch_slot) {
@@ -508,7 +507,7 @@ int objective_args(gicpContext* h, const Switches& sw, bool sliced, bool has_T0,
     const int np = S.plan.n_clouds;
     if (np != T.plan.n_clouds) return fail("source has %d clouds, target %d", np, T.plan.n_clouds);
     lp = plan_loop(sw, S.plan, sliced, Ranks{h->comm != nullptr, h->n_ranks, h->rank}, h->prof_on, has_T0,
-                   h->robust_kind != GICP_ROBUST_NONE);
+                   h->robust_kind != GICP_ROBUST_NONE, h->robust_adaptive);
     a.src_meta = S.nng().meta.as<CloudMeta>();
     a.src_spts = S.nng().spts.as<PRec<Real>>();
     a.src_cov = S.covnn().as<Real>();
@@ -537,6 +536,9 @@ int objective_args(gicpContext* h, const Switches& sw, bool sliced, bool has_T0,
     a.n_list = nullptr;
     a.robust_kind = h->robust_kind;
     a.robust_scale = h->robust_scale;
+    a.pair_scale = nullptr;
+    a.scale_kappa = h->robust_kappa;
+    a.scale_min = h->robust_min_scale;
     a.ppt = lp.acc_ppt;
     a.blocks_per_pair = lp.bpp;
     CU(h->partial.ensure((size_t)np * lp.bpp * Dim<D>::NRED * sizeof(double)));
@@ -576,12 +578,46 @@ int ensure_state(gicpContext* h, const double* h_T0, double* d_T, double* d_T_hi
     return 0;
 }
 
+// the multi-launch select's scratch: the histograms and arrival counters start at zero (the last block of every pair
+// leaves them so); a.pair_scale is where the accumulation reads the scale
+template <int D, typename Real>
+int prepare_select(gicpContext* h, ObjArgs<Real>& a, ScaleArgs& sc, cudaStream_t st) {
+    const int np = h->src.plan.n_clouds;
+    CU(h->sel_keys.ensure((size_t)std::max<int64_t>(h->src.plan.n_total, 1) * sizeof(unsigned long long)));
+    CU(h->sel_hist.ensure((size_t)np * SEL_BINS * sizeof(unsigned)));
+    CU(h->sel_arrived.ensure((size_t)np * sizeof(unsigned)));
+    CU(h->sel_state.ensure((size_t)np * sizeof(SelState)));
+    CU(h->pair_scale.ensure((size_t)np * sizeof(double)));
+    CU(cudaMemsetAsync(h->sel_hist.p, 0, (size_t)np * SEL_BINS * sizeof(unsigned), st));
+    CU(cudaMemsetAsync(h->sel_arrived.p, 0, (size_t)np * sizeof(unsigned), st));
+    sc.keys = h->sel_keys.as<unsigned long long>();
+    sc.hist = h->sel_hist.as<unsigned>();
+    sc.arrived = h->sel_arrived.as<unsigned>();
+    sc.sel = h->sel_state.as<SelState>();
+    sc.scale = h->pair_scale.as<double>();
+    a.pair_scale = sc.scale;
+    return 0;
+}
+
+// every pair's scale at its current matches: SEL_PASSES launches over the accumulation's blocks (a.ppt, bpp x gy)
+template <int D, typename Real>
+int launch_select(gicpContext* h, const ObjArgs<Real>& a, const ScaleArgs& sc, int bpp, int gy, cudaStream_t st) {
+    for (int pass = 0; pass < SEL_PASSES; ++pass)
+        scale_select_kernel<D, Real><<<dim3(bpp, gy), OBJ_THREADS, 0, st>>>(a, sc, pass);
+    h->launches += SEL_PASSES;
+    CU(cudaGetLastError());
+    return 0;
+}
+
 template <int D, typename Real>
 int do_register(gicpContext* h, const Switches& sw, const double* h_T0, double* d_T, int* d_n_outer, int* d_converged,
                 double* d_loss_hist, double* d_T_hist, int* d_inliers, cudaStream_t st) {
     ObjArgs<Real> oa;
     LoopPlan lp;
     if (objective_args<D, Real>(h, sw, true, h_T0 != nullptr, oa, lp)) return 1;
+    if (lp.adaptive && lp.sharded)
+        return fail("an adaptive robust scale needs every source point on one rank: sharded-source registration "
+                    "(gicpCommInit) takes a fixed scale (gicpSetRobustKernel) or none");
     const int np = h->src.plan.n_clouds;
     const int bpp = lp.bpp;
     h->last_stream = st;
@@ -618,8 +654,10 @@ int do_register(gicpContext* h, const Switches& sw, const double* h_T0, double* 
         oa.blocks_per_pair = 1;
         sa.blocks_per_pair = 1;
         sa.n_active = nullptr;   // nobody polls
-        const size_t smem = obj_smem(oa.ppt);
-        auto loop_kernel = lp.robust ? register_loop_kernel<D, Real, true> : register_loop_kernel<D, Real, false>;
+        // with an adaptive scale the select's keys (8 B per source point) follow the search's shared memory
+        const size_t smem = obj_smem(oa.ppt) + (lp.adaptive ? (size_t)OBJ_THREADS * oa.ppt * sizeof(unsigned long long) : 0);
+        auto loop_kernel = lp.adaptive ? register_loop_kernel<D, Real, true, true>
+                           : lp.robust ? register_loop_kernel<D, Real, true> : register_loop_kernel<D, Real, false>;
         CU(cudaFuncSetAttribute(loop_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         ProfScope prof(h, GICP_STAGE_CORRESPOND, st);
         loop_kernel<<<np, OBJ_THREADS, smem, st>>>(oa, sa, lp.self_init ? h->tgt.knn.bbox.as<double>() : nullptr);
@@ -633,6 +671,8 @@ int do_register(gicpContext* h, const Switches& sw, const double* h_T0, double* 
         sa.partial = h->partial2.as<double>();
         sa.blocks_per_pair = bpp2;
     }
+    ScaleArgs sc{};
+    if (lp.adaptive && prepare_select<D, Real>(h, oa, sc, st)) return 1;
     ObjArgs<Real> oc = oa;
     oc.ppt = lp.search_ppt;
     auto acc_kernel = lp.robust ? accumulate_kernel<D, Real, true> : accumulate_kernel<D, Real, false>;
@@ -675,6 +715,10 @@ int do_register(gicpContext* h, const Switches& sw, const double* h_T0, double* 
         {
             ProfScope prof(h, GICP_STAGE_CORRESPOND, st);
             correspond_kernel<D, Real><<<dim3(lp.search_bpp, gy), OBJ_THREADS, obj_smem(oc.ppt), st>>>(oc);
+        }
+        if (lp.adaptive) {
+            ProfScope prof(h, GICP_STAGE_SCALE_SELECT, st);
+            if (launch_select<D, Real>(h, oa, sc, bpp, gy, st)) return 1;
         }
         {
             ProfScope prof(h, GICP_STAGE_ACCUMULATE, st);
@@ -721,7 +765,7 @@ int do_register(gicpContext* h, const Switches& sw, const double* h_T0, double* 
 
 template <int D, typename Real>
 int do_stage(gicpContext* h, const Switches& sw, const double* h_T, int* d_idx, double* d_dist, double* d_W,
-             double* h_out, cudaStream_t st) {
+             double* h_out, double* h_scale, cudaStream_t st) {
     ObjArgs<Real> oa;
     LoopPlan lp;
     // stage entry points always cover the whole source (no slicing), so their outputs are complete
@@ -736,10 +780,14 @@ int do_stage(gicpContext* h, const Switches& sw, const double* h_T, int* d_idx, 
     oa.out_dist = d_dist;
     oa.out_W = d_W;
     oa.ignore_status = 1;
+    ScaleArgs sc{};
+    if (lp.adaptive && prepare_select<D, Real>(h, oa, sc, st)) return 1;
     correspond_kernel<D, Real><<<dim3(bpp, np), OBJ_THREADS, obj_smem(oa.ppt), st>>>(oa);
+    if (lp.adaptive && launch_select<D, Real>(h, oa, sc, bpp, np, st)) return 1;
     auto acc_kernel = lp.robust ? accumulate_kernel<D, Real, true> : accumulate_kernel<D, Real, false>;
     if (d_W || h_out) acc_kernel<<<dim3(bpp, np), OBJ_THREADS, 0, st>>>(oa);
     h->launches += 2;
+    if (h_scale) CU(cudaMemcpyAsync(h_scale, sc.scale, (size_t)np * sizeof(double), cudaMemcpyDeviceToHost, st));
     if (h_out) {
         SolveArgs sa;
         memset(&sa, 0, sizeof sa);
@@ -979,7 +1027,7 @@ int check(gicpHandle h) {
 extern "C" {
 
 const char* gicpGetLastError(void) { return g_last_error.c_str(); }
-int gicpVersion(void) { return 102; }
+int gicpVersion(void) { return 103; }
 
 int gicpDefaultParams(gicpParams* p) {
     if (!p) return fail("null params");
@@ -1029,7 +1077,7 @@ int gicpDestroy(gicpHandle h) {
     for (SetupScratch& sc : h->scr) sc.release();
     h->vox.release();
     DevBuf* bufs[] = {&h->state, &h->partial, &h->partial2, &h->red, &h->T_dev, &h->n_active, &h->prev_match, &h->slack,
-                      &h->active_list};
+                      &h->active_list, &h->sel_keys, &h->sel_hist, &h->sel_arrived, &h->sel_state, &h->pair_scale};
     for (DevBuf* b : bufs) b->release();
     if (h->h_poll) cudaFreeHost(h->h_poll);
     for (cudaEvent_t e : h->poll_ev) if (e) cudaEventDestroy(e);
@@ -1065,6 +1113,23 @@ int gicpSetRobustKernel(gicpHandle h, int kind, double scale) {
     // the set-up source and target stay valid: the weights enter only the accumulation of later calls
     h->robust_kind = kind;
     h->robust_scale = kind == GICP_ROBUST_NONE ? 0.0 : scale;
+    h->robust_adaptive = false;
+    return 0;
+}
+
+int gicpSetRobustKernelAdaptive(gicpHandle h, int kind, double kappa, double min_scale) {
+    if (check(h)) return 1;
+    if (kind < GICP_ROBUST_HUBER || kind > GICP_ROBUST_TUKEY)
+        return fail("adaptive robust kernel must be GICP_ROBUST_HUBER 1, CAUCHY 2 or TUKEY 3 (got %d; switch the kernel "
+                    "off with gicpSetRobustKernel(h, GICP_ROBUST_NONE, 0))", kind);
+    if (!(std::isfinite(kappa) && kappa > 0)) return fail("adaptive robust kappa must be finite and > 0 (got %g)", kappa);
+    if (!(std::isfinite(min_scale) && min_scale > 0))
+        return fail("adaptive robust min_scale must be finite and > 0 (got %g)", min_scale);
+    h->robust_kind = kind;
+    h->robust_scale = 0.0;
+    h->robust_adaptive = true;
+    h->robust_kappa = kappa;
+    h->robust_min_scale = min_scale;
     return 0;
 }
 
@@ -1142,14 +1207,27 @@ int gicpCovariances(gicpHandle h, int which, double* d_cov, void* stream) {
 
 int gicpCorrespond(gicpHandle h, const double* h_T, int32_t* d_idx, double* d_dist, double* d_W, void* stream) {
     if (check(h)) return 1;
-    return DISPATCH(h, do_stage, h, read_switches(), h_T, d_idx, d_dist, d_W, (double*)nullptr, (cudaStream_t)stream);
+    return DISPATCH(h, do_stage, h, read_switches(), h_T, d_idx, d_dist, d_W, (double*)nullptr, (double*)nullptr,
+                    (cudaStream_t)stream);
 }
 
 int gicpNormalEquations(gicpHandle h, const double* h_T, double* h_out, void* stream) {
     if (check(h)) return 1;
     if (!h_out) return fail("h_out is required");
     return DISPATCH(h, do_stage, h, read_switches(), h_T, (int*)nullptr, (double*)nullptr, (double*)nullptr, h_out,
-                    (cudaStream_t)stream);
+                    (double*)nullptr, (cudaStream_t)stream);
+}
+
+int gicpRobustScales(gicpHandle h, const double* h_T, double* h_scale, void* stream) {
+    if (check(h)) return 1;
+    if (!h_T || !h_scale) return fail("h_T and h_scale are required");
+    if (!h->src.ready || !h->tgt.ready) return fail("set source and target first");
+    if (!h->robust_adaptive) {   // a fixed scale, or 0 without a kernel: nothing to compute
+        for (int p = 0; p < h->src.plan.n_clouds; ++p) h_scale[p] = h->robust_scale;
+        return 0;
+    }
+    return DISPATCH(h, do_stage, h, read_switches(), h_T, (int*)nullptr, (double*)nullptr, (double*)nullptr,
+                    (double*)nullptr, h_scale, (cudaStream_t)stream);
 }
 
 int gicpSourceCovariancesAt(gicpHandle h, const double* h_T, int32_t n_T, double* d_out, void* stream) {
@@ -1226,11 +1304,14 @@ int gicpProfile(gicpHandle h, int enable) {
     return 0;
 }
 
-int gicpProfileRead(gicpHandle h, double ms_out[GICP_N_STAGES], int64_t count_out[GICP_N_STAGES]) {
+int gicpProfileReadStages(gicpHandle h, int32_t n_stages, double* ms_out, int64_t* count_out) {
     if (check(h)) return 1;
+    if (n_stages < 0 || n_stages > GICP_N_STAGES_ALL) return fail("n_stages must be in [0, %d]", GICP_N_STAGES_ALL);
+    if (n_stages && (!ms_out || !count_out)) return fail("ms_out and count_out are required");
     CU(cudaDeviceSynchronize());
-    for (int i = 0; i < GICP_N_STAGES; ++i) { ms_out[i] = 0.0; count_out[i] = 0; }
+    for (int i = 0; i < n_stages; ++i) { ms_out[i] = 0.0; count_out[i] = 0; }
     for (auto& r : h->prof_recs) {
+        if (r.stage >= n_stages) continue;
         float ms = 0.f;
         CU(cudaEventElapsedTime(&ms, r.a, r.b));
         ms_out[r.stage] += ms;
@@ -1239,6 +1320,10 @@ int gicpProfileRead(gicpHandle h, double ms_out[GICP_N_STAGES], int64_t count_ou
     h->prof_recs.clear();
     h->ev_used = 0;
     return 0;
+}
+
+int gicpProfileRead(gicpHandle h, double ms_out[GICP_N_STAGES], int64_t count_out[GICP_N_STAGES]) {
+    return gicpProfileReadStages(h, GICP_N_STAGES, ms_out, count_out);
 }
 
 }  // extern "C"

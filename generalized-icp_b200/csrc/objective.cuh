@@ -65,7 +65,18 @@ template <typename Real> struct ObjArgs {
     // robust kernel (gicpSetRobustKernel): read only by the Robust instantiations of accumulate_block
     int robust_kind;
     double robust_scale;
+    // adaptive scale (gicpSetRobustKernelAdaptive, scale.cuh): c_p = adaptive_scale(scale_kappa, median, scale_min).
+    // pair_scale: the scale of every pair at this iteration, written by the select of the multi-launch loop and read by
+    // the Robust accumulation instead of robust_scale when set
+    const double* pair_scale;
+    double scale_kappa, scale_min;
 };
+
+// dynamic shared memory of the search blocks: one mbarrier per warp (128 B), the warps' TMA stages, the work list of
+// ppt * OBJ_THREADS indices.  The fused loop with an adaptive scale appends the select's keys behind it.
+__host__ __device__ inline size_t obj_smem(int ppt) {
+    return 128 + (size_t)(OBJ_THREADS / 32) * OBJ_STAGE_BYTES + (size_t)OBJ_THREADS * ppt * sizeof(int);
+}
 
 // ---- the two fp32 bounds of the exact search (host-callable: tests/host_harness/bounds_host.cu checks them) ----
 // Filter: for a candidate c, a query p' (fp64) and its fp32 rounding f, d2_32 = |c - f|^2 in fp32 satisfies
@@ -109,6 +120,28 @@ __host__ __device__ __forceinline__ double robust_weight(int kind, double d, dou
         return u < 1.0 ? robust_mul(a, a) : 0.0;
     }
     return 1.0;
+}
+
+// ---- adaptive scale (semantics in include/gicp_b200.h): c = max(min_scale, kappa * m), kappa * m rounded once, and
+// min_scale when the two are equal.  m = 0 (no gated-in correspondence) gives min_scale.  Host-callable:
+// tests/host_harness/adaptive_host.cu checks it bit for bit against numpy. ----
+__host__ __device__ __forceinline__ double adaptive_scale(double kappa, double m, double min_scale) {
+    const double c = robust_mul(kappa, m);
+    return c > min_scale ? c : min_scale;
+}
+
+// p' = R p + t (gicp.py:119).  K3b and the scale select (scale.cuh) both form it here, so the distance the select
+// orders is bit for bit the one K3b gates on and weights with (the device contracts these products into FMAs).
+template <int D, typename Real>
+__device__ __forceinline__ void transform_point(const double (&R)[D][D], const double (&t)[D], const PRec<Real>& p,
+                                                double (&pp)[3]) {
+    const double px = (double)p.x, py = (double)p.y, pz = (double)p.z;
+#pragma unroll
+    for (int i = 0; i < D; ++i) {
+        double v = R[i][0] * px + R[i][1] * py + t[i];
+        if constexpr (D == 3) v += R[i][2] * pz;
+        pp[i] = v;
+    }
 }
 
 template <typename Real>
@@ -447,10 +480,11 @@ __global__ void __launch_bounds__(OBJ_THREADS, (D == 3 && sizeof(Real) == 4) ? 1
 // (a.partial[pair][bx]; the fused loop passes its shared-memory sum and state instead).
 // Robust: every gated-in correspondence is weighted by robust_weight(kind, d, c) - W, v = W e and e^T W e are scaled by
 // w before they enter the accumulators, so the reduced form is that of sum w_i r_i^T W_i r_i.  A compile-time switch:
-// the Robust = false instantiations are the unweighted kernels, instruction for instruction.
+// the Robust = false instantiations are the unweighted kernels, instruction for instruction.  `c` is the pair's scale
+// (the fixed robust_scale, or this iteration's adaptive one); Robust = false ignores it.
 template <int D, typename Real, bool Robust = false>
 __device__ __forceinline__ void accumulate_block(const ObjArgs<Real>& a, const int pair, const int bx,
-                                                 const PairState* stp, double* out) {
+                                                 const PairState* stp, double* out, const double c = 0.0) {
     using DD = Dim<D>;
     using AccT = Real;
     constexpr int NP = DD::NP, NS = DD::NS, NH = DD::NH, NQ = DD::NQ, NRED = DD::NRED;
@@ -553,17 +587,8 @@ __device__ __forceinline__ void accumulate_block(const ObjArgs<Real>& a, const i
             }
             continue;
         }
-        const PRec<Real> p = g.p;
         double pp[3] = {0.0, 0.0, 0.0};  // p' = R p + t (gicp.py:119)
-        {
-            const double px = (double)p.x, py = (double)p.y, pz = (double)p.z;
-#pragma unroll
-            for (int i = 0; i < D; ++i) {
-                double v = R[i][0] * px + R[i][1] * py + t[i];
-                if constexpr (D == 3) v += R[i][2] * pz;
-                pp[i] = v;
-            }
-        }
+        transform_point<D, Real>(R, t, g.p, pp);
         // ---- W = inv(C_tgt[j] + R C_src[i] R^T), e = q - p' ----
         const PRec<Real> q = g.q;
         double w_rob = 1.0;   // robust kernel weight at the current distance (Robust only)
@@ -575,7 +600,7 @@ __device__ __forceinline__ void accumulate_block(const ObjArgs<Real>& a, const i
                 }
                 continue;
             }
-            if constexpr (Robust) w_rob = robust_weight(a.robust_kind, sqrt(d2), a.robust_scale);
+            if constexpr (Robust) w_rob = robust_weight(a.robust_kind, sqrt(d2), c);
         }
         double Cs[NS], M[NS], W[NS], e[D], v[D];
         {
@@ -689,8 +714,10 @@ template <int D, typename Real, bool Robust = false>
 __global__ void __launch_bounds__(OBJ_THREADS, (sizeof(Real) == 8 && D == 3) ? 2 : 4) accumulate_kernel(const ObjArgs<Real> a) {
     const int pair = obj_pair_of_block(a);
     if (pair < 0) return;
+    double c = 0.0;
+    if constexpr (Robust) c = a.pair_scale ? a.pair_scale[pair] : a.robust_scale;
     accumulate_block<D, Real, Robust>(a, pair, blockIdx.x, a.state + pair,
-                              a.partial + ((size_t)pair * a.blocks_per_pair + blockIdx.x) * Dim<D>::NRED);
+                              a.partial + ((size_t)pair * a.blocks_per_pair + blockIdx.x) * Dim<D>::NRED, c);
 }
 
 }  // namespace gicp

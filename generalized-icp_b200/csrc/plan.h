@@ -176,16 +176,20 @@ struct LoopPlan {
     bool sharded = false;       // all-reduce between K3b and K4; blocking polls every poll_every-th iteration
     int poll_every = 1;
     bool robust = false;        // the accumulation weights the correspondences: the Robust instantiations of K3b / the fused loop
+    bool adaptive = false;      // ... at a scale selected every iteration: the select (scale.cuh) runs before K3b
 };
 
 // `sliced`: the registration loop of a sharded handle covers the rank's slice; the stage entry points always cover the
 // whole source, so that their outputs are complete.
 inline LoopPlan plan_loop(const Switches& sw, const SetupPlan& src, bool sliced, const Ranks& ranks, bool prof_on,
-                          bool has_T0, bool robust = false) {
+                          bool has_T0, bool robust = false, bool adaptive = false) {
     LoopPlan p;
     // a robust kernel other than GICP_ROBUST_NONE: every launch of the accumulation takes its Robust instantiation (the
     // unweighted kernels are left exactly as they are); nothing else of the loop changes
     p.robust = robust;
+    // an adaptive scale: the fused loop selects it inside its Robust instantiation, the multi-launch loop and the stage
+    // entry points launch scale_select_kernel between K3a and K3b
+    p.adaptive = robust && adaptive;
     const int np = src.n_clouds;
     p.sharded = ranks.on && np == 1;
     int span = src.max_n;

@@ -73,16 +73,39 @@ class GicpEngine:
             setattr(self.params, k, v)
         _lib.check(self.lib.gicpSetParams(self._h, C.byref(self.params)))
 
-    def set_robust_kernel(self, kind, scale=None):
+    def set_robust_kernel(self, kind, scale=None, *, adaptive=None, min_scale=None):
         """Weight every gated-in correspondence by a robust kernel of its distance d (IRLS, weights frozen at T_k):
         ``kind`` None (no weighting, the default), "huber", "cauchy" or "tukey"; ``scale`` c > 0 in the units of the
-        points, like max_distance_correspondence.  Semantics in include/gicp_b200.h.  Applies to every later
-        register / correspond / normal_equations; the set-up clouds are kept."""
+        points, like max_distance_correspondence.  Or, instead of ``scale``, ``adaptive`` = kappa with ``min_scale``:
+        every pair's scale is set at every outer iteration to max(min_scale, kappa * median of its gated-in
+        distances).  Semantics in include/gicp_b200.h.  Applies to every later register / correspond /
+        normal_equations / robust_scales; the set-up clouds are kept."""
         if kind not in ROBUST_KINDS:
             raise ValueError(f"unknown robust kernel {kind!r}; expected one of None, 'huber', 'cauchy', 'tukey'")
-        if kind is not None and scale is None:
-            raise ValueError(f"the {kind} kernel needs a scale")
-        _lib.check(self.lib.gicpSetRobustKernel(self._h, ROBUST_KINDS[kind], 0.0 if scale is None else float(scale)))
+        if kind is None:
+            if adaptive is not None or min_scale is not None:
+                raise ValueError("adaptive / min_scale need a kernel")
+            _lib.check(self.lib.gicpSetRobustKernel(self._h, 0, 0.0))
+            return
+        if (scale is None) == (adaptive is None):
+            raise ValueError(f"the {kind} kernel needs exactly one of a scale and adaptive=kappa")
+        if adaptive is None:
+            if min_scale is not None:
+                raise ValueError("min_scale goes with adaptive=kappa")
+            _lib.check(self.lib.gicpSetRobustKernel(self._h, ROBUST_KINDS[kind], float(scale)))
+            return
+        if min_scale is None:
+            raise ValueError("an adaptive scale needs min_scale")
+        _lib.check(self.lib.gicpSetRobustKernelAdaptive(self._h, ROBUST_KINDS[kind], float(adaptive), float(min_scale)))
+
+    def robust_scales(self, T):
+        """(P,) float64 numpy: every pair's robust scale at the transforms T (P, d+1, d+1) - the adaptive scale at the
+        correspondences of T, a fixed scale as set, 0 without a kernel."""
+        n_pairs = self._n[SOURCE][1]
+        T, tp = self._T_arg(T)
+        out = np.zeros((n_pairs,), dtype=np.float64)
+        _lib.check(self.lib.gicpRobustScales(self._h, tp, out.ctypes.data_as(C.POINTER(C.c_double)), self._stream()))
+        return out
 
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
@@ -409,12 +432,14 @@ class GicpEngine:
     def profile(self, enable=True):
         _lib.check(self.lib.gicpProfile(self._h, int(bool(enable))))
 
-    def profile_read(self):
-        """{stage: (milliseconds, timed sections)} since the last read (device-synchronising)."""
-        ms = (C.c_double * 5)()
-        cnt = (C.c_int64 * 5)()
-        _lib.check(self.lib.gicpProfileRead(self._h, ms, cnt))
-        return {s: (float(ms[i]), int(cnt[i])) for i, s in enumerate(self.STAGES)}
+    def profile_read(self, scale_select=False):
+        """{stage: (milliseconds, timed sections)} since the last read (device-synchronising).  With
+        ``scale_select`` also "scale_select": the adaptive robust scale's select of the multi-launch loop."""
+        names = self.STAGES + (("scale_select",) if scale_select else ())
+        ms = (C.c_double * len(names))()
+        cnt = (C.c_int64 * len(names))()
+        _lib.check(self.lib.gicpProfileReadStages(self._h, len(names), ms, cnt))
+        return {s: (float(ms[i]), int(cnt[i])) for i, s in enumerate(names)}
 
     @property
     def launch_count(self):

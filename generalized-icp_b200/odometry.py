@@ -27,14 +27,16 @@ class ScanOdometry:
     """Feed scans one at a time; every scan after the first yields the 3x3 transform of the pair
     (previous -> current) and the integrated pose."""
 
-    def __init__(self, start_pose=(50.0, 400.0, 0.0), storage="f64", robust_kernel=None, robust_scale=None, **params):
-        """``robust_kernel`` / ``robust_scale``: see GicpEngine.set_robust_kernel (scale in pixels)."""
+    def __init__(self, start_pose=(50.0, 400.0, 0.0), storage="f64", robust_kernel=None, robust_scale=None,
+                 robust_adaptive=None, robust_min_scale=None, **params):
+        """``robust_kernel`` / ``robust_scale``, or ``robust_adaptive`` (kappa) / ``robust_min_scale``: see
+        GicpEngine.set_robust_kernel (scales in pixels)."""
         from .engine import GicpEngine
         self.eng = GicpEngine(2, storage)
         p = dict(max_distance_nearest_neighbors=200.0, tolerance=1.0)   # robot-visualization.py:160-161
         p.update(params)
         self.eng.set_params(**p)
-        self.eng.set_robust_kernel(robust_kernel, robust_scale)
+        self.eng.set_robust_kernel(robust_kernel, robust_scale, adaptive=robust_adaptive, min_scale=robust_min_scale)
         self.pose = tuple(start_pose)
         self.poses = [self.pose]
         self.transforms = []

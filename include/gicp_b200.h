@@ -94,6 +94,18 @@ int gicpSetParams(gicpHandle h, const gicpParams* p);
  * source and target, so one set-up can be registered with and without a kernel.                                  */
 enum { GICP_ROBUST_NONE = 0, GICP_ROBUST_HUBER = 1, GICP_ROBUST_CAUCHY = 2, GICP_ROBUST_TUKEY = 3 };
 int gicpSetRobustKernel(gicpHandle h, int kind, double scale);
+/* Adaptive scale: the kernel `kind` (HUBER, CAUCHY or TUKEY; NONE is rejected - switch the kernel off with
+ * gicpSetRobustKernel(h, GICP_ROBUST_NONE, 0)) with a scale set per pair p at every outer iteration k:
+ *   c_{p,k} = max(min_scale, kappa * m_{p,k})
+ * m_{p,k} is the lower median of the distances d_i of pair p's gated-in correspondences at T_k: the element of rank
+ * floor((n-1)/2) in ascending order, ties included, of the very float64 d_i the gate tests and the weight takes (not
+ * recomputed another way).  kappa * m is rounded once; the max takes min_scale when the two are equal; with no gated-in
+ * correspondence c = min_scale.  The weights are then robust_weight(kind, d_i, c_{p,k}), and everything above holds
+ * unchanged: weights frozen with the matches, min_loss the weighted minimum, every gated-in match an inlier.
+ * kappa and min_scale must be finite and > 0.  Like gicpSetRobustKernel it keeps the set-up clouds; a later
+ * gicpSetRobustKernel returns the handle to a fixed scale or to no kernel.  gicpRegister with a sharded source
+ * (gicpCommInit, one pair) and an adaptive scale fails: the median would need every rank's distances.            */
+int gicpSetRobustKernelAdaptive(gicpHandle h, int kind, double kappa, double min_scale);
 
 /* ---- clouds: grid build (replaces KDTree(points), gicp.py:21,127) and per-point
  *      covariances (replaces compute_covariance_matrix, gicp.py:19-35) ---------------------
@@ -153,6 +165,10 @@ int gicpCorrespond(gicpHandle h, const double* h_T, int32_t* d_idx, double* d_di
  *   [26..27] mu.  With a robust kernel every term is that of w_i W_i (the weighted inner problem); the count is
  *   still the gated-in count.  Synchronises the stream.                                                          */
 int gicpNormalEquations(gicpHandle h, const double* h_T, double* h_out, void* stream);
+/* the robust scale of every pair at the given transforms: h_scale (n_clouds) f64 - with an adaptive scale c_p at the
+ * correspondences of h_T (those gicpCorrespond reports; its d_W and gicpNormalEquations use the same c_p), with a fixed
+ * scale that scale, without a kernel 0.  Synchronises the stream.                                                   */
+int gicpRobustScales(gicpHandle h, const double* h_T, double* h_scale, void* stream);
 
 /* source covariances as the reference recomputes them on the transformed cloud every outer
  * iteration (gicp.py:120): C_src,k = R_k C_src,0 R_k^T.  h_T (n_T, n_clouds, dim+1, dim+1);
@@ -204,11 +220,16 @@ int64_t gicpLaunchCount(gicpHandle h);
 
 /* per-stage device timing with CUDA events on the launching stream (bench.py's roofline leg).
  * gicpProfile(h, 1) starts recording; gicpProfileRead synchronises the device, returns the summed
- * milliseconds and the number of timed launches/sections per stage, and clears the records.   */
+ * milliseconds and the number of timed launches/sections per stage, and clears the records.
+ * gicpProfileReadStages does the same for the first n_stages (<= GICP_N_STAGES_ALL) stages; stage
+ * GICP_STAGE_SCALE_SELECT is the adaptive robust scale's select of the multi-launch loop (one section per outer
+ * iteration), which gicpProfileRead leaves out.                                                                   */
 enum { GICP_STAGE_GRID = 0, GICP_STAGE_KNN_COV = 1, GICP_STAGE_CORRESPOND = 2, GICP_STAGE_ACCUMULATE = 3,
        GICP_STAGE_SOLVE = 4, GICP_N_STAGES = 5 };
+enum { GICP_STAGE_SCALE_SELECT = 5, GICP_N_STAGES_ALL = 6 };
 int gicpProfile(gicpHandle h, int enable);
 int gicpProfileRead(gicpHandle h, double ms_out[GICP_N_STAGES], int64_t count_out[GICP_N_STAGES]);
+int gicpProfileReadStages(gicpHandle h, int32_t n_stages, double* ms_out, int64_t* count_out);
 
 #ifdef __cplusplus
 }

@@ -17,7 +17,7 @@ want = {
     "correspond_kernel_3_float": "_ZN4gicp17correspond_kernelILi3EfEEvNS_7ObjArgsIT0_EE",
     "accumulate_kernel_3_float": "_ZN4gicp17accumulate_kernelILi3EfLb0EEEvNS_7ObjArgsIT0_EE",
     "solve_kernel_3": "_ZN4gicp12solve_kernelILi3EEEvNS_9SolveArgsE",
-    "register_loop_kernel_2_double": "_ZN4gicp20register_loop_kernelILi2EdLb0EEEvNS_7ObjArgsIT0_EENS_9SolveArgsEPKd",
+    "register_loop_kernel_2_double": "_ZN4gicp20register_loop_kernelILi2EdLb0ELb0EEEvNS_7ObjArgsIT0_EENS_9SolveArgsEPKd",
 }
 rows = []
 for part in re.split(r"(?=\n\s+Function : )", txt):
