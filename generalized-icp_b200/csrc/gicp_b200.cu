@@ -1027,7 +1027,7 @@ int check(gicpHandle h) {
 extern "C" {
 
 const char* gicpGetLastError(void) { return g_last_error.c_str(); }
-int gicpVersion(void) { return 103; }
+int gicpVersion(void) { return 104; }
 
 int gicpDefaultParams(gicpParams* p) {
     if (!p) return fail("null params");
@@ -1097,6 +1097,11 @@ int gicpSetParams(gicpHandle h, const gicpParams* p) {
     if (!(p->max_distance_nearest_neighbors > 0)) return fail("max_distance_nearest_neighbors must be > 0");
     if (!(p->max_distance_correspondence > 0)) return fail("max_distance_correspondence must be > 0");
     if (p->covariance_model < 0 || p->covariance_model > 2) return fail("covariance_model must be 0, 1 or 2");
+    // a zero lambda_normal makes C_B + R C_A R^T singular wherever two normals align, a negative one makes W indefinite
+    if (!(std::isfinite(p->lambda_tangent) && p->lambda_tangent > 0))
+        return fail("lambda_tangent must be finite and > 0 (got %g)", p->lambda_tangent);
+    if (!(std::isfinite(p->lambda_normal) && p->lambda_normal > 0))
+        return fail("lambda_normal must be finite and > 0 (got %g)", p->lambda_normal);
     h->prm = *p;
     if (h->prm.inner_max_iterations <= 0) h->prm.inner_max_iterations = 50;
     h->src.ready = false;

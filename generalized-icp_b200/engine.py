@@ -67,11 +67,15 @@ class GicpEngine:
 
     # ---- parameters (names of gicp.py:78 plus the engine's own) ----
     def set_params(self, **kw):
+        """Set the named fields (include/gicp_b200.h, gicpParams).  A rejected set leaves the engine's parameters and
+        set-up clouds as they were."""
+        p = GicpParams.from_buffer_copy(self.params)
         for k, v in kw.items():
-            if not hasattr(self.params, k):
+            if not hasattr(p, k):
                 raise TypeError(f"unknown parameter {k!r}")
-            setattr(self.params, k, v)
-        _lib.check(self.lib.gicpSetParams(self._h, C.byref(self.params)))
+            setattr(p, k, v)
+        _lib.check(self.lib.gicpSetParams(self._h, C.byref(p)))
+        self.params = p
 
     def set_robust_kernel(self, kind, scale=None, *, adaptive=None, min_scale=None):
         """Weight every gated-in correspondence by a robust kernel of its distance d (IRLS, weights frozen at T_k):

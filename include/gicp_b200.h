@@ -50,9 +50,10 @@ typedef struct gicpParams {
     double  tolerance;            /* gicp.py:78 tolerance = 1e-6 : stop when |last_loss - loss| < tol     */
     double  max_distance_correspondence;     /* gicp.py:78 (=150): reject when d > d_max (strict, :136)   */
     double  max_distance_nearest_neighbors;  /* gicp.py:78 (=50):  k-NN bound, exclusive (:24)            */
-    double  lambda_tangent;       /* gicp.py:5   epsilon = 100                                            */
-    double  lambda_normal;        /* gicp.py:11  epsilon * 0.1 = 10                                       */
-    int32_t inner_max_iterations; /* LM iterations of the on-device inner solve (replaces fmin_cg, :152)  */
+    double  lambda_tangent;       /* gicp.py:5   epsilon = 100; finite and > 0                            */
+    double  lambda_normal;        /* gicp.py:11  epsilon * 0.1 = 10; finite and > 0                       */
+    int32_t inner_max_iterations; /* LM iterations of the on-device inner solve (replaces fmin_cg, :152);
+                                   * <= 0 means the default, 50                                            */
     int32_t covariance_model;     /* ICP family through the same kernels (presentation/main.typ:446-462):
                                    * 0 plane-to-plane = GICP (the reference), 1 point-to-point (C_A = 0, C_B = I),
                                    * 2 point-to-plane (C_A = 0, C_B = the target's surface-aligned covariance)    */
@@ -72,6 +73,14 @@ const char* gicpGetLastError(void);
 int gicpVersion(void);
 /* fills *p with the reference's defaults (gicp.py:78, :5, :11, :24) */
 int gicpDefaultParams(gicpParams* p);
+/* Validates every field and fails, naming the field, on: k outside [1, 32]; max_iterations < 1; a distance that is not
+ * > 0; covariance_model outside {0, 1, 2}; lambda_tangent or lambda_normal not finite and > 0 (0 makes C_B + R C_A R^T
+ * singular where two normals align, a negative value makes W indefinite).  A failed call changes nothing: the handle
+ * keeps its previous parameters and its set-up clouds.  inner_max_iterations <= 0 is taken as 50.  A successful call
+ * discards the set-up source and target (set them again before gicpRegister).
+ * The covariances are stored in the handle's storage type, so with f32 storage every entry is rounded once: the
+ * smallest eigenvalue of a stored C can move by about 3 * 2^-24 * max(lambda) (1.8e-7 relative), which a ratio
+ * lambda_min / lambda_max near 1e-7 no longer resolves.                                                             */
 int gicpSetParams(gicpHandle h, const gicpParams* p);
 
 /* ---- robust kernels (M-estimators) on the correspondence distance ----------------------------------------------

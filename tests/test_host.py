@@ -219,10 +219,21 @@ def test_covariance_tail_host(solve_host):
     compiled for the host) against numpy's eigh on the formula of gicp.py:11-16 / the oracle's
     covariances_from_neighbors: generic, nearly planar, nearly collinear and badly scaled scatter matrices; non-finite
     input gives the identity (gicp.py:31-32)."""
+    _check_covariance_tail(solve_host, 100.0, 10.0)
+
+
+# (lambda_tangent, lambda_normal) away from the defaults: the regularisation of fast_gicp / small_gicp, equal lambdas
+# (C = lam I exactly), an inverted pair and a ratio of 1e-7
+@pytest.mark.parametrize("lam_t,lam_n", [(1.0, 1e-3), (1.0, 1.0), (10.0, 100.0), (1e4, 1e-3)])
+def test_covariance_tail_host_lambdas(solve_host, lam_t, lam_n):
+    """The same checks with other regularisations."""
+    _check_covariance_tail(solve_host, lam_t, lam_n)
+
+
+def _check_covariance_tail(solve_host, lam_t, lam_n):
     import ctypes
     dp = ctypes.POINTER(ctypes.c_double)
     rng = np.random.default_rng(11)
-    lam_t, lam_n = 100.0, 10.0
 
     def want(S, dim):
         evals, evecs = np.linalg.eigh(S)
@@ -258,8 +269,11 @@ def test_covariance_tail_host(solve_host):
             S = (Q * ev) @ Q.T * scale
             S = 0.5 * (S + S.T)
             gap = (ev[-1] - ev[-2]) if dim == 2 else (ev[1] - ev[0])
-            tol = 1e-9 * (lam_t - lam_n) / max(gap / ev[-1], 1e-12) * 10
-            assert np.abs(got(S, dim) - want(S, dim)).max() <= max(tol, 1e-9), (dim, case, ev)
+            tol = 1e-9 * abs(lam_t - lam_n) / max(gap / ev[-1], 1e-12) * 10
+            C = got(S, dim)
+            assert np.abs(C - want(S, dim)).max() <= max(tol, 1e-9), (dim, case, ev)
+            if lam_t == lam_n:
+                assert np.array_equal(C, lam_t * np.eye(dim))
         bad = np.full((dim, dim), np.nan)
         assert np.array_equal(got(bad, dim), np.eye(dim))
 

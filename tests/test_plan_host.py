@@ -327,3 +327,27 @@ def test_read_switches(plan, monkeypatch):
         got = read()
         for k in names:
             assert got[k] == (int(want != 0) if k in flags else want), (k, value)
+
+
+def test_param_table_reaches_its_plans(plan):
+    """The fixed tables of tests/test_gpu_params.py reach the plans they are meant to: every cell row its cell edges,
+    shared or unshared grid, budget and grid build on each input of part D; every K2 row of part A its k-NN path."""
+    from test_gpu_params import CELL_DMAX, CELL_R, CELL_ROWS, CELL_SIZES, K2_PATHS, K2_RADIUS
+    for case, (ns, nt) in CELL_SIZES.items():
+        f32 = case == "3d_f32"
+        k = 6 if case == "2d_f64" else 20
+        for name, knobs, h_knn, h_nn, shared, budget, single_small in CELL_ROWS:
+            prm = dict(k=k, max_distance_nearest_neighbors=CELL_R, max_distance_correspondence=CELL_DMAX, **knobs)
+            for which, sizes in ((SOURCE, ns), (TARGET, nt)):
+                got = _check_setup(plan, prm, {}, _offs(sizes), which=which, f32=f32)
+                assert (got["knn_cell"], got["nn_cell"], got["shared"]) == (h_knn, h_nn, shared), (case, name)
+                if budget is not None:
+                    assert got["budget"] == budget, (case, name)
+                assert got["single_block"] == int(single_small and max(sizes) <= SMALL_GRID_MAX), (case, name)
+    for name, n, ks, storages in K2_PATHS:
+        for dim, k in ks.items():
+            for storage in storages:
+                prm = dict(k=k, max_distance_nearest_neighbors=K2_RADIUS[dim], max_distance_correspondence=3.0)
+                got = _check_setup(plan, prm, {}, _offs([n]), f32=storage == "f32")
+                want = {"brute": BRUTE, "general_latency": GENERAL, "hist": HIST_GENERAL}.get(name, GENERAL)
+                assert got["knn"] == want, (name, dim, storage, got["knn"])
