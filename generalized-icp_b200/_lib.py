@@ -13,7 +13,7 @@ SYMBOLS = [
     "gicpSetTarget", "gicpSetSource", "gicpSetPair", "gicpPromoteTargetToSource", "gicpRegister", "gicpKnn", "gicpCovariances", "gicpCorrespond",
     "gicpNormalEquations", "gicpSourceCovariancesAt", "gicpCommGetUniqueId", "gicpCommInit", "gicpCommDestroy",
     "gicpLaunchCount", "gicpProfile", "gicpProfileRead", "gicpRayCast", "gicpVoxelDownsample",
-    "gicpSetRobustKernel", "gicpSetRobustKernelAdaptive", "gicpRobustScales", "gicpProfileReadStages",
+    "gicpSetRobustKernel", "gicpSetRobustKernelAdaptive", "gicpRobustScales", "gicpProfileReadStages", "gicpEvaluate",
 ]
 
 
@@ -56,6 +56,7 @@ def load():
     lib.gicpSetRobustKernel.argtypes = [vp, C.c_int, C.c_double]
     lib.gicpSetRobustKernelAdaptive.argtypes = [vp, C.c_int, C.c_double, C.c_double]
     lib.gicpRobustScales.argtypes = [vp, dp, dp, vp]
+    lib.gicpEvaluate.argtypes = [vp, vp, vp, vp, vp, vp]
     for f in (lib.gicpSetTarget, lib.gicpSetSource):
         f.argtypes = [vp, vp, C.POINTER(i64), i32, vp]
     lib.gicpSetPair.argtypes = [vp, vp, C.POINTER(i64), vp, C.POINTER(i64), i32, vp]

@@ -53,7 +53,7 @@ def gicp_extended(source_points, target_points, max_iterations=100, tolerance=1e
                   max_distance_correspondence=150, max_distance_nearest_neighbors=50, k=6,
                   lambda_tangent=100.0, lambda_normal=10.0, storage="f64", full_history=True, covariance_model=0,
                   voxel_size=None, robust_kernel=None, robust_scale=None, robust_adaptive=None, robust_min_scale=None,
-                  **engine_params):
+                  evaluate=False, **engine_params):
     """The registration with everything the engine knows (SURVEY.md discrepancy 3: the reference
     computes ``min_loss`` and drops it; here the loss history, inlier counts and the fitness-like
     final loss are returned as well).  Returns a dict.  With ``voxel_size`` both clouds are first
@@ -61,7 +61,10 @@ def gicp_extended(source_points, target_points, max_iterations=100, tolerance=1e
     ``target_points`` (float64) and every per-point output refers to them.  ``robust_kernel`` (None, "huber",
     "cauchy" or "tukey") with ``robust_scale`` weights every correspondence by a robust kernel of its distance
     (GicpEngine.set_robust_kernel); ``hw_src`` / ``hw_tgt`` then rank the weighted matrices w W.  ``robust_adaptive``
-    (kappa) with ``robust_min_scale`` replaces ``robust_scale`` by the adaptive scale of every outer iteration."""
+    (kappa) with ``robust_min_scale`` replaces ``robust_scale`` by the adaptive scale of every outer iteration.
+    With ``evaluate`` the dict also holds the registration's quality at the returned T (GicpEngine.evaluate):
+    ``n_inliers``, ``fitness``, ``inlier_rmse``, ``information`` (H, rotation first) and ``gradient`` (-2 b, the
+    gradient of the objective under a left perturbation of T)."""
     import torch
 
     src = np.asarray(source_points)
@@ -90,6 +93,11 @@ def gicp_extended(source_points, target_points, max_iterations=100, tolerance=1e
                tgt_cov=r["tgt_cov"], src_cov0=r["src_cov0"])
     if voxel_size is not None:
         out["source_points"], out["target_points"] = src, tgt
+    if evaluate:
+        q = eng.evaluate(out["T"].reshape(1, dim + 1, dim + 1))
+        out["n_inliers"] = int(q.n_inliers[0])
+        out["fitness"], out["inlier_rmse"] = float(q.fitness[0]), float(q.inlier_rmse[0])
+        out["information"], out["gradient"] = q.H[0].cpu().numpy(), (-2.0 * q.b[0]).cpu().numpy()
     if full_history:
         covs = eng.source_covariances_at(T_hist[:n_outer].reshape(n_outer, 1, dim + 1, dim + 1)).cpu().numpy()
         out["all_src_cov"] = [covs[i] for i in range(n_outer)]

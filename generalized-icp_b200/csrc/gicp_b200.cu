@@ -25,6 +25,7 @@
 #include "fused.cuh"
 #include "scale.cuh"
 #include "voxel.cuh"
+#include "quality.cuh"
 #include "plan.h"
 
 using namespace gicp;
@@ -169,6 +170,7 @@ struct gicpContext {
     VoxelScratch vox;
     DevBuf state, partial, partial2, red, T_dev, n_active, prev_match, slack, active_list;
     DevBuf sel_keys, sel_hist, sel_arrived, sel_state, pair_scale;   // the adaptive scale's select (scale.cuh)
+    DevBuf eval_idx, eval_dist;   // gicpEvaluate: the correspondences at the evaluated transforms (input order)
     static constexpr int NPOLL = 8;
     int* h_poll = nullptr;  // pinned [NPOLL]: progress polls in flight
     cudaEvent_t poll_ev[NPOLL] = {};
@@ -763,32 +765,27 @@ int do_register(gicpContext* h, const Switches& sw, const double* h_T0, double* 
     return 0;
 }
 
+// One stage pass at the DEVICE transforms d_T, enqueued on `st` without a synchronisation: the correspondences
+// (d_idx / d_dist in input order), with an adaptive scale every pair's scale (sc.scale), the weight matrices d_W and,
+// with `fold`, every pair's reduced form (+mu) in h->red.  `oa` / `lp` come from objective_args.
 template <int D, typename Real>
-int do_stage(gicpContext* h, const Switches& sw, const double* h_T, int* d_idx, double* d_dist, double* d_W,
-             double* h_out, double* h_scale, cudaStream_t st) {
-    ObjArgs<Real> oa;
-    LoopPlan lp;
-    // stage entry points always cover the whole source (no slicing), so their outputs are complete
-    if (objective_args<D, Real>(h, sw, false, true, oa, lp)) return 1;
+int stage_pass(gicpContext* h, ObjArgs<Real>& oa, const LoopPlan& lp, const double* d_T, int* d_idx, double* d_dist,
+               double* d_W, bool fold, ScaleArgs& sc, cudaStream_t st) {
     const int np = h->src.plan.n_clouds;
     const int bpp = lp.bpp;
-    if (!h_T) return fail("h_T is required");
     if (ensure_state<D, Real>(h, nullptr, nullptr, nullptr, nullptr, nullptr, st)) return 1;
-    if (upload_T(h, h_T, (size_t)np * (D + 1) * (D + 1) * sizeof(double), st)) return 1;
-    oa.T_override = h->T_dev.as<double>();
+    oa.T_override = d_T;
     oa.out_idx = d_idx;
     oa.out_dist = d_dist;
     oa.out_W = d_W;
     oa.ignore_status = 1;
-    ScaleArgs sc{};
     if (lp.adaptive && prepare_select<D, Real>(h, oa, sc, st)) return 1;
     correspond_kernel<D, Real><<<dim3(bpp, np), OBJ_THREADS, obj_smem(oa.ppt), st>>>(oa);
     if (lp.adaptive && launch_select<D, Real>(h, oa, sc, bpp, np, st)) return 1;
     auto acc_kernel = lp.robust ? accumulate_kernel<D, Real, true> : accumulate_kernel<D, Real, false>;
-    if (d_W || h_out) acc_kernel<<<dim3(bpp, np), OBJ_THREADS, 0, st>>>(oa);
+    if (d_W || fold) acc_kernel<<<dim3(bpp, np), OBJ_THREADS, 0, st>>>(oa);
     h->launches += 2;
-    if (h_scale) CU(cudaMemcpyAsync(h_scale, sc.scale, (size_t)np * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (h_out) {
+    if (fold) {
         SolveArgs sa;
         memset(&sa, 0, sizeof sa);
         sa.partial = h->partial.as<double>();
@@ -798,9 +795,49 @@ int do_stage(gicpContext* h, const Switches& sw, const double* h_T, int* d_idx, 
         sa.state = h->state.as<PairState>();
         solve_kernel<D><<<(np + SOLVE_WARPS - 1) / SOLVE_WARPS, SOLVE_WARPS * 32, 0, st>>>(sa);
         h->launches += 1;
-        CU(cudaMemcpyAsync(h_out, h->red.p, (size_t)np * Dim<D>::NRED * sizeof(double), cudaMemcpyDeviceToHost, st));
     }
+    CU(cudaGetLastError());
+    return 0;
+}
+
+template <int D, typename Real>
+int do_stage(gicpContext* h, const Switches& sw, const double* h_T, int* d_idx, double* d_dist, double* d_W,
+             double* h_out, double* h_scale, cudaStream_t st) {
+    ObjArgs<Real> oa;
+    LoopPlan lp;
+    // stage entry points always cover the whole source (no slicing), so their outputs are complete
+    if (objective_args<D, Real>(h, sw, false, true, oa, lp)) return 1;
+    const int np = h->src.plan.n_clouds;
+    if (!h_T) return fail("h_T is required");
+    if (upload_T(h, h_T, (size_t)np * (D + 1) * (D + 1) * sizeof(double), st)) return 1;
+    ScaleArgs sc{};
+    if (stage_pass<D, Real>(h, oa, lp, h->T_dev.as<double>(), d_idx, d_dist, d_W, h_out != nullptr, sc, st)) return 1;
+    if (h_scale) CU(cudaMemcpyAsync(h_scale, sc.scale, (size_t)np * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (h_out)
+        CU(cudaMemcpyAsync(h_out, h->red.p, (size_t)np * Dim<D>::NRED * sizeof(double), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
+    CU(cudaGetLastError());
+    return 0;
+}
+
+// gicpEvaluate: a stage pass at the caller's device transforms into the handle's own correspondence scratch, then one
+// quality_kernel block per pair.  Stream-ordered, no synchronisation.
+template <int D, typename Real>
+int do_evaluate(gicpContext* h, const Switches& sw, const double* d_T, double* d_quality, double* d_H, double* d_b,
+                cudaStream_t st) {
+    ObjArgs<Real> oa;
+    LoopPlan lp;
+    if (objective_args<D, Real>(h, sw, false, true, oa, lp)) return 1;
+    const int np = h->src.plan.n_clouds;
+    const size_t n_src = (size_t)std::max<int64_t>(h->src.plan.n_total, 1);
+    CU(h->eval_idx.ensure(n_src * sizeof(int)));
+    CU(h->eval_dist.ensure(n_src * sizeof(double)));
+    ScaleArgs sc{};
+    if (stage_pass<D, Real>(h, oa, lp, d_T, h->eval_idx.as<int>(), h->eval_dist.as<double>(), nullptr, true, sc, st))
+        return 1;
+    quality_kernel<D><<<np, QUALITY_THREADS, 0, st>>>(h->red.as<double>(), oa.src_meta, h->eval_idx.as<int>(),
+                                                      h->eval_dist.as<double>(), d_quality, d_H, d_b);
+    h->launches += 1;
     CU(cudaGetLastError());
     return 0;
 }
@@ -1027,7 +1064,7 @@ int check(gicpHandle h) {
 extern "C" {
 
 const char* gicpGetLastError(void) { return g_last_error.c_str(); }
-int gicpVersion(void) { return 104; }
+int gicpVersion(void) { return 105; }
 
 int gicpDefaultParams(gicpParams* p) {
     if (!p) return fail("null params");
@@ -1077,7 +1114,8 @@ int gicpDestroy(gicpHandle h) {
     for (SetupScratch& sc : h->scr) sc.release();
     h->vox.release();
     DevBuf* bufs[] = {&h->state, &h->partial, &h->partial2, &h->red, &h->T_dev, &h->n_active, &h->prev_match, &h->slack,
-                      &h->active_list, &h->sel_keys, &h->sel_hist, &h->sel_arrived, &h->sel_state, &h->pair_scale};
+                      &h->active_list, &h->sel_keys, &h->sel_hist, &h->sel_arrived, &h->sel_state, &h->pair_scale,
+                      &h->eval_idx, &h->eval_dist};
     for (DevBuf* b : bufs) b->release();
     if (h->h_poll) cudaFreeHost(h->h_poll);
     for (cudaEvent_t e : h->poll_ev) if (e) cudaEventDestroy(e);
@@ -1233,6 +1271,12 @@ int gicpRobustScales(gicpHandle h, const double* h_T, double* h_scale, void* str
     }
     return DISPATCH(h, do_stage, h, read_switches(), h_T, (int*)nullptr, (double*)nullptr, (double*)nullptr,
                     (double*)nullptr, h_scale, (cudaStream_t)stream);
+}
+
+int gicpEvaluate(gicpHandle h, const double* d_T, double* d_quality, double* d_H, double* d_b, void* stream) {
+    if (check(h)) return 1;
+    if (!d_T) return fail("d_T is required");
+    return DISPATCH(h, do_evaluate, h, read_switches(), d_T, d_quality, d_H, d_b, (cudaStream_t)stream);
 }
 
 int gicpSourceCovariancesAt(gicpHandle h, const double* h_T, int32_t n_T, double* d_out, void* stream) {

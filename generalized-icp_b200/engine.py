@@ -31,6 +31,18 @@ class RegistrationResult:
     inliers: torch.Tensor | None     # (P, max_it) i32
 
 
+@dataclass
+class RegistrationQuality:
+    """Device-resident outputs of :meth:`GicpEngine.evaluate` at given transforms T (one row per pair; definitions in
+    include/gicp_b200.h, gicpEvaluate).  xi = (rotation, translation), left perturbation T(xi) = Exp(xi) T."""
+    n_inliers: torch.Tensor     # (P,) i32    gated-in correspondences at T
+    fitness: torch.Tensor       # (P,) f64    n_inliers / source size (0 for an empty source)
+    inlier_rmse: torch.Tensor   # (P,) f64    sqrt(mean d_i^2) over the inliers, Euclidean (0 without inliers)
+    loss: torch.Tensor          # (P,) f64    sum w_i e_i^T W_i e_i (gicpNormalEquations' loss slot)
+    H: torch.Tensor             # (P, 6, 6) / (P, 3, 3) f64  sum J^T w W J: information matrix, rotation first
+    b: torch.Tensor             # (P, 6) / (P, 3) f64        sum J^T w W e: GN step H^-1 b, gradient -2 b
+
+
 def _ptr(t):
     return C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p(0)
 
@@ -183,6 +195,24 @@ class GicpEngine:
                                          _ptr(inl), self._stream()))
         return RegistrationResult(T, n_outer, conv, loss, T_hist, inl)
 
+    def evaluate(self, T) -> RegistrationQuality:
+        """Quality of every pair at the transforms T (P, d+1, d+1) through gicpEvaluate: inlier count, fitness, inlier
+        RMSE, loss, information matrix H and vector b, as device tensors.  Stream-ordered, no synchronisation: a
+        contiguous float64 T on the engine's device (e.g. ``register().T``) is read in place, anything else is copied
+        there first."""
+        n_pairs = self._n[SOURCE][1]
+        d1, npar = self.dim + 1, 6 if self.dim == 3 else 3
+        if not (isinstance(T, torch.Tensor) and T.device == self.device and T.dtype == torch.float64
+                and T.is_contiguous()):
+            T = torch.as_tensor(np.asarray(T, dtype=np.float64) if not isinstance(T, torch.Tensor) else T)
+            T = T.to(device=self.device, dtype=torch.float64).contiguous()
+        T = T.reshape(n_pairs, d1, d1)
+        q = torch.empty((n_pairs, 4), dtype=torch.float64, device=self.device)
+        H = torch.empty((n_pairs, npar, npar), dtype=torch.float64, device=self.device)
+        b = torch.empty((n_pairs, npar), dtype=torch.float64, device=self.device)
+        _lib.check(self.lib.gicpEvaluate(self._h, _ptr(T), _ptr(q), _ptr(H), _ptr(b), self._stream()))
+        return RegistrationQuality(q[:, 0].to(torch.int32), q[:, 1], q[:, 2], q[:, 3], H, b)
+
     def register_pair_host(self, src, tgt):
         """One pair given as HOST arrays, everything the reference's 7-tuple needs back as host numpy arrays, with
         the fewest host<->device round trips: both clouds travel in ONE staged copy (pinned, cached), every output
@@ -251,11 +281,13 @@ class GicpEngine:
                     src_cov0=hd[offs[3]:offs[4]].reshape(n_s, d, d), tgt_cov=hd[offs[4]:offs[5]].reshape(n_t, d, d),
                     n_outer=n_outer, converged_at=conv, inliers=hi[2:2 + mi][:n_outer])
 
-    def register_next_scan_host(self, scan, have_previous):
+    def register_next_scan_host(self, scan, have_previous, evaluate=False):
         """Scan sequences with HOST scans (robot-visualization.py:246-252): the previous target is promoted to the
         source (grids + covariances reused), `scan` becomes the target, the pair is registered.  One staged upload, one
         read-back (T, n_outer, converged_at), no per-call allocations; the first scan of a sequence
-        (`have_previous=False`) is only set up.  Returns None or dict(T, n_outer, converged_at)."""
+        (`have_previous=False`) is only set up.  Returns None or dict(T, n_outer, converged_at).  With ``evaluate``
+        gicpEvaluate runs on the device T before the read-back and the dict also holds ``quality``: dict(n_inliers,
+        fitness, inlier_rmse, loss, H, b) at T, brought back by the same copy."""
         d, d1 = self.dim, self.dim + 1
         np_dt = np.float64 if self.storage == "f64" else np.float32
         scan = np.ascontiguousarray(scan, dtype=np_dt)
@@ -282,14 +314,29 @@ class GicpEngine:
         _lib.check(self.lib.gicpSetTarget(self._h, vp(self._sc_dev[slot].data_ptr()), (C.c_int64 * 2)(0, n), 1, st))
         if not have_previous:
             return None
-        dp = self._sc_out_dev.data_ptr()
+        # outputs: [T | n_outer, converged_at (i32)] and, with evaluate, [quality (4) | H | b] behind them
+        npar = 6 if d == 3 else 3
+        if evaluate and getattr(self, "_sc_q_dev", None) is None:
+            n_q = d1 * d1 + 1 + 4 + npar * npar + npar
+            self._sc_q_dev = torch.empty((n_q,), dtype=torch.float64, device=self.device)
+            self._sc_q_host = torch.empty((n_q,), dtype=torch.float64, pin_memory=True)
+        out_dev, out_host = (self._sc_q_dev, self._sc_q_host) if evaluate else (self._sc_out_dev, self._sc_out_host)
+        dp = out_dev.data_ptr()
         ip = dp + 8 * d1 * d1
         _lib.check(self.lib.gicpRegister(self._h, None, vp(dp), vp(ip), vp(ip + 4), None, None, None, st))
-        self._sc_out_host.copy_(self._sc_out_dev, non_blocking=True)
+        if evaluate:
+            qp = ip + 8
+            _lib.check(self.lib.gicpEvaluate(self._h, vp(dp), vp(qp), vp(qp + 32), vp(qp + 32 + 8 * npar * npar), st))
+        out_host.copy_(out_dev, non_blocking=True)
         torch.cuda.current_stream(self.device).synchronize()
-        hd = self._sc_out_host.numpy().copy()
-        hi = hd[d1 * d1:].view(np.int32)
-        return dict(T=hd[:d1 * d1].reshape(d1, d1), n_outer=int(hi[0]), converged_at=int(hi[1]))
+        hd = out_host.numpy().copy()
+        hi = hd[d1 * d1:d1 * d1 + 1].view(np.int32)
+        r = dict(T=hd[:d1 * d1].reshape(d1, d1), n_outer=int(hi[0]), converged_at=int(hi[1]))
+        if evaluate:
+            q = hd[d1 * d1 + 1:]
+            r["quality"] = dict(n_inliers=int(q[0]), fitness=float(q[1]), inlier_rmse=float(q[2]), loss=float(q[3]),
+                                H=q[4:4 + npar * npar].reshape(npar, npar), b=q[4 + npar * npar:])
+        return r
 
     def register_host_batch(self, h_src, h_tgt, offsets, chunk_pairs=1024, history=False):
         """Batches that live in (pinned) HOST memory: pairs are registered in chunks, and the host->device

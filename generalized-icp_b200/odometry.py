@@ -28,9 +28,11 @@ class ScanOdometry:
     (previous -> current) and the integrated pose."""
 
     def __init__(self, start_pose=(50.0, 400.0, 0.0), storage="f64", robust_kernel=None, robust_scale=None,
-                 robust_adaptive=None, robust_min_scale=None, **params):
+                 robust_adaptive=None, robust_min_scale=None, evaluate=False, **params):
         """``robust_kernel`` / ``robust_scale``, or ``robust_adaptive`` (kappa) / ``robust_min_scale``: see
-        GicpEngine.set_robust_kernel (scales in pixels)."""
+        GicpEngine.set_robust_kernel (scales in pixels).  With ``evaluate`` every step's quality at its transform
+        (dict(n_inliers, fitness, inlier_rmse, loss, H, b), GicpEngine.evaluate) is appended to ``self.quality``; it
+        comes back with the transform in one copy."""
         from .engine import GicpEngine
         self.eng = GicpEngine(2, storage)
         p = dict(max_distance_nearest_neighbors=200.0, tolerance=1.0)   # robot-visualization.py:160-161
@@ -41,16 +43,20 @@ class ScanOdometry:
         self.poses = [self.pose]
         self.transforms = []
         self.iterations = []
+        self.evaluate = bool(evaluate)
+        self.quality = []
         self._have = False
 
     def push(self, scan):
-        r = self.eng.register_next_scan_host(np.asarray(scan, dtype=np.float64), self._have)
+        r = self.eng.register_next_scan_host(np.asarray(scan, dtype=np.float64), self._have, evaluate=self.evaluate)
         if not self._have:
             self._have = True
             return None
         T = r["T"]
         self.transforms.append(T)
         self.iterations.append(r["n_outer"])
+        if self.evaluate:
+            self.quality.append(r["quality"])
         self.pose = integrate_pose(self.pose, T)
         self.poses.append(self.pose)
         return T

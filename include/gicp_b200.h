@@ -179,6 +179,37 @@ int gicpNormalEquations(gicpHandle h, const double* h_T, double* h_out, void* st
  * scale that scale, without a kernel 0.  Synchronises the stream.                                                   */
 int gicpRobustScales(gicpHandle h, const double* h_T, double* h_scale, void* stream);
 
+/* ---- registration quality at device-resident transforms (Open3D evaluate_registration +
+ *      get_information_matrix_from_point_clouds, fast_gicp getFitnessScore / getFinalHessian) ------------------------
+ * d_T (n_clouds, dim+1, dim+1) f64 in DEVICE memory, e.g. the d_T gicpRegister just wrote.  Stream-ordered: the call
+ * does not synchronise, so it may directly follow the fused loop's immediately-returning gicpRegister; d_T must stay
+ * valid until the work completes.  Any output may be NULL.
+ * For every pair the correspondences at T are those gicpCorrespond reports at the same T (same search, same strict
+ * d_max gate, same W_i = inv(C_tgt + R C_src R^T)); with a robust kernel w_i is the weight at the same distance, with an
+ * adaptive scale the scale is the pair's scale at T (gicpRobustScales).  n = the gated-in count, p'_i = R p_i + t,
+ * e_i = q_i - p'_i, d_i = |e_i| (the float64 Euclidean distance the gate tests).
+ *  d_quality (n_clouds, GICP_NQUALITY) f64:
+ *    [0] n                     = count(d_idx >= 0) of gicpCorrespond = the count slot of gicpNormalEquations (a Tukey
+ *                                weight of 0 still counts)
+ *    [1] fitness               = n / source cloud size; 0 for an empty source (Open3D's definition)
+ *    [2] inlier RMSE           = sqrt(sum d_i^2 / n), Euclidean and unweighted in every covariance_model and with any
+ *                                kernel; 0 when n = 0
+ *    [3] loss                  = sum w_i e_i^T W_i e_i = slot [72] (dim 3) / [24] (dim 2) of gicpNormalEquations
+ *  d_H (n_clouds, 6, 6) in dim 3, (n_clouds, 3, 3) in dim 2;  d_b (n_clouds, 6) / (n_clouds, 3):
+ *    left perturbation about the target frame's origin, rotation first: T(xi) = Exp(xi) T, xi = (w, v) in dim 3
+ *    (to first order T(xi) p = p' + w x p' + v), xi = (theta, vx, vy) in dim 2.  J_i = d(T(xi) p_i)/d xi at 0:
+ *    [ -[p'_i]x | I3 ] in dim 3, [ (-p'_iy, p'_ix)^T | I2 ] in dim 2.
+ *      H = sum J_i^T (w_i W_i) J_i   the Gauss-Newton Hessian of the objective (the Fisher information of xi when the
+ *                                    W_i are inverse residual covariances)
+ *      b = sum J_i^T w_i W_i e_i     the GN step is xi = H^-1 b, and the gradient of the objective at xi = 0 is -2 b
+ *    The ordering and perturbation are those of Open3D's information matrix: with covariance_model 1 and no kernel,
+ *    H is Open3D's sum G^T G over the same correspondences with G evaluated at p'_i (Open3D evaluates it at the
+ *    matched target point q_i, which differs by the residual).  GICP's lambda-regularised covariances leave the
+ *    absolute scale of H uncalibrated; its eigenstructure (degenerate directions: corridors, planes) is meaningful as
+ *    is.  A pair with n = 0 gets zeros in every output.                                                           */
+#define GICP_NQUALITY 4
+int gicpEvaluate(gicpHandle h, const double* d_T, double* d_quality, double* d_H, double* d_b, void* stream);
+
 /* source covariances as the reference recomputes them on the transformed cloud every outer
  * iteration (gicp.py:120): C_src,k = R_k C_src,0 R_k^T.  h_T (n_T, n_clouds, dim+1, dim+1);
  * d_out (n_T, n_src_total, dim, dim) f64 in input order.  all_source_cov_matrices, gicp.py:121. */
