@@ -66,7 +66,7 @@ template <int N> __host__ __device__ inline bool spd_solve(double A[N][N], doubl
     return true;
 }
 
-__device__ inline void rodrigues(const double w[3], double R[3][3]) {
+__host__ __device__ inline void rodrigues(const double w[3], double R[3][3]) {
     const double th2 = w[0] * w[0] + w[1] * w[1] + w[2] * w[2];
     double A, B;  // R = I + A K + B K^2
     if (th2 < 1e-16) { A = 1.0 - th2 / 6.0; B = 0.5 - th2 / 24.0; }
@@ -82,8 +82,8 @@ __device__ inline void rodrigues(const double w[3], double R[3][3]) {
 
 // dR for the candidate step; dim 2 keeps the accumulated angle so dR is always an exact rot(dtheta)
 template <int D>
-__device__ inline void compose_rotation(const double* step_rot, const double dR[D][D], double dtheta,
-                                        double dRn[D][D], double* dtheta_n) {
+__host__ __device__ inline void compose_rotation(const double* step_rot, const double dR[D][D], double dtheta,
+                                                 double dRn[D][D], double* dtheta_n) {
     if constexpr (D == 2) {
         const double th = dtheta + step_rot[0];
         double s, c;
@@ -99,8 +99,8 @@ __device__ inline void compose_rotation(const double* step_rot, const double dR[
     }
 }
 
-// (spd_solve, dense_H_entry and inner_solve_2d are __host__ __device__: tests/test_host.py compiles them for the host
-// and checks the minimiser on the reference's own inner problems without a GPU.)
+// (spd_solve, dense_H_entry, inner_solve_2d and inner_solve_warp are __host__ __device__: tests/test_host.py and
+// tests/test_solve3_host.py compile them for the host and check the minimiser without a GPU.)
 // 2-D, ONE LANE: Levenberg-Marquardt on the reduced form  f(Z) = c - 2<G,Z> + <Z, H Z>,  Z = [dt | dR - I]  (the same
 // iteration as the warp-cooperative 3-D version below: same damping, acceptance and stop rules), evaluated on the
 // projection of the form onto the four numbers Z depends on.  With dR = rot(th):
@@ -192,6 +192,19 @@ __host__ __device__ inline void inner_solve_2d(const double* Hq, const double* G
     *fmin = f;
 }
 
+// Host builds of inner_solve_warp (tests/host_harness/solve3_host.cu) run its 32 lanes as 32 threads; the harness
+// defines this hook as a barrier over them.  The library never calls the solver on the host.
+extern void (*g_host_warp_sync)();
+
+// the warp's barrier between the solver's phases: __syncwarp() on the device, the harness's barrier on the host
+__host__ __device__ __forceinline__ void solve_warp_sync() {
+#ifdef __CUDA_ARCH__
+    __syncwarp();
+#else
+    g_host_warp_sync();
+#endif
+}
+
 // Minimise the reduced form  f(Z) = c - 2<G,Z> + <Z, H Z>,  Z = [dt | dR - I]  (flat index c * NP + a), over
 // (dt, dR in SO(D)) by Levenberg-Marquardt.  WARP-COOPERATIVE: all 32 lanes of one warp call this with the same
 // arguments; the matrix-vector products, tangents and normal equations are spread over the lanes (one row or one
@@ -199,7 +212,7 @@ __host__ __device__ inline void inner_solve_2d(const double* Hq, const double* G
 // version of the same algorithm executed ~17 k instructions per LM iteration in 3-D (it was the slowest kernel of a
 // small registration: 37 us per launch); this one executes ~1.3 k.  Results in sc.dR, sc.dt, sc.dtheta, sc.f.
 template <int D>
-__device__ void inner_solve_warp(SolveScratch<D>& sc, const double* G, double c0, int max_it, int lane) {
+__host__ __device__ void inner_solve_warp(SolveScratch<D>& sc, const double* G, double c0, int max_it, int lane) {
     using SS = SolveScratch<D>;
     constexpr int NP = SS::NP, DN = SS::DN, NPAR = SS::NPAR;
     if (lane == 0) {
@@ -212,7 +225,7 @@ __device__ void inner_solve_warp(SolveScratch<D>& sc, const double* G, double c0
         sc.lam = 1e-9;
     }
     if (lane < DN) sc.Z[lane] = 0.0;
-    __syncwarp();
+    solve_warp_sync();
     for (int it = 0; it < max_it; ++it) {
         // gradient wrt Z: Gam = 2 (H Z - G)
         if (lane < DN) {
@@ -239,7 +252,7 @@ __device__ void inner_solve_warp(SolveScratch<D>& sc, const double* G, double c0
             }
             sc.dZ[x][e] = v;
         }
-        __syncwarp();
+        solve_warp_sync();
         for (int q = lane; q < NPAR * DN; q += 32) {
             const int x = q / DN, r = q % DN;
             const double* row = sc.Hd + r * DN;
@@ -247,7 +260,7 @@ __device__ void inner_solve_warp(SolveScratch<D>& sc, const double* G, double c0
             for (int e = 0; e < DN; ++e) s += row[e] * sc.dZ[x][e];
             sc.HdZ[x][r] = s;
         }
-        __syncwarp();
+        solve_warp_sync();
         if (lane < NPAR) {
             double s = 0.0;
             for (int e = 0; e < DN; ++e) s += sc.Gam[e] * sc.dZ[lane][e];
@@ -261,7 +274,7 @@ __device__ void inner_solve_warp(SolveScratch<D>& sc, const double* G, double c0
                 sc.A[x][y] = sc.A[y][x] = 2.0 * s;
             }
         }
-        __syncwarp();
+        solve_warp_sync();
         if (lane == 0) {
             double f = sc.f, lam = sc.lam;
             double gmax = 0.0;
@@ -346,7 +359,7 @@ __device__ void inner_solve_warp(SolveScratch<D>& sc, const double* G, double c0
             sc.lam = lam;
             sc.go = go ? 1 : 0;
         }
-        __syncwarp();
+        solve_warp_sync();
         if (!sc.go) break;
     }
 }

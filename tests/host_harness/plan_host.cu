@@ -70,6 +70,20 @@ void gicp_test_plan_loop(const gicpParams* prm, const FlatSwitches* sw, const in
                     p.fused_ppt, p.presum, p.bpp2, p.active_list, p.sharded, p.poll_every};
 }
 
+// the loop a registration of one batch takes with a robust kernel (robust) and an adaptive scale (adaptive):
+// out = {fused, robust, adaptive, presum}
+void gicp_test_plan_loop_kernel(const gicpParams* prm, const FlatSwitches* sw, const int64_t* off, int n_clouds,
+                                int robust, int adaptive, int* out) {
+    const Switches s = unflat(*sw);
+    const Ranks ranks{false, 1, 0};
+    const SetupPlan src = plan_setup(*prm, s, off, n_clouds, GICP_SOURCE, false, ranks);
+    const LoopPlan p = plan_loop(s, src, true, ranks, false, false, robust != 0, adaptive != 0);
+    out[0] = p.fused;
+    out[1] = p.robust;
+    out[2] = p.adaptive;
+    out[3] = p.presum;
+}
+
 int gicp_test_pair_overlap(const FlatSwitches* sw, int comm, int prof_on, long long n_target, long long n_source) {
     return pair_overlap(unflat(*sw), Ranks{comm != 0, 1, 0}, prof_on != 0, n_target, n_source);
 }

@@ -147,11 +147,12 @@ class Batch:
         return r
 
 
-def check_loop(b, r, T0=None, nonconvex=()):
+def check_loop(b, r, T0=None, nonconvex=(), weight=None):
     """Part 1: every executed iteration k of every pair against the exact 1-NN of the source under T_hist[k]:
     the stage search's indices, the loop's inlier count, and the loop's min_loss as the frozen objective of the exact
     matches at T_hist[k + 1] (at the converged iteration, where T is not updated: the frozen problem's minimum, found
-    by the oracle's Newton solver; for the pairs in `nonconvex` the device only has to do at least as well)."""
+    by the oracle's Newton solver; for the pairs in `nonconvex` the device only has to do at least as well).
+    With a robust kernel, weight(p, k, d) gives the weights of pair p's gated-in matches at distances d."""
     from oracle import gicp_oracle as O
     d, d1 = b.dim, b.dim + 1
     d_max = float(b.params.get("max_distance_correspondence", 150.0))
@@ -194,6 +195,8 @@ def check_loop(b, r, T0=None, nonconvex=()):
             Rk = Tk[:d, :d]
             q = t[m[g]]
             W = np.linalg.inv(Rk @ cs[b.off_s[p]:b.off_s[p + 1]][g] @ Rk.T + ct[b.off_t[p]:b.off_t[p + 1]][m[g]])
+            if weight is not None:
+                W = weight(p, k, np.sqrt(np.sum((q - pp[g]) ** 2, axis=1)))[:, None, None] * W
             if conv[p] == k:
                 _, want_loss, _, _ = O.inner_newton(_offset(Tk, d), s[g], q, W)
                 tol = max(rel, 1e-8)

@@ -62,6 +62,7 @@ def plan(tmp_path_factory):
     lib.gicp_test_plan_loop.argtypes = [P, S, I64] + [C.c_int] * 7 + [C.POINTER(Loop)]
     lib.gicp_test_pair_overlap.argtypes = [S, C.c_int, C.c_int, C.c_longlong, C.c_longlong]
     lib.gicp_test_read_switches.argtypes = [S]
+    lib.gicp_test_plan_loop_kernel.argtypes = [P, S, I64, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int)]
 
     def params(**kw):
         p = GicpParams(k=6, max_iterations=100, tolerance=1e-6, max_distance_correspondence=150.0,
@@ -90,7 +91,14 @@ def plan(tmp_path_factory):
     def overlap(sw, comm, prof_on, n_t, n_s):
         return lib.gicp_test_pair_overlap(C.byref(Switches(**{**DEFAULT_SW, **sw})), comm, prof_on, n_t, n_s)
 
-    lib.setup, lib.loop, lib.overlap = setup, loop, overlap
+    def loop_kernel(prm, sw, off, robust, adaptive):
+        off = np.ascontiguousarray(off, dtype=np.int64)
+        out = (C.c_int * 4)()
+        lib.gicp_test_plan_loop_kernel(C.byref(params(**prm)), C.byref(Switches(**{**DEFAULT_SW, **sw})),
+                                       off.ctypes.data_as(I64), len(off) - 1, int(robust), int(adaptive), out)
+        return dict(zip(("fused", "robust", "adaptive", "presum"), out))
+
+    lib.setup, lib.loop, lib.overlap, lib.loop_kernel = setup, loop, overlap, loop_kernel
     return lib
 
 
@@ -351,3 +359,34 @@ def test_param_table_reaches_its_plans(plan):
                 got = _check_setup(plan, prm, {}, _offs([n]), f32=storage == "f32")
                 want = {"brute": BRUTE, "general_latency": GENERAL, "hist": HIST_GENERAL}.get(name, GENERAL)
                 assert got["knn"] == want, (name, dim, storage, got["knn"])
+
+
+def test_inner_minimum_rows_reach_their_loops(plan):
+    """Every row of tests/test_gpu_inner_minimum.py reaches the loop it names: fused or multi-launch, plain, robust or
+    adaptive, so the GPU table runs every instantiation of register_loop_kernel, accumulate_kernel, scale_select_kernel
+    and solve_kernel it claims.  The 20 k-point row also folds its block partials first (presum_kernel)."""
+    from test_gpu_inner_minimum import INPUTS, ROWS
+    seen = set()
+    for name, inp, storage, loop, kernel, model in ROWS:
+        dim, n, params = INPUTS[inp]
+        prm = {k: v for k, v in params.items() if k != "max_iterations"}
+        sw = {"fused_loop": int(loop == "fused")} if n <= 2048 else {}
+        got = plan.loop_kernel(dict(prm, covariance_model=model), sw, _offs([n]), kernel is not None,
+                               kernel is not None and kernel[0] == "adaptive")
+        want_kind = "plain" if kernel is None else kernel[0]
+        assert got["fused"] == int(loop == "fused"), name
+        assert got["robust"] == int(kernel is not None) and got["adaptive"] == int(want_kind == "adaptive"), name
+        if inp == "big":
+            assert got["presum"] == 1, name
+        seen.add((dim, storage, loop, want_kind))
+        seen.add((dim, storage, model))
+    for dim, storage in itertools.product((2, 3), ("f32", "f64")):
+        for kind in ("plain", "fixed", "adaptive"):                       # register_loop_kernel<D, Real, robust, adaptive>
+            assert (dim, storage, "fused", kind) in seen, (dim, storage, kind)
+        for kind in ("plain", "adaptive"):                                # accumulate_kernel, scale_select_kernel
+            assert (dim, storage, "multi", kind) in seen, (dim, storage, kind)
+        for model in (0, 1, 2):
+            assert (dim, storage, model) in seen, (dim, storage, model)
+    for dim, model in itertools.product((2, 3), (1, 2)):                  # models 1 and 2 in both loops
+        for loop in ("fused", "multi"):
+            assert any(INPUTS[r[1]][0] == dim and r[3] == loop and r[5] == model for r in ROWS), (dim, model, loop)
