@@ -26,7 +26,7 @@ namespace gicp {
 constexpr int OBJ_THREADS = 128;
 constexpr int OBJ_STAGE_BYTES = 2048;  // per warp (small: occupancy matters more than window size here)
 constexpr int OBJ_GROUP_REACH = 4;
-constexpr int OBJ_MAX_PPT = 16;   // search blocks and the fused loop; the accumulation alone runs up to twice that
+constexpr int OBJ_MAX_PPT = 16;   // loop search, fused loop; K3b and the stage entry points' K3a (at K3b's ppt) run up to twice that
 
 template <typename Real> struct ObjArgs {
     const CloudMeta* src_meta;

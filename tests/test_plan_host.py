@@ -390,3 +390,34 @@ def test_inner_minimum_rows_reach_their_loops(plan):
     for dim, model in itertools.product((2, 3), (1, 2)):                  # models 1 and 2 in both loops
         for loop in ("fused", "multi"):
             assert any(INPUTS[r[1]][0] == dim and r[3] == loop and r[5] == model for r in ROWS), (dim, model, loop)
+
+
+def test_block_shape_rows_reach_their_plans(plan):
+    """Every row of tests/test_gpu_block_shapes.py reaches the accumulation and search blocks, the partial fold and the
+    active list it names, and the p-rows (whose full pairs are the same tensors) all get the same cell budget, so their
+    grids and the exact search's results are the same in every row.  The benchmark's default batch and the config-5
+    pair reach acc_ppt 32 as the table says."""
+    from test_gpu_block_shapes import BENCH_PAIRS, BENCH_PLAN, CONFIG5_N, CONFIG5_PLAN, P_ROWS, P3, P2, ROWS, row_sizes
+    keys = ("acc_ppt", "search_ppt", "search_bpp", "bpp", "presum", "bpp2", "active_list")
+    budgets = set()
+    cases = [(name, row_sizes(name), ROWS[name][5], P2 if ROWS[name][0] == 2 else P3) for name in ROWS]
+    cases += [("bench", [(32768, 32768)] * BENCH_PAIRS, BENCH_PLAN, P3), ("config5", [(CONFIG5_N, CONFIG5_N)],
+                                                                          CONFIG5_PLAN, P3)]
+    for name, sizes, want, prm in cases:
+        prm = {k: v for k, v in prm.items() if k not in ("max_iterations", "tolerance")}
+        off_s, off_t = _offs([s for s, _ in sizes]), _offs([t for _, t in sizes])
+        got = plan.loop(prm, {}, off_s)
+        assert got == parent_loop(prm, {}, off_s), name
+        assert tuple(got[k] for k in keys) == want, (name, {k: got[k] for k in keys})
+        assert got["fused"] == 0, name
+        if name in P_ROWS:
+            for off in (off_s, off_t):
+                budgets.add(_check_setup(plan, prm, {}, off)["budget"])
+    assert len(budgets) == 1, budgets
+    # fillers end on every kind of block edge below max_n: warp and thread-run edges, the row's block edge, one point
+    # short of the pair's last block
+    for name in ("p8", "p17", "p32"):
+        ppt, bpp = ROWS[name][5][0], ROWS[name][5][3]
+        n_src = {s for s, _ in row_sizes(name)}
+        want = {0, 1, 127, 128, 129, ppt * 128 - 1, ppt * 128, ppt * 128 + 1, bpp * ppt * 128 - 1}
+        assert {n for n in want if n < 32768} <= n_src, name
