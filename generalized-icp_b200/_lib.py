@@ -14,6 +14,7 @@ SYMBOLS = [
     "gicpNormalEquations", "gicpSourceCovariancesAt", "gicpCommGetUniqueId", "gicpCommInit", "gicpCommDestroy",
     "gicpLaunchCount", "gicpProfile", "gicpProfileRead", "gicpRayCast", "gicpVoxelDownsample",
     "gicpSetRobustKernel", "gicpSetRobustKernelAdaptive", "gicpRobustScales", "gicpProfileReadStages", "gicpEvaluate",
+    "gicpSetVoxelized",
 ]
 
 
@@ -74,6 +75,7 @@ def load():
     lib.gicpLaunchCount.restype = i64
     lib.gicpRayCast.argtypes = [C.c_int, vp, i32, i32, vp, i32, vp, i32, C.c_double, vp, vp, vp, vp]
     lib.gicpVoxelDownsample.argtypes = [vp, vp, C.POINTER(i64), i32, C.c_double, i32, vp, C.POINTER(i64), vp, vp, vp]
+    lib.gicpSetVoxelized.argtypes = [vp, C.c_int, vp, C.POINTER(i64), i32, C.c_double, i32, vp, C.POINTER(i64), vp]
     lib.gicpProfile.argtypes = [vp, C.c_int]
     lib.gicpProfileRead.argtypes = [vp, dp, C.POINTER(i64)]
     lib.gicpProfileReadStages.argtypes = [vp, i32, dp, C.POINTER(i64)]

@@ -53,7 +53,7 @@ def gicp_extended(source_points, target_points, max_iterations=100, tolerance=1e
                   max_distance_correspondence=150, max_distance_nearest_neighbors=50, k=6,
                   lambda_tangent=100.0, lambda_normal=10.0, storage="f64", full_history=True, covariance_model=0,
                   voxel_size=None, robust_kernel=None, robust_scale=None, robust_adaptive=None, robust_min_scale=None,
-                  evaluate=False, **engine_params):
+                  evaluate=False, voxel_distributions=False, voxel_min_points=1, **engine_params):
     """The registration with everything the engine knows (SURVEY.md discrepancy 3: the reference
     computes ``min_loss`` and drops it; here the loss history, inlier counts and the fitness-like
     final loss are returned as well).  Returns a dict.  With ``voxel_size`` both clouds are first
@@ -64,7 +64,11 @@ def gicp_extended(source_points, target_points, max_iterations=100, tolerance=1e
     (kappa) with ``robust_min_scale`` replaces ``robust_scale`` by the adaptive scale of every outer iteration.
     With ``evaluate`` the dict also holds the registration's quality at the returned T (GicpEngine.evaluate):
     ``n_inliers``, ``fitness``, ``inlier_rmse``, ``information`` (H, rotation first) and ``gradient`` (-2 b, the
-    gradient of the objective under a left perturbation of T)."""
+    gradient of the objective under a left perturbation of T).  With ``voxel_distributions`` (and ``voxel_size``) both
+    sides are instead set up as voxel distributions (GicpEngine.set_source_voxelized / set_target_voxelized: the
+    voxels with >= ``voxel_min_points`` points, each carrying the covariance of its own points, no k-NN search);
+    ``source_points`` / ``target_points``, ``src_cov0`` / ``tgt_cov`` and every per-point output then refer to the
+    voxels."""
     import torch
 
     src = np.asarray(source_points)
@@ -75,7 +79,10 @@ def gicp_extended(source_points, target_points, max_iterations=100, tolerance=1e
     if dim not in (2, 3) or tgt.shape[1] != dim:
         raise ValueError(f"expected (N, 2) or (N, 3) clouds of equal dimension, got {src.shape} and {tgt.shape}")
     eng = _engine(dim, storage)
-    if voxel_size is not None:
+    if voxel_distributions and voxel_size is None:
+        raise ValueError("voxel_distributions needs voxel_size")
+    raw_src, raw_tgt = src, tgt
+    if voxel_size is not None and not voxel_distributions:
         src = _downsample(eng, src[:, :dim], voxel_size, 1)
         tgt = _downsample(eng, tgt[:, :dim], voxel_size, 1)
     eng.set_params(k=k, max_iterations=int(max_iterations), tolerance=float(tolerance),
@@ -84,7 +91,11 @@ def gicp_extended(source_points, target_points, max_iterations=100, tolerance=1e
                    lambda_tangent=float(lambda_tangent), lambda_normal=float(lambda_normal),
                    covariance_model=int(covariance_model), **engine_params)
     eng.set_robust_kernel(robust_kernel, robust_scale, adaptive=robust_adaptive, min_scale=robust_min_scale)
-    r = eng.register_pair_host(src[:, :dim], tgt[:, :dim])  # gicp.py:104, 111, 116-167 in one staged round trip
+    if voxel_distributions:
+        r = _register_voxelized(eng, raw_src[:, :dim], raw_tgt[:, :dim], voxel_size, voxel_min_points)
+        src, tgt = r["source_points"], r["target_points"]
+    else:
+        r = eng.register_pair_host(src[:, :dim], tgt[:, :dim])  # gicp.py:104, 111, 116-167 in one staged round trip
     n_outer, conv = r["n_outer"], r["converged_at"]
     n_T = n_outer if conv >= 0 else n_outer + 1             # appendix A rule 12
     T_hist = r["T_hist"][:n_T]
@@ -119,10 +130,16 @@ def gicp_extended(source_points, target_points, max_iterations=100, tolerance=1e
                           covariance_model=int(covariance_model), **engine_params)
             eh.set_robust_kernel(robust_kernel, robust_scale, adaptive=robust_adaptive, min_scale=robust_min_scale)
             n_s, n_t = len(src64), len(tgt64)
-            eh.set_target(torch.as_tensor(np.tile(np.ascontiguousarray(tgt[:, :dim], dtype=np_dt), (reps, 1)), device=eh.device),
-                          np.arange(reps + 1, dtype=np.int64) * n_t)
-            eh.set_source(torch.as_tensor(np.tile(np.ascontiguousarray(src[:, :dim], dtype=np_dt), (reps, 1)), device=eh.device),
-                          np.arange(reps + 1, dtype=np.int64) * n_s)
+            if voxel_distributions:      # the raw clouds replicated, every copy voxelized as the pair's own sides were
+                for setv, cloud in ((eh.set_target_voxelized, raw_tgt), (eh.set_source_voxelized, raw_src)):
+                    setv(torch.as_tensor(np.tile(np.ascontiguousarray(cloud[:, :dim], dtype=np_dt), (reps, 1)),
+                                         device=eh.device), np.arange(reps + 1, dtype=np.int64) * len(cloud),
+                         voxel_size=voxel_size, min_points=voxel_min_points)
+            else:
+                eh.set_target(torch.as_tensor(np.tile(np.ascontiguousarray(tgt[:, :dim], dtype=np_dt), (reps, 1)), device=eh.device),
+                              np.arange(reps + 1, dtype=np.int64) * n_t)
+                eh.set_source(torch.as_tensor(np.tile(np.ascontiguousarray(src[:, :dim], dtype=np_dt), (reps, 1)), device=eh.device),
+                              np.arange(reps + 1, dtype=np.int64) * n_s)
             idx_all, _, W_all = eh.correspond(T_hist[:reps])
             idx_all = idx_all.cpu().numpy().reshape(reps, n_s)
             W_all = W_all.cpu().numpy().reshape(reps, n_s, dim, dim)
@@ -140,6 +157,24 @@ def gicp_extended(source_points, target_points, max_iterations=100, tolerance=1e
             hw_t.append(q[order])
         out["hw_src"], out["hw_tgt"] = hw_s, hw_t
     return out
+
+
+def _register_voxelized(eng, src, tgt, voxel_size, min_points):
+    """Both sides of one pair set up as voxel distributions, registered; the host arrays register_pair_host returns,
+    plus the voxel means as ``source_points`` / ``target_points`` (float64)."""
+    from .engine import SOURCE, TARGET
+    np_dt = np.float64 if eng.storage == "f64" else np.float32
+    tm, _ = eng.set_target_voxelized(np.ascontiguousarray(tgt, dtype=np_dt), voxel_size=voxel_size, min_points=min_points)
+    sm, _ = eng.set_source_voxelized(np.ascontiguousarray(src, dtype=np_dt), voxel_size=voxel_size, min_points=min_points)
+    res = eng.register(history=True)
+    n_outer, conv = int(res.n_outer[0]), int(res.converged_at[0])
+    T_hist = res.T_hist[0].cpu().numpy()
+    T_hist[(n_outer if conv >= 0 else n_outer + 1):] = np.nan   # rows the loop wrote: SURVEY appendix A rule 12
+    return dict(T=res.T[0].cpu().numpy(), T_hist=T_hist,
+                loss_hist=res.loss_hist[0].cpu().numpy()[:n_outer], inliers=res.inliers[0].cpu().numpy()[:n_outer],
+                src_cov0=eng.covariances(SOURCE).cpu().numpy(), tgt_cov=eng.covariances(TARGET).cpu().numpy(),
+                n_outer=n_outer, converged_at=conv, source_points=sm.cpu().numpy().astype(np.float64),
+                target_points=tm.cpu().numpy().astype(np.float64))
 
 
 def gicp(source_points, target_points, max_iterations=100, tolerance=1e-6, max_distance_correspondence=150,

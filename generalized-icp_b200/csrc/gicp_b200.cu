@@ -142,12 +142,13 @@ struct SetupScratch {
 // scratch of gicpVoxelDownsample: its own, so a downsample between gicpSetPair and gicpRegister leaves both sides alone
 struct VoxelScratch {
     DevBuf offsets, part, vb, keys, keys_alt, vals, vals_alt, rid, orow, out_off, big, cub_tmp;
+    DevBuf cov;                 // gicpSetVoxelized: each output row's covariance, in output-row order
     double* h_vb = nullptr;     // pinned: per-cloud voxel bounds
     int* h_out_off = nullptr;   // pinned: output offsets
     int h_cap = 0;              // clouds the pinned buffers hold
     std::vector<int> off32;
     void release() {
-        for (DevBuf* b : {&offsets, &part, &vb, &keys, &keys_alt, &vals, &vals_alt, &rid, &orow, &out_off, &big, &cub_tmp})
+        for (DevBuf* b : {&offsets, &part, &vb, &keys, &keys_alt, &vals, &vals_alt, &rid, &orow, &out_off, &big, &cub_tmp, &cov})
             b->release();
         if (h_vb) cudaFreeHost(h_vb);
         if (h_out_off) cudaFreeHost(h_out_off);
@@ -435,6 +436,19 @@ int launch_knn(gicpContext* h, CloudSet& cs, KnnPath path, int* d_idx, double* d
     return 0;
 }
 
+// the side's offsets to the device, unless its plan passes a single cloud's size as a kernel argument
+int upload_offsets(CloudSet& cs, const int64_t* h_offsets, cudaStream_t st) {
+    const int n_clouds = cs.plan.n_clouds;
+    CU(cs.d_offsets.ensure((size_t)(n_clouds + 1) * sizeof(int)));
+    // no stream synchronisation here: a copy from pageable memory is staged by the driver before the call returns,
+    // and the staging vector lives in the handle
+    if (cs.plan.inline_n < 0) {
+        cs.off32.assign(h_offsets, h_offsets + n_clouds + 1);
+        CU(cudaMemcpyAsync(cs.d_offsets.p, cs.off32.data(), cs.off32.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+    }
+    return 0;
+}
+
 template <int D, typename Real>
 int set_cloud(gicpContext* h, const Switches& sw, int which, const void* d_points, const int64_t* h_offsets,
               int n_clouds, cudaStream_t st, int scratch_slot) {
@@ -448,13 +462,7 @@ int set_cloud(gicpContext* h, const Switches& sw, int which, const void* d_point
     if (p.error) return fail("%s (%d clouds)", p.error, n_clouds);
     if (p.n_total > 0 && !d_points) return fail("null point array");
     cs.raw = d_points;
-    CU(cs.d_offsets.ensure((size_t)(n_clouds + 1) * sizeof(int)));
-    // no stream synchronisation here: a copy from pageable memory is staged by the driver before the call returns,
-    // and the staging vector lives in the handle
-    if (p.inline_n < 0) {
-        cs.off32.assign(h_offsets, h_offsets + n_clouds + 1);
-        CU(cudaMemcpyAsync(cs.d_offsets.p, cs.off32.data(), cs.off32.size() * sizeof(int), cudaMemcpyHostToDevice, st));
-    }
+    if (upload_offsets(cs, h_offsets, st)) return 1;
 
     if (build_grid<D, Real>(h, cs, cs.knn, p.knn_cell, st, sc)) return 1;
     const size_t n_cov = (size_t)std::max<int64_t>(p.sharded ? p.slice_len * h->n_ranks : p.n_total, 1);
@@ -846,6 +854,9 @@ template <int D, typename Real>
 int do_knn(gicpContext* h, int which, int* d_idx, double* d_dist, cudaStream_t st) {
     CloudSet& cs = which == GICP_TARGET ? h->tgt : h->src;
     if (!cs.ready) return fail("cloud not set");
+    if (cs.plan.knn_whole == KnnPath::None)
+        return fail("the %s was set up by gicpSetVoxelized: a voxelized side has no k-NN lists",
+                    which == GICP_TARGET ? "target" : "source");
     // re-runs K2 over the whole cloud set with the index outputs enabled; the covariances are rewritten with the
     // values of that run (the set-up's own values unless the set-up ran a constant model or a sharded slice)
     return launch_knn<D, Real>(h, cs, cs.plan.knn_whole, d_idx, d_dist, st, -1, -1, h->scr[0]);
@@ -891,9 +902,10 @@ int bit_length(unsigned long long v) {
 
 // gicpVoxelDownsample (voxel.cuh).  Two host synchronisations: the per-cloud voxel bounds (they size the key fields and
 // are checked against the limits) and the output offsets.
+// With `stats` (gicpSetVoxelized) the centroid kernels also write every output row's covariance to h->vox.cov.
 template <int D, typename Real>
 int do_voxel(gicpContext* h, const void* d_points, const int64_t* h_off, int nc, double leaf, int min_points,
-             void* d_out, int64_t* h_out_off, int* d_voxel_of, int* d_counts, cudaStream_t st) {
+             void* d_out, int64_t* h_out_off, int* d_voxel_of, int* d_counts, cudaStream_t st, bool stats = false) {
     VoxelScratch& v = h->vox;
     int max_n = 0;
     if (const char* e = check_offsets(h_off, nc, &max_n)) return fail("%s (%d clouds)", e, nc);
@@ -1037,14 +1049,69 @@ int do_voxel(gicpContext* h, const void* d_points, const int64_t* h_off, int nc,
     CU(cudaMemsetAsync(big_count, 0, sizeof(int), st));
     VoxOutArgs oa{rid, n, run_begin, run_end, R, orow, v.out_off.as<int>(), nc, min_points, d_voxel_of, d_counts,
                   v.big.as<int>(), big_count};
-    voxel_centroid_kernel<D, Real><<<nb, 256, 0, st>>>(oa, pts, static_cast<Real*>(d_out));
     const int big_blocks = std::max(1, std::min(n / (VOX_SEQ_MAX + 1), 148 * 8));
-    voxel_centroid_block_kernel<D, Real><<<big_blocks, VOX_THREADS, 0, st>>>(oa, pts, static_cast<Real*>(d_out));
+    if (stats) {
+        CU(v.cov.ensure((size_t)n * ns_of(D) * sizeof(Real)));
+        const VoxCovArgs<Real> cv{v.cov.as<Real>(), h->prm.lambda_tangent, h->prm.lambda_normal};
+        ProfScope prof(h, GICP_STAGE_KNN_COV, st);
+        voxel_centroid_kernel<D, Real, true><<<nb, 256, 0, st>>>(oa, pts, static_cast<Real*>(d_out), cv);
+        voxel_centroid_block_kernel<D, Real, true><<<big_blocks, VOX_THREADS, 0, st>>>(oa, pts, static_cast<Real*>(d_out), cv);
+    } else {
+        voxel_centroid_kernel<D, Real, false><<<nb, 256, 0, st>>>(oa, pts, static_cast<Real*>(d_out), VoxCovArgs<Real>{});
+        voxel_centroid_block_kernel<D, Real, false><<<big_blocks, VOX_THREADS, 0, st>>>(oa, pts, static_cast<Real*>(d_out),
+                                                                                        VoxCovArgs<Real>{});
+    }
     h->launches += 2;
     CU(cudaMemcpyAsync(v.h_out_off, v.out_off.p, (size_t)(nc + 1) * sizeof(int), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     CU(cudaGetLastError());
     for (int i = 0; i <= nc; ++i) h_out_off[i] = v.h_out_off[i];
+    return 0;
+}
+
+// a voxelized side's covariances, computed in output-row order, in the order of its grid
+template <int D, typename Real>
+__global__ void sort_cov_kernel(const CloudMeta* __restrict__ meta, const PRec<Real>* __restrict__ spts,
+                                const Real* __restrict__ cov_rows, Real* __restrict__ cov_sorted) {
+    constexpr int NS = Dim<D>::NS;
+    const CloudMeta m = meta[blockIdx.y];
+    const int s = m.pt_begin + blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= m.pt_end) return;
+    const size_t g = (size_t)m.pt_begin + (size_t)spts[s].idx;
+#pragma unroll
+    for (int i = 0; i < NS; ++i) cov_sorted[(size_t)s * NS + i] = cov_rows[g * NS + i];
+}
+
+// gicpSetVoxelized: the voxel pass with moments into the handle's voxel scratch, then - only once it has succeeded and
+// the voxel means have a plan - the side: its one grid over d_out and the covariances in that grid's order.  A refused
+// call leaves both sides as they were.
+template <int D, typename Real>
+int set_voxelized(gicpContext* h, const Switches& sw, int which, const void* d_points, const int64_t* h_off, int nc,
+                  double leaf, int min_points, void* d_out, int64_t* h_out_off, cudaStream_t st) {
+    if (do_voxel<D, Real>(h, d_points, h_off, nc, leaf, min_points, d_out, h_out_off, nullptr, nullptr, st, true)) return 1;
+    const SetupPlan plan = plan_setup_voxelized(h->prm, sw, h_out_off, nc, which, std::is_same<Real, float>::value);
+    if (plan.error) return fail("%s (%d clouds)", plan.error, nc);
+    CloudSet& cs = which == GICP_TARGET ? h->tgt : h->src;
+    cs.ready = false;
+    h->last_stream = st;
+    cs.plan = plan;
+    cs.raw = d_out;
+    if (upload_offsets(cs, h_out_off, st)) return 1;
+    const SetupPlan& p = cs.plan;
+    if (build_grid<D, Real>(h, cs, cs.knn, p.knn_cell, st, h->scr[0])) return 1;
+    const size_t n = (size_t)std::max<int64_t>(p.n_total, 1);
+    CU(cs.cov_knn.ensure(n * ns_of(D) * sizeof(Real)));
+    if (p.cov != CovSource::Voxel) {
+        const Real diag = p.cov == CovSource::Identity ? Real(1) : Real(0);
+        fill_cov_kernel<D, Real><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(cs.cov_knn.as<Real>(), n, diag);
+        h->launches += 1;
+    } else if (p.n_total > 0) {
+        sort_cov_kernel<D, Real><<<dim3((p.max_n + 255) / 256, nc), 256, 0, st>>>(
+            cs.knn.meta.as<CloudMeta>(), cs.knn.spts.as<PRec<Real>>(), h->vox.cov.as<Real>(), cs.cov_knn.as<Real>());
+        h->launches += 1;
+    }
+    CU(cudaGetLastError());
+    cs.ready = true;
     return 0;
 }
 
@@ -1064,7 +1131,7 @@ int check(gicpHandle h) {
 extern "C" {
 
 const char* gicpGetLastError(void) { return g_last_error.c_str(); }
-int gicpVersion(void) { return 105; }
+int gicpVersion(void) { return 106; }
 
 int gicpDefaultParams(gicpParams* p) {
     if (!p) return fail("null params");
@@ -1295,6 +1362,20 @@ int gicpVoxelDownsample(gicpHandle h, const void* d_points, const int64_t* h_off
     if (min_points < 1) return fail("min_points must be >= 1 (got %d)", min_points);
     return DISPATCH(h, do_voxel, h, d_points, h_offsets, n_clouds, voxel_size, min_points, d_out, h_out_offsets,
                     d_voxel_of, d_counts, (cudaStream_t)stream);
+}
+
+int gicpSetVoxelized(gicpHandle h, int which, const void* d_points, const int64_t* h_offsets, int32_t n_clouds,
+                     double voxel_size, int32_t min_points, void* d_out, int64_t* h_out_offsets, void* stream) {
+    if (check(h)) return 1;
+    if (which != GICP_SOURCE && which != GICP_TARGET)
+        return fail("which must be GICP_SOURCE 0 or GICP_TARGET 1 (got %d)", which);
+    if (h->comm) return fail("gicpSetVoxelized: a handle with a communicator (gicpCommInit) takes raw sides only");
+    if (!h_offsets || !h_out_offsets) return fail("null offsets");
+    if (d_points && d_out == d_points) return fail("d_out must not alias d_points");
+    if (!(std::isfinite(voxel_size) && voxel_size > 0)) return fail("voxel_size must be finite and > 0 (got %g)", voxel_size);
+    if (min_points < 1) return fail("min_points must be >= 1 (got %d)", min_points);
+    return DISPATCH(h, set_voxelized, h, read_switches(), which, d_points, h_offsets, n_clouds, voxel_size, min_points,
+                    d_out, h_out_offsets, (cudaStream_t)stream);
 }
 
 int gicpCommGetUniqueId(char id[128]) {

@@ -68,10 +68,11 @@ inline const char* check_offsets(const int64_t* off, int n_clouds, int* max_n) {
     return nullptr;
 }
 
-enum class CovSource { Zero, Identity, Knn };   // C = 0, C = I, or estimated by K2
+// C = 0, C = I, estimated by K2, or the covariance of the voxel's own points (gicpSetVoxelized, voxel.cuh)
+enum class CovSource { Zero, Identity, Knn, Voxel };
 // knn_brute_kernel (one block per cloud, one launch); knn_general_kernel alone (one launch); knn_hist_kernel with
-// the overflow hand-over to knn_general_kernel (two launches)
-enum class KnnPath { Brute, General, HistGeneral };
+// the overflow hand-over to knn_general_kernel (two launches); None: a voxelized side, which has no k-NN lists
+enum class KnnPath { Brute, General, HistGeneral, None };
 
 struct SetupPlan {
     const char* error = nullptr;   // why the clouds cannot be set up; nothing below is valid then
@@ -158,6 +159,23 @@ inline SetupPlan plan_setup(const gicpParams& prm, const Switches& sw, const int
     p.knn = pick_knn(p, sw, prm.k, f32, p.sharded);
     p.knn_whole = pick_knn(p, sw, prm.k, f32, false);
     p.kc = prm.k <= 6 ? 6 : prm.k <= 20 ? 20 : 32;
+    return p;
+}
+
+// gicpSetVoxelized: a side of voxel means (`off` are the output offsets of the voxel pass) whose covariances come from
+// each voxel's own points.  It needs one grid only, the one a raw side of the same points would search
+// (CloudSet::nng()): the k-NN-cell grid under a shared plan, else the nn_cell grid, so K3a keeps its cell choice and a
+// voxelized source keeps the grid order, and with it the accumulation order, of a raw set-up of the same array.  That
+// grid sits in the k-NN grid's slot (shared = true), where gicpCovariances, gicpSourceCovariancesAt and the loop's
+// centring read a side.  No K2 runs: covariance_model 1 and 2 still force C = I / C = 0 as they do for a raw side.
+inline SetupPlan plan_setup_voxelized(const gicpParams& prm, const Switches& sw, const int64_t* off, int n_clouds,
+                                      int which, bool f32) {
+    SetupPlan p = plan_setup(prm, sw, off, n_clouds, which, f32, Ranks{});
+    if (p.error) return p;
+    if (!p.shared) p.knn_cell = p.nn_cell;
+    p.shared = true;
+    if (p.cov == CovSource::Knn) p.cov = CovSource::Voxel;
+    p.knn = p.knn_whole = KnnPath::None;
     return p;
 }
 

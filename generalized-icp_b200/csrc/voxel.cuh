@@ -5,8 +5,11 @@
 // Pipeline: per-cloud voxel bounds -> 64-bit key per row (cloud | cloud-relative voxel coordinates) -> stable sort
 // of (key, row) -> run heads / tails in sorted order -> keep flag at each kept voxel's head row (input order) ->
 // exclusive scan = output row -> fixed-order fp64 centroid per run.
+// gicpSetVoxelized runs the same pipeline with Stats = true: the centroid pass also accumulates each voxel's second
+// moments and writes its regularised covariance (vox_cov_finish).
 #pragma once
 #include "common.cuh"
+#include "knn_cov.cuh"
 
 namespace gicp {
 
@@ -206,10 +209,53 @@ __device__ __forceinline__ void vox_write(const VoxOutArgs& a, Real* __restrict_
     if (a.counts) a.counts[o] = count;
 }
 
-// one thread per voxel: the centroid of a voxel of <= VOX_SEQ_MAX points, summed in fp64 in ascending row order
-// starting from the first point (a -0.0 coordinate survives); longer voxels go to the block kernel
+// where the Stats kernels write the covariance of output row o (cov + o * NS) and its regularisation
+template <typename Real>
+struct VoxCovArgs {
+    Real* cov;
+    double lam_t, lam_n;
+};
+
+// The covariance of one voxel from its moments about its first point p0: n points, sd = sum (p - p0), sq = sum
+// (p - p0)(p - p0)^T (packed upper triangle, Dim<D>::NS entries).  The sample covariance (ddof = 1) about the mean
+// is (sq - n m m^T) / (n - 1) with m = sd / n - the formula of knn_finish_cov, whose moments are about the query
+// point - then regularised_cov; a voxel of one point, or a non-finite scatter, gets the identity (gicp.py:27, 31-34).
+// The shift by p0 bounds the cancellation by the voxel's extent instead of its distance from the origin.
+template <int D>
+__host__ __device__ inline void vox_cov_finish(int n, const double sd[D], const double sq[Dim<D>::NS], double lam_t,
+                                               double lam_n, double C[Dim<D>::NS]) {
+    double S[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};   // regularised_cov's layout: 00 01 02 11 12 22 (2-D: 00 01 11)
+    const bool ident = n <= 1;
+    if (!ident) {
+        const double inv = 1.0 / n;
+        const double f = 1.0 / (n - 1);   // ddof = 1 (np.cov default, gicp.py:12)
+        double m[D];
+#pragma unroll
+        for (int c = 0; c < D; ++c) m[c] = sd[c] * inv;
+#pragma unroll
+        for (int i = 0; i < D; ++i)
+#pragma unroll
+            for (int j = i; j < D; ++j) S[symidx(3, i, j)] = (sq[symidx(D, i, j)] - n * m[i] * m[j]) * f;
+    }
+    regularised_cov<D>(S, ident, lam_t, lam_n, C);
+}
+
 template <int D, typename Real>
-__global__ void voxel_centroid_kernel(VoxOutArgs a, const Real* __restrict__ pts, Real* __restrict__ out) {
+__device__ __forceinline__ void vox_write_cov(const VoxCovArgs<Real>& cv, int o, int count, const double sd[D],
+                                              const double sq[Dim<D>::NS]) {
+    constexpr int NS = Dim<D>::NS;
+    double C[NS];
+    vox_cov_finish<D>(count, sd, sq, cv.lam_t, cv.lam_n, C);
+#pragma unroll
+    for (int i = 0; i < NS; ++i) cv.cov[(size_t)o * NS + i] = (Real)C[i];
+}
+
+// one thread per voxel: the centroid of a voxel of <= VOX_SEQ_MAX points, summed in fp64 in ascending row order
+// starting from the first point (a -0.0 coordinate survives); longer voxels go to the block kernel.  With Stats the
+// same pass accumulates the moments about the first point and writes the voxel's covariance.
+template <int D, typename Real, bool Stats>
+__global__ void voxel_centroid_kernel(VoxOutArgs a, const Real* __restrict__ pts, Real* __restrict__ out,
+                                      VoxCovArgs<Real> cv) {
     const int r = blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= a.rid[a.n]) return;
     const int b = a.run_begin[r], e = a.run_end[r];
@@ -222,8 +268,15 @@ __global__ void voxel_centroid_kernel(VoxOutArgs a, const Real* __restrict__ pts
     const int head = a.rows[b];
     const int o = a.orow[head];
     const int local = a.voxel_of ? o - a.out_off[vox_cloud_of(a.out_off, a.n_clouds, o)] : 0;
-    double s[D];
+    constexpr int NS = Dim<D>::NS;
+    double s[D], p0[D], sd[D], sq[NS];
     vox_load<D, Real>(pts, head, s);
+    if constexpr (Stats) {
+#pragma unroll
+        for (int c = 0; c < D; ++c) { p0[c] = s[c]; sd[c] = 0.0; }
+#pragma unroll
+        for (int i = 0; i < NS; ++i) sq[i] = 0.0;
+    }
     if (a.voxel_of) a.voxel_of[head] = local;
 #pragma unroll 4
     for (int j = b + 1; j < e; ++j) {
@@ -232,27 +285,48 @@ __global__ void voxel_centroid_kernel(VoxOutArgs a, const Real* __restrict__ pts
         vox_load<D, Real>(pts, row, v);
 #pragma unroll
         for (int c = 0; c < D; ++c) s[c] += v[c];
+        if constexpr (Stats) {
+            double d[D];
+#pragma unroll
+            for (int c = 0; c < D; ++c) { d[c] = v[c] - p0[c]; sd[c] += d[c]; }
+#pragma unroll
+            for (int i = 0, k = 0; i < D; ++i)
+#pragma unroll
+                for (int jj = i; jj < D; ++jj, ++k) sq[k] += d[i] * d[jj];
+        }
         if (a.voxel_of) a.voxel_of[row] = local;
     }
     vox_write<D, Real>(a, out, o, s, count);
+    if constexpr (Stats) vox_write_cov<D, Real>(cv, o, count, sd, sq);
 }
 
 // one block per long voxel (persistent over the list): thread t sums points t, t + 256, ... in row order, then a
 // fixed shared-memory tree.  The order depends only on the voxel's own points, so a batch and its clouds one at a
 // time give identical bits.  -0.0 is the identity of IEEE addition (-0.0 + x == x for every x, +0.0 included).
-template <int D, typename Real>
+// With Stats every thread also sums its points' moments about the voxel's first point, and the tree reduces them too:
+// rows [0, D) of sm hold the sums, [D, 2D) the offsets from p0, [2D, 2D + NS) their outer products.
+template <int D, typename Real, bool Stats>
 __global__ void __launch_bounds__(VOX_THREADS) voxel_centroid_block_kernel(VoxOutArgs a, const Real* __restrict__ pts,
-                                                                           Real* __restrict__ out) {
-    __shared__ double sm[D][VOX_THREADS];
+                                                                           Real* __restrict__ out, VoxCovArgs<Real> cv) {
+    constexpr int NS = Dim<D>::NS;
+    constexpr int NM = Stats ? 2 * D + NS : D;
+    __shared__ double sm[NM][VOX_THREADS];
     const int n_big = *a.big_count;
     for (int k = blockIdx.x; k < n_big; k += gridDim.x) {
         const int r = a.big_list[k];
         const int b = a.run_begin[r], e = a.run_end[r];
         const int o = a.orow[a.rows[b]];
         const int local = a.voxel_of ? o - a.out_off[vox_cloud_of(a.out_off, a.n_clouds, o)] : 0;
-        double s[D];
+        double s[D], p0[D], sd[D], sq[NS];
 #pragma unroll
         for (int c = 0; c < D; ++c) s[c] = -0.0;
+        if constexpr (Stats) {
+            vox_load<D, Real>(pts, a.rows[b], p0);
+#pragma unroll
+            for (int c = 0; c < D; ++c) sd[c] = 0.0;
+#pragma unroll
+            for (int i = 0; i < NS; ++i) sq[i] = 0.0;
+        }
 #pragma unroll 4
         for (int j = b + threadIdx.x; j < e; j += VOX_THREADS) {
             const int row = a.rows[j];
@@ -260,21 +334,43 @@ __global__ void __launch_bounds__(VOX_THREADS) voxel_centroid_block_kernel(VoxOu
             vox_load<D, Real>(pts, row, v);
 #pragma unroll
             for (int c = 0; c < D; ++c) s[c] += v[c];
+            if constexpr (Stats) {
+                double d[D];
+#pragma unroll
+                for (int c = 0; c < D; ++c) { d[c] = v[c] - p0[c]; sd[c] += d[c]; }
+#pragma unroll
+                for (int i = 0, k = 0; i < D; ++i)
+#pragma unroll
+                    for (int jj = i; jj < D; ++jj, ++k) sq[k] += d[i] * d[jj];
+            }
             if (a.voxel_of) a.voxel_of[row] = local;
         }
 #pragma unroll
         for (int c = 0; c < D; ++c) sm[c][threadIdx.x] = s[c];
+        if constexpr (Stats) {
+#pragma unroll
+            for (int c = 0; c < D; ++c) sm[D + c][threadIdx.x] = sd[c];
+#pragma unroll
+            for (int i = 0; i < NS; ++i) sm[2 * D + i][threadIdx.x] = sq[i];
+        }
         __syncthreads();
         for (int w = VOX_THREADS / 2; w > 0; w >>= 1) {
             if (threadIdx.x < w)
 #pragma unroll
-                for (int c = 0; c < D; ++c) sm[c][threadIdx.x] += sm[c][threadIdx.x + w];
+                for (int c = 0; c < NM; ++c) sm[c][threadIdx.x] += sm[c][threadIdx.x + w];
             __syncthreads();
         }
         if (threadIdx.x == 0) {
 #pragma unroll
             for (int c = 0; c < D; ++c) s[c] = sm[c][0];
             vox_write<D, Real>(a, out, o, s, e - b);
+            if constexpr (Stats) {
+#pragma unroll
+                for (int c = 0; c < D; ++c) sd[c] = sm[D + c][0];
+#pragma unroll
+                for (int i = 0; i < NS; ++i) sq[i] = sm[2 * D + i][0];
+                vox_write_cov<D, Real>(cv, o, e - b, sd, sq);
+            }
         }
         __syncthreads();
     }

@@ -418,6 +418,38 @@ class GicpEngine:
             return pts, out_off, vox, cnt[:m].clone()
         return pts, out_off
 
+    # ---- voxel distributions (VGICP) ----
+    def _set_voxelized(self, which, points, offsets, voxel_size, min_points):
+        points, off = self._prep(points, offsets)
+        n, nc = points.shape[0], len(off) - 1
+        out = torch.empty((n, self.dim), dtype=self.dtype, device=self.device)
+        out_off = np.zeros(nc + 1, dtype=np.int64)
+        i64p = C.POINTER(C.c_int64)
+        _lib.check(self.lib.gicpSetVoxelized(self._h, which, _ptr(points), off.ctypes.data_as(i64p), nc,
+                                             float(voxel_size), int(min_points), _ptr(out),
+                                             out_off.ctypes.data_as(i64p), self._stream()))
+        m = int(out_off[-1])
+        self._keep[which] = out     # the side's point array: the library reads it in every later call
+        self._n[which] = (m, nc)
+        return out[:m], out_off
+
+    def set_target_voxelized(self, points, offsets=None, *, voxel_size, min_points=1):
+        """Set the target(s) up as voxel distributions (gicpSetVoxelized; semantics in include/gicp_b200.h): one point
+        per voxel of edge ``voxel_size`` with >= ``min_points`` finite points - exactly what :meth:`voxel_downsample`
+        returns - carrying the regularised covariance of that voxel's own points, with no k-NN search.  Returns
+        ``(means, out_offsets)`` like voxel_downsample; ``means`` is the side's array (a view of a buffer the engine
+        keeps alive), and every later per-point output of this side (covariances, correspondence indices) refers to
+        its rows.  Inlier counts and fitness then count voxels.  A refused call leaves both sides as they were.
+        Memory: the voxel count is known only after the call, so the side's array is allocated at the input's row
+        count and kept alive whole while the side is set up (the library reads it in place); with dense clouds that
+        is the input's size again, of which only the first M rows are used.  It is released when the side is set up
+        again."""
+        return self._set_voxelized(TARGET, points, offsets, voxel_size, min_points)
+
+    def set_source_voxelized(self, points, offsets=None, *, voxel_size, min_points=1):
+        """The source side of :meth:`set_target_voxelized`."""
+        return self._set_voxelized(SOURCE, points, offsets, voxel_size, min_points)
+
     # ---- stage entry points ----
     def knn(self, which, with_dist=True):
         n = self._n[which][0]

@@ -237,6 +237,33 @@ int gicpVoxelDownsample(gicpHandle h, const void* d_points, const int64_t* h_off
                         double voxel_size, int32_t min_points, void* d_out, int64_t* h_out_offsets,
                         int32_t* d_voxel_of, int32_t* d_counts, void* stream);
 
+/* ---- voxel distributions (VGICP: Koide et al., ICRA 2021; FastVGICP of fast_gicp / small_gicp) ----------------
+ * Sets up side `which` (GICP_SOURCE or GICP_TARGET) with one point per occupied voxel, carrying the covariance of that
+ * voxel's own points, instead of the raw points with k-NN covariances (no k-NN search runs).
+ *  - The side's points are exactly what gicpVoxelDownsample(h, d_points, h_offsets, n_clouds, voxel_size, min_points,
+ *    d_out, h_out_offsets, NULL, NULL, stream) writes, bit for bit: same voxels, rows, order, offsets, limits and errors.
+ *    d_out becomes the side's point array and must stay valid until the next set-up of that side; cloud-local indices
+ *    reported later (gicpCorrespond, match indices) are rows of d_out.
+ *  - The covariance of an output row is the reference's estimator (gicp.py:11-16, 27, 31-34) with every finite point of
+ *    the voxel as the neighbourhood: the float64 sample covariance (ddof = 1) of the raw input rows about their float64
+ *    mean, regularised to lambda_tangent I - (lambda_tangent - lambda_normal) n n^T (3-D, n the eigenvector of the
+ *    smallest eigenvalue; 2-D lambda_normal I + (lambda_tangent - lambda_normal) v v^T, v of the largest); the identity
+ *    for a voxel of one point or a non-finite scatter; rounded once to the storage type.  k and
+ *    max_distance_nearest_neighbors do not apply.  covariance_model 1 and 2 force C = I / C = 0 as for a raw side.
+ *  - Sums are float64 in a fixed order per voxel: a batch and its clouds one at a time give identical bits.
+ *  - Every voxel counts once, whatever its point count (the plain, unweighted objective; correspondences are not
+ *    weighted by the voxels' sizes).  So on a voxelized side the inlier counts, gicpEvaluate's n and fitness and
+ *    d_inliers count voxels, not raw points.
+ *  - Either side may be voxelized on its own: a voxelized target with a raw source is fast_gicp's VGICP split, both
+ *    sides voxelized is distribution-to-distribution.  The voxel means are searched by the exact 1-NN search and gated
+ *    by max_distance_correspondence like raw points.  gicpCovariances returns the voxel covariances in output-row
+ *    order; the other entry points work unchanged, except gicpKnn, which fails: the side has no k-NN lists.
+ * Fails, leaving both sides of the handle as they were, on a bad `which`, a voxel_size that is not finite and > 0,
+ * min_points < 1, the per-axis limit of gicpVoxelDownsample, or a handle with a communicator (gicpCommInit).
+ * Synchronises the stream (the offsets come back to the host).                                                    */
+int gicpSetVoxelized(gicpHandle h, int which, const void* d_points, const int64_t* h_offsets, int32_t n_clouds,
+                     double voxel_size, int32_t min_points, void* d_out, int64_t* h_out_offsets, void* stream);
+
 /* ---- multi-GPU: one large pair with the source sharded over ranks (BASELINE config 5) ----
  * Every rank holds both full clouds; rank r computes covariances for its slice of the
  * target (all-gathered once) and runs the per-iteration reduction on its slice of the
