@@ -14,7 +14,7 @@ SYMBOLS = [
     "gicpNormalEquations", "gicpSourceCovariancesAt", "gicpCommGetUniqueId", "gicpCommInit", "gicpCommDestroy",
     "gicpLaunchCount", "gicpProfile", "gicpProfileRead", "gicpRayCast", "gicpVoxelDownsample",
     "gicpSetRobustKernel", "gicpSetRobustKernelAdaptive", "gicpRobustScales", "gicpProfileReadStages", "gicpEvaluate",
-    "gicpSetVoxelized",
+    "gicpSetVoxelized", "gicpSetPairList",
 ]
 
 
@@ -62,6 +62,7 @@ def load():
         f.argtypes = [vp, vp, C.POINTER(i64), i32, vp]
     lib.gicpSetPair.argtypes = [vp, vp, C.POINTER(i64), vp, C.POINTER(i64), i32, vp]
     lib.gicpPromoteTargetToSource.argtypes = [vp]
+    lib.gicpSetPairList.argtypes = [vp, i32, C.POINTER(i32), C.POINTER(i32), C.c_int, C.POINTER(i64), vp]
     lib.gicpRegister.argtypes = [vp, dp, vp, vp, vp, vp, vp, vp, vp]
     lib.gicpKnn.argtypes = [vp, C.c_int, vp, vp, vp]
     lib.gicpCovariances.argtypes = [vp, C.c_int, vp, vp]

@@ -177,6 +177,47 @@ def _register_voxelized(eng, src, tgt, voxel_size, min_points):
                 target_points=tm.cpu().numpy().astype(np.float64))
 
 
+def register_pairs(clouds, pairs, T0=None, *, storage="f64", evaluate=True, **params):
+    """Register every ``(source, target)`` pair of cloud indices over one set-up of ``clouds`` (a list of (N_i, d)
+    arrays): each cloud's grids and covariances are built once, as a target set, and every pair registers its source
+    cloud onto its target cloud (GicpEngine.set_pair_list with source_set=TARGET).  ``params`` are gicpParams fields
+    (k, max_iterations, max_distance_correspondence, ...) over the library's defaults; ``T0`` (E, d+1, d+1) optional
+    initial transforms.  Returns a dict of per-pair numpy arrays, the inputs of a pose graph: ``T`` (E, d+1, d+1),
+    which maps the source cloud's points onto the target cloud's, ``n_outer`` and ``converged_at``, and with
+    ``evaluate`` the quality at T: ``n_inliers``, ``fitness``, ``inlier_rmse`` and ``information`` (H, rotation
+    first; include/gicp_b200.h, gicpEvaluate)."""
+    import ctypes
+
+    import torch
+    from ._lib import GicpParams
+    from .engine import TARGET
+
+    if len(clouds) == 0:
+        raise ValueError("no clouds")
+    dim = int(np.asarray(clouds[0]).shape[1])
+    if dim not in (2, 3):
+        raise ValueError(f"expected (N, 2) or (N, 3) clouds, got {np.asarray(clouds[0]).shape}")
+    pr = np.asarray(pairs, dtype=np.int64).reshape(-1, 2)
+    eng = _engine(dim, storage, "pairs")
+    defaults = GicpParams()
+    eng.lib.gicpDefaultParams(ctypes.byref(defaults))
+    eng.set_params(**{**{f: getattr(defaults, f) for f, _ in GicpParams._fields_}, **params})
+    eng.set_robust_kernel(None)
+    np_dt = np.float64 if storage == "f64" else np.float32
+    arrs = [np.asarray(c, dtype=np_dt).reshape(-1, dim) for c in clouds]
+    off = np.zeros(len(arrs) + 1, dtype=np.int64)
+    off[1:] = np.cumsum([len(a) for a in arrs])
+    eng.set_target(torch.as_tensor(np.concatenate(arrs, axis=0), device=eng.device), off)
+    eng.set_pair_list(pr[:, 0], pr[:, 1], source_set=TARGET)
+    r = eng.register(T0, history=False)
+    out = dict(T=r.T.cpu().numpy(), n_outer=r.n_outer.cpu().numpy(), converged_at=r.converged_at.cpu().numpy())
+    if evaluate:
+        q = eng.evaluate(r.T)
+        out.update(n_inliers=q.n_inliers.cpu().numpy(), fitness=q.fitness.cpu().numpy(),
+                   inlier_rmse=q.inlier_rmse.cpu().numpy(), information=q.H.cpu().numpy())
+    return out
+
+
 def gicp(source_points, target_points, max_iterations=100, tolerance=1e-6, max_distance_correspondence=150,
          max_distance_nearest_neighbors=50):
     """Same call, same 7-tuple as the reference (gicp.py:78,174):

@@ -26,6 +26,7 @@
 #include "scale.cuh"
 #include "voxel.cuh"
 #include "quality.cuh"
+#include "pairs.cuh"
 #include "plan.h"
 
 using namespace gicp;
@@ -81,6 +82,7 @@ struct CloudSet {
     const void* raw = nullptr;
     SetupPlan plan;           // sizes, grids and kernels of this cloud set, fixed by its set-up
     std::vector<int> off32;   // staging copy of the offsets for the asynchronous upload (must outlive the call)
+    std::vector<int64_t> h_off;   // the set-up's offsets on the host (n_clouds + 1): the sizes gicpSetPairList reads
     DevBuf d_offsets;   // int32 [n_clouds+1]; not uploaded when plan.inline_n >= 0
     Grid knn;           // grid of the covariance neighbourhoods (cell ~ knn radius / 4)
     Grid nn;            // grid of the correspondence search (cell ~ d_max / 2): the target is searched in it,
@@ -92,6 +94,19 @@ struct CloudSet {
     Grid& nng() { return plan.shared ? knn : nn; }
     DevBuf& covnn() { return plan.shared ? cov_knn : cov_nn; }
     void release() { d_offsets.release(); knn.release(); nn.release(); cov_knn.release(); cov_nn.release(); }
+};
+
+// gicpSetPairList: the listed pairs' sources gathered into pair order with per-pair metadata (pairs.cuh).  While `on`,
+// the loop and the stage entry points run over the pairs (loop_view) instead of source cloud i against target cloud i.
+struct PairList {
+    bool on = false;
+    SetupPlan view;            // plan_pairs: n_clouds = n_pairs, max_n and n_total over the pairs' sources
+    std::vector<int> h_list;   // staging of the upload: [n_pairs][3] source cloud, target cloud, first row
+    DevBuf list, src_meta, tgt_meta, tgt_bbox, spts, cov;
+    void release() {
+        for (DevBuf* b : {&list, &src_meta, &tgt_meta, &tgt_bbox, &spts, &cov}) b->release();
+        on = false;
+    }
 };
 
 // NCCL through dlopen: the engine must load without NCCL when no communicator is requested.
@@ -166,6 +181,7 @@ struct gicpContext {
     bool robust_adaptive = false;         // gicpSetRobustKernelAdaptive: c = max(robust_min_scale, robust_kappa * median)
     double robust_kappa = 0.0, robust_min_scale = 0.0;
     CloudSet src, tgt;
+    PairList pairs;   // gicpSetPairList; discarded whenever a side or the parameters change
     // [0]: every call on the caller's stream; [1]: the source side of gicpSetPair while it runs on the internal stream
     SetupScratch scr[2];
     VoxelScratch vox;
@@ -440,6 +456,7 @@ int launch_knn(gicpContext* h, CloudSet& cs, KnnPath path, int* d_idx, double* d
 int upload_offsets(CloudSet& cs, const int64_t* h_offsets, cudaStream_t st) {
     const int n_clouds = cs.plan.n_clouds;
     CU(cs.d_offsets.ensure((size_t)(n_clouds + 1) * sizeof(int)));
+    cs.h_off.assign(h_offsets, h_offsets + n_clouds + 1);
     // no stream synchronisation here: a copy from pageable memory is staged by the driver before the call returns,
     // and the staging vector lives in the handle
     if (cs.plan.inline_n < 0) {
@@ -455,6 +472,7 @@ int set_cloud(gicpContext* h, const Switches& sw, int which, const void* d_point
     SetupScratch& sc = h->scr[scratch_slot];
     CloudSet& cs = which == GICP_TARGET ? h->tgt : h->src;
     cs.ready = false;
+    h->pairs.on = false;
     h->last_stream = st;
     cs.plan = plan_setup(h->prm, sw, h_offsets, n_clouds, which, std::is_same<Real, float>::value,
                          Ranks{h->comm != nullptr, h->n_ranks, h->rank});
@@ -510,18 +528,33 @@ int zero_source_cov(gicpContext* h, cudaStream_t st) {
     return 0;
 }
 
+// What the loop and the pair-indexed entry points run over: source cloud i against target cloud i, or the pair list.
+// `plan` sizes the loop (n_clouds = pairs, max_n and n_total of the sources), `tgt_bbox` holds every pair's target box
+// (the centring point and the fused loop's self-initialisation).
+struct LoopView {
+    const SetupPlan& plan;
+    const double* tgt_bbox;
+    bool ready;   // something to register: both sides set up, or a pair list (which needs no source set)
+};
+LoopView loop_view(gicpContext* h) {
+    if (h->pairs.on) return LoopView{h->pairs.view, h->pairs.tgt_bbox.as<double>(), true};
+    return LoopView{h->src.plan, h->tgt.knn.bbox.as<double>(), h->src.ready && h->tgt.ready};
+}
+
 template <int D, typename Real>
 int objective_args(gicpContext* h, const Switches& sw, bool sliced, bool has_T0, ObjArgs<Real>& a, LoopPlan& lp) {
     CloudSet &S = h->src, &T = h->tgt;
-    if (!S.ready || !T.ready) return fail("set source and target first");
-    const int np = S.plan.n_clouds;
-    if (np != T.plan.n_clouds) return fail("source has %d clouds, target %d", np, T.plan.n_clouds);
-    lp = plan_loop(sw, S.plan, sliced, Ranks{h->comm != nullptr, h->n_ranks, h->rank}, h->prof_on, has_T0,
+    const PairList& pl = h->pairs;
+    const LoopView lv = loop_view(h);
+    if (!lv.ready) return fail("set source and target first");
+    const int np = lv.plan.n_clouds;
+    if (!pl.on && np != T.plan.n_clouds) return fail("source has %d clouds, target %d", np, T.plan.n_clouds);
+    lp = plan_loop(sw, lv.plan, sliced, Ranks{h->comm != nullptr, h->n_ranks, h->rank}, h->prof_on, has_T0,
                    h->robust_kind != GICP_ROBUST_NONE, h->robust_adaptive);
-    a.src_meta = S.nng().meta.as<CloudMeta>();
-    a.src_spts = S.nng().spts.as<PRec<Real>>();
-    a.src_cov = S.covnn().as<Real>();
-    a.tgt_meta = T.nng().meta.as<CloudMeta>();
+    a.src_meta = pl.on ? pl.src_meta.as<CloudMeta>() : S.nng().meta.as<CloudMeta>();
+    a.src_spts = pl.on ? pl.spts.as<PRec<Real>>() : S.nng().spts.as<PRec<Real>>();
+    a.src_cov = pl.on ? pl.cov.as<Real>() : S.covnn().as<Real>();
+    a.tgt_meta = pl.on ? pl.tgt_meta.as<CloudMeta>() : T.nng().meta.as<CloudMeta>();
     a.tgt_cell_start = T.nng().cell_start.as<int>();
     a.tgt_lut = T.nng().lut.as<int>();
     a.tgt_spts = T.nng().spts.as<PRec<Real>>();
@@ -554,9 +587,9 @@ int objective_args(gicpContext* h, const Switches& sw, bool sliced, bool has_T0,
     CU(h->partial.ensure((size_t)np * lp.bpp * Dim<D>::NRED * sizeof(double)));
     CU(h->red.ensure((size_t)np * Dim<D>::NRED * sizeof(double)));
     a.partial = h->partial.as<double>();
-    CU(h->prev_match.ensure((size_t)std::max<int64_t>(S.plan.n_total, 1) * sizeof(int)));
+    CU(h->prev_match.ensure((size_t)std::max<int64_t>(lv.plan.n_total, 1) * sizeof(int)));
     a.match = h->prev_match.as<int>();
-    CU(h->slack.ensure((size_t)std::max<int64_t>(S.plan.n_total, 1) * sizeof(float)));
+    CU(h->slack.ensure((size_t)std::max<int64_t>(lv.plan.n_total, 1) * sizeof(float)));
     a.slack = nullptr;
     return 0;
 }
@@ -572,7 +605,8 @@ int upload_T(gicpContext* h, const double* h_T, size_t bytes, cudaStream_t st) {
 template <int D, typename Real>
 int ensure_state(gicpContext* h, const double* h_T0, double* d_T, double* d_T_hist, int* d_n_outer,
                  int* d_converged, cudaStream_t st) {
-    const int np = h->src.plan.n_clouds;
+    const LoopView lv = loop_view(h);
+    const int np = lv.plan.n_clouds;
     CU(h->state.ensure((size_t)np * sizeof(PairState)));
     CU(h->n_active.ensure(sizeof(int)));
     const double* d_T0 = nullptr;
@@ -580,7 +614,7 @@ int ensure_state(gicpContext* h, const double* h_T0, double* d_T, double* d_T_hi
         if (upload_T(h, h_T0, (size_t)np * (D + 1) * (D + 1) * sizeof(double), st)) return 1;
         d_T0 = h->T_dev.as<double>();
     }
-    init_state_kernel<D><<<(np + 127) / 128, 128, 0, st>>>(h->state.as<PairState>(), d_T0, h->tgt.knn.bbox.as<double>(), np,
+    init_state_kernel<D><<<(np + 127) / 128, 128, 0, st>>>(h->state.as<PairState>(), d_T0, lv.tgt_bbox, np,
                                                            d_T, d_T_hist, h->prm.max_iterations, d_n_outer, d_converged,
                                                            h->n_active.as<int>());
     h->launches += 1;
@@ -592,8 +626,9 @@ int ensure_state(gicpContext* h, const double* h_T0, double* d_T, double* d_T_hi
 // leaves them so); a.pair_scale is where the accumulation reads the scale
 template <int D, typename Real>
 int prepare_select(gicpContext* h, ObjArgs<Real>& a, ScaleArgs& sc, cudaStream_t st) {
-    const int np = h->src.plan.n_clouds;
-    CU(h->sel_keys.ensure((size_t)std::max<int64_t>(h->src.plan.n_total, 1) * sizeof(unsigned long long)));
+    const SetupPlan& sp = loop_view(h).plan;
+    const int np = sp.n_clouds;
+    CU(h->sel_keys.ensure((size_t)std::max<int64_t>(sp.n_total, 1) * sizeof(unsigned long long)));
     CU(h->sel_hist.ensure((size_t)np * SEL_BINS * sizeof(unsigned)));
     CU(h->sel_arrived.ensure((size_t)np * sizeof(unsigned)));
     CU(h->sel_state.ensure((size_t)np * sizeof(SelState)));
@@ -628,7 +663,8 @@ int do_register(gicpContext* h, const Switches& sw, const double* h_T0, double* 
     if (lp.adaptive && lp.sharded)
         return fail("an adaptive robust scale needs every source point on one rank: sharded-source registration "
                     "(gicpCommInit) takes a fixed scale (gicpSetRobustKernel) or none");
-    const int np = h->src.plan.n_clouds;
+    const LoopView lv = loop_view(h);
+    const int np = lv.plan.n_clouds;
     const int bpp = lp.bpp;
     h->last_stream = st;
     if (lp.self_init) {
@@ -636,8 +672,8 @@ int do_register(gicpContext* h, const Switches& sw, const double* h_T0, double* 
     } else {
         if (ensure_state<D, Real>(h, h_T0, d_T, d_T_hist, d_n_outer, d_converged, st)) return 1;
         // last iteration's match per source point (bounds the next search); -1 = none yet
-        CU(cudaMemsetAsync(h->prev_match.p, 0xFF, (size_t)std::max<int64_t>(h->src.plan.n_total, 1) * sizeof(int), st));
-        CU(cudaMemsetAsync(h->slack.p, 0, (size_t)std::max<int64_t>(h->src.plan.n_total, 1) * sizeof(float), st));
+        CU(cudaMemsetAsync(h->prev_match.p, 0xFF, (size_t)std::max<int64_t>(lv.plan.n_total, 1) * sizeof(int), st));
+        CU(cudaMemsetAsync(h->slack.p, 0, (size_t)std::max<int64_t>(lv.plan.n_total, 1) * sizeof(float), st));
     }
     oa.use_prev = 1;
     oa.slack = sw.no_skip ? nullptr : h->slack.as<float>();
@@ -670,7 +706,7 @@ int do_register(gicpContext* h, const Switches& sw, const double* h_T0, double* 
                            : lp.robust ? register_loop_kernel<D, Real, true> : register_loop_kernel<D, Real, false>;
         CU(cudaFuncSetAttribute(loop_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         ProfScope prof(h, GICP_STAGE_CORRESPOND, st);
-        loop_kernel<<<np, OBJ_THREADS, smem, st>>>(oa, sa, lp.self_init ? h->tgt.knn.bbox.as<double>() : nullptr);
+        loop_kernel<<<np, OBJ_THREADS, smem, st>>>(oa, sa, lp.self_init ? lv.tgt_bbox : nullptr);
         h->launches += 1;
         CU(cudaGetLastError());
         return 0;
@@ -779,7 +815,7 @@ int do_register(gicpContext* h, const Switches& sw, const double* h_T0, double* 
 template <int D, typename Real>
 int stage_pass(gicpContext* h, ObjArgs<Real>& oa, const LoopPlan& lp, const double* d_T, int* d_idx, double* d_dist,
                double* d_W, bool fold, ScaleArgs& sc, cudaStream_t st) {
-    const int np = h->src.plan.n_clouds;
+    const int np = loop_view(h).plan.n_clouds;
     const int bpp = lp.bpp;
     if (ensure_state<D, Real>(h, nullptr, nullptr, nullptr, nullptr, nullptr, st)) return 1;
     oa.T_override = d_T;
@@ -815,7 +851,7 @@ int do_stage(gicpContext* h, const Switches& sw, const double* h_T, int* d_idx, 
     LoopPlan lp;
     // stage entry points always cover the whole source (no slicing), so their outputs are complete
     if (objective_args<D, Real>(h, sw, false, true, oa, lp)) return 1;
-    const int np = h->src.plan.n_clouds;
+    const int np = loop_view(h).plan.n_clouds;
     if (!h_T) return fail("h_T is required");
     if (upload_T(h, h_T, (size_t)np * (D + 1) * (D + 1) * sizeof(double), st)) return 1;
     ScaleArgs sc{};
@@ -836,8 +872,9 @@ int do_evaluate(gicpContext* h, const Switches& sw, const double* d_T, double* d
     ObjArgs<Real> oa;
     LoopPlan lp;
     if (objective_args<D, Real>(h, sw, false, true, oa, lp)) return 1;
-    const int np = h->src.plan.n_clouds;
-    const size_t n_src = (size_t)std::max<int64_t>(h->src.plan.n_total, 1);
+    const SetupPlan& sp = loop_view(h).plan;
+    const int np = sp.n_clouds;
+    const size_t n_src = (size_t)std::max<int64_t>(sp.n_total, 1);
     CU(h->eval_idx.ensure(n_src * sizeof(int)));
     CU(h->eval_dist.ensure(n_src * sizeof(double)));
     ScaleArgs sc{};
@@ -880,15 +917,18 @@ int do_cov(gicpContext* h, int which, double* d_cov, cudaStream_t st) {
 template <int D, typename Real>
 int do_rotcov(gicpContext* h, const double* h_T, int n_T, double* d_out, cudaStream_t st) {
     CloudSet& cs = h->src;
-    if (!cs.ready) return fail("source not set");
-    const SetupPlan& p = cs.plan;
+    const PairList& pl = h->pairs;
+    if (!pl.on && !cs.ready) return fail("source not set");
+    const SetupPlan& p = loop_view(h).plan;
     if (n_T <= 0 || p.n_total == 0) return 0;
     if (n_T > 65535) return fail("n_T too large");
     if (upload_T(h, h_T, (size_t)n_T * p.n_clouds * (D + 1) * (D + 1) * sizeof(double), st)) return 1;
     const int bx = (p.max_n + 255) / 256;
+    // a pair list's sources: the gathered copies (search-grid order; the output is in input order either way)
     rotated_cov_kernel<D, Real><<<dim3(bx, p.n_clouds, n_T), 256, 0, st>>>(
-        cs.knn.meta.as<CloudMeta>(), cs.knn.spts.as<PRec<Real>>(), cs.cov_knn.as<Real>(), h->T_dev.as<double>(),
-        p.n_clouds, (size_t)p.n_total, d_out);
+        pl.on ? pl.src_meta.as<CloudMeta>() : cs.knn.meta.as<CloudMeta>(),
+        pl.on ? pl.spts.as<PRec<Real>>() : cs.knn.spts.as<PRec<Real>>(), pl.on ? pl.cov.as<Real>() : cs.cov_knn.as<Real>(),
+        h->T_dev.as<double>(), p.n_clouds, (size_t)p.n_total, d_out);
     h->launches += 1;
     CU(cudaGetLastError());
     return 0;
@@ -1093,6 +1133,7 @@ int set_voxelized(gicpContext* h, const Switches& sw, int which, const void* d_p
     if (plan.error) return fail("%s (%d clouds)", plan.error, nc);
     CloudSet& cs = which == GICP_TARGET ? h->tgt : h->src;
     cs.ready = false;
+    h->pairs.on = false;
     h->last_stream = st;
     cs.plan = plan;
     cs.raw = d_out;
@@ -1112,6 +1153,49 @@ int set_voxelized(gicpContext* h, const Switches& sw, int which, const void* d_p
     }
     CU(cudaGetLastError());
     cs.ready = true;
+    return 0;
+}
+
+// gicpSetPairList: validate (plan_pairs), then gather the pairs' sources and metadata on `st`.  A refused list leaves
+// the handle as it was.
+template <int D, typename Real>
+int set_pair_list(gicpContext* h, int n_pairs, const int32_t* src_cloud, const int32_t* tgt_cloud, int source_set,
+                  int64_t* h_pair_offsets, cudaStream_t st) {
+    auto sizes = [](const CloudSet& cs) { return cs.ready ? SetSizes{cs.h_off.data(), cs.plan.n_clouds} : SetSizes{}; };
+    PairPlan pp = plan_pairs(n_pairs, src_cloud, tgt_cloud, source_set, sizes(h->src), sizes(h->tgt), h->comm != nullptr);
+    if (pp.error) return fail("gicpSetPairList refused: %s", pp.error);
+    PairList& pl = h->pairs;
+    pl.on = false;   // until the new list is in place: a CUDA failure below leaves the handle one-to-one
+    CloudSet& from = source_set == GICP_TARGET ? h->tgt : h->src;
+    const size_t n = (size_t)std::max<int64_t>(pp.view.n_total, 1);
+    CU(pl.list.ensure((size_t)n_pairs * 3 * sizeof(int)));
+    CU(pl.src_meta.ensure((size_t)n_pairs * sizeof(CloudMeta)));
+    CU(pl.tgt_meta.ensure((size_t)n_pairs * sizeof(CloudMeta)));
+    CU(pl.tgt_bbox.ensure((size_t)n_pairs * 6 * sizeof(double)));
+    CU(pl.spts.ensure(n * sizeof(PRec<Real>)));
+    CU(pl.cov.ensure(n * ns_of(D) * sizeof(Real)));
+    pl.h_list.resize((size_t)n_pairs * 3);
+    for (int p = 0; p < n_pairs; ++p) {
+        pl.h_list[3 * p] = src_cloud[p];
+        pl.h_list[3 * p + 1] = tgt_cloud[p];
+        pl.h_list[3 * p + 2] = (int)pp.offsets[p];
+    }
+    CU(cudaMemcpyAsync(pl.list.p, pl.h_list.data(), pl.h_list.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+    // a target set's covariances are those of a target (I, or the estimated ones under covariance_model 1 / 2); a
+    // source set up as such has C = 0 there
+    const bool zero_cov = source_set == GICP_TARGET && h->prm.covariance_model != GICP_PLANE_TO_PLANE;
+    PairGatherArgs<Real> a{pl.list.as<int>(), from.nng().meta.as<CloudMeta>(), from.nng().spts.as<PRec<Real>>(),
+                           zero_cov ? nullptr : from.covnn().as<Real>(), h->tgt.nng().meta.as<CloudMeta>(),
+                           h->tgt.knn.bbox.as<double>(), pl.src_meta.as<CloudMeta>(), pl.tgt_meta.as<CloudMeta>(),
+                           pl.tgt_bbox.as<double>(), pl.spts.as<PRec<Real>>(), pl.cov.as<Real>()};
+    const int bx = std::max(1, (pp.view.max_n + PAIR_GATHER_ROWS - 1) / PAIR_GATHER_ROWS);
+    pair_gather_kernel<D, Real><<<dim3(bx, n_pairs), PAIR_GATHER_THREADS, 0, st>>>(a);
+    h->launches += 1;
+    CU(cudaGetLastError());
+    h->last_stream = st;
+    pl.view = pp.view;
+    pl.on = true;
+    if (h_pair_offsets) std::copy(pp.offsets.begin(), pp.offsets.end(), h_pair_offsets);
     return 0;
 }
 
@@ -1178,6 +1262,7 @@ int gicpDestroy(gicpHandle h) {
     if (h->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(h->comm);
     h->src.release();
     h->tgt.release();
+    h->pairs.release();
     for (SetupScratch& sc : h->scr) sc.release();
     h->vox.release();
     DevBuf* bufs[] = {&h->state, &h->partial, &h->partial2, &h->red, &h->T_dev, &h->n_active, &h->prev_match, &h->slack,
@@ -1211,6 +1296,7 @@ int gicpSetParams(gicpHandle h, const gicpParams* p) {
     if (h->prm.inner_max_iterations <= 0) h->prm.inner_max_iterations = 50;
     h->src.ready = false;
     h->tgt.ready = false;
+    h->pairs.on = false;
     return 0;
 }
 
@@ -1291,8 +1377,16 @@ int gicpPromoteTargetToSource(gicpHandle h) {
     if (!h->tgt.ready) return fail("no target to promote");
     std::swap(h->src, h->tgt);   // both sides own the same kind of state (two grids + covariances)
     h->tgt.ready = false;
+    h->pairs.on = false;
     if (h->prm.covariance_model != GICP_PLANE_TO_PLANE) return DISPATCH(h, zero_source_cov, h, h->last_stream);
     return 0;
+}
+
+int gicpSetPairList(gicpHandle h, int32_t n_pairs, const int32_t* h_source_cloud, const int32_t* h_target_cloud,
+                    int source_set, int64_t* h_pair_offsets, void* stream) {
+    if (check(h)) return 1;
+    return DISPATCH(h, set_pair_list, h, n_pairs, h_source_cloud, h_target_cloud, source_set, h_pair_offsets,
+                    (cudaStream_t)stream);
 }
 
 int gicpRegister(gicpHandle h, const double* h_T0, double* d_T, int32_t* d_n_outer, int32_t* d_converged,
@@ -1331,9 +1425,10 @@ int gicpNormalEquations(gicpHandle h, const double* h_T, double* h_out, void* st
 int gicpRobustScales(gicpHandle h, const double* h_T, double* h_scale, void* stream) {
     if (check(h)) return 1;
     if (!h_T || !h_scale) return fail("h_T and h_scale are required");
-    if (!h->src.ready || !h->tgt.ready) return fail("set source and target first");
+    const LoopView lv = loop_view(h);
+    if (!lv.ready) return fail("set source and target first");
     if (!h->robust_adaptive) {   // a fixed scale, or 0 without a kernel: nothing to compute
-        for (int p = 0; p < h->src.plan.n_clouds; ++p) h_scale[p] = h->robust_scale;
+        for (int p = 0; p < lv.plan.n_clouds; ++p) h_scale[p] = h->robust_scale;
         return 0;
     }
     return DISPATCH(h, do_stage, h, read_switches(), h_T, (int*)nullptr, (double*)nullptr, (double*)nullptr,
@@ -1399,6 +1494,7 @@ int gicpCommInit(gicpHandle h, int32_t n_ranks, int32_t rank, const char id[128]
     h->n_ranks = n_ranks;
     h->rank = rank;
     h->src.ready = h->tgt.ready = false;
+    h->pairs.on = false;
     return 0;
 }
 

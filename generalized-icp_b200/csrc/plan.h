@@ -8,6 +8,7 @@
 #include <climits>
 #include <cstdint>
 #include <cstdlib>
+#include <vector>
 
 #include "../../include/gicp_b200.h"
 #include "grid.cuh"
@@ -250,6 +251,68 @@ inline LoopPlan plan_loop(const Switches& sw, const SetupPlan& src, bool sliced,
     p.active_list = !p.sharded && np >= 64 && sw.active_list;
     // with a communicator every rank must issue the same all-reduces: a blocking poll on a fixed schedule
     p.poll_every = p.sharded ? 2 : 1;
+    return p;
+}
+
+// A set-up side as gicpSetPairList sees it: its host offsets (n_clouds + 1), or off = nullptr when it is not set up
+struct SetSizes {
+    const int64_t* off = nullptr;
+    int n_clouds = 0;
+};
+
+struct PairPlan {
+    const char* error = nullptr;   // why the list is refused; nothing below is valid then
+    std::vector<int64_t> offsets;  // n_pairs + 1: pair p's rows of the pair-ordered sources and per-point outputs
+    SetupPlan view;                // what plan_loop takes: n_clouds = n_pairs, max_n and n_total over the pairs' sources
+};
+
+// gicpSetPairList: pair p registers cloud src_cloud[p] of the set `source_set` names (the source set, or the target
+// set itself) onto cloud tgt_cloud[p] of the target set.  The view is the source plan of the one-to-one batch whose
+// p-th source is that cloud: plan_loop then makes every choice of the loop (ppt, blocks per pair, fused, active list,
+// presum) exactly as for that batch.
+inline PairPlan plan_pairs(int n_pairs, const int32_t* src_cloud, const int32_t* tgt_cloud, int source_set,
+                           const SetSizes& source, const SetSizes& target, bool comm) {
+    PairPlan p;
+    if (comm) {
+        p.error = "a handle with a communicator (gicpCommInit) registers one-to-one only";
+        return p;
+    }
+    if (n_pairs < 1 || n_pairs > 65535) {
+        p.error = "n_pairs must be in [1, 65535]";
+        return p;
+    }
+    if (source_set != GICP_SOURCE && source_set != GICP_TARGET) {
+        p.error = "source_set must be GICP_SOURCE 0 or GICP_TARGET 1";
+        return p;
+    }
+    const SetSizes& from = source_set == GICP_TARGET ? target : source;
+    if (!target.off || !from.off) {
+        p.error = source_set == GICP_TARGET ? "set the target first" : "set source and target first";
+        return p;
+    }
+    if (!src_cloud || !tgt_cloud) {
+        p.error = "null cloud index array";
+        return p;
+    }
+    p.offsets.assign(n_pairs + 1, 0);
+    int max_n = 0;
+    for (int i = 0; i < n_pairs; ++i) {
+        const int s = src_cloud[i], t = tgt_cloud[i];
+        if (s < 0 || s >= from.n_clouds || t < 0 || t >= target.n_clouds) {
+            p.error = "a cloud index is out of range";
+            return p;
+        }
+        const int64_t n = from.off[s + 1] - from.off[s];
+        p.offsets[i + 1] = p.offsets[i] + n;
+        if (p.offsets[i + 1] >= (1LL << 31) - 1024) {
+            p.error = "more than 2^31 points over the pairs' sources";
+            return p;
+        }
+        max_n = std::max<int>(max_n, (int)n);
+    }
+    p.view.n_clouds = n_pairs;
+    p.view.max_n = max_n;
+    p.view.n_total = p.offsets[n_pairs];
     return p;
 }
 

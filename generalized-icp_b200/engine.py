@@ -65,6 +65,7 @@ class GicpEngine:
         _lib.check(self.lib.gicpDefaultParams(C.byref(self.params)))
         self._keep = {}
         self._n = {SOURCE: (0, 0), TARGET: (0, 0)}
+        self._pairs = None   # set_pair_list: (source rows over the pairs, n_pairs); None = cloud i against cloud i
 
     def close(self):
         if getattr(self, "_h", None) is not None and self._h.value:
@@ -88,6 +89,7 @@ class GicpEngine:
             setattr(p, k, v)
         _lib.check(self.lib.gicpSetParams(self._h, C.byref(p)))
         self.params = p
+        self._pairs = None
 
     def set_robust_kernel(self, kind, scale=None, *, adaptive=None, min_scale=None):
         """Weight every gated-in correspondence by a robust kernel of its distance d (IRLS, weights frozen at T_k):
@@ -117,11 +119,15 @@ class GicpEngine:
     def robust_scales(self, T):
         """(P,) float64 numpy: every pair's robust scale at the transforms T (P, d+1, d+1) - the adaptive scale at the
         correspondences of T, a fixed scale as set, 0 without a kernel."""
-        n_pairs = self._n[SOURCE][1]
+        n_pairs = self._loop_n()[1]
         T, tp = self._T_arg(T)
         out = np.zeros((n_pairs,), dtype=np.float64)
         _lib.check(self.lib.gicpRobustScales(self._h, tp, out.ctypes.data_as(C.POINTER(C.c_double)), self._stream()))
         return out
+
+    def _loop_n(self):
+        """(source rows, pairs) of what register and the stage entry points run over: the pair list or the sides."""
+        return self._pairs if self._pairs is not None else self._n[SOURCE]
 
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
@@ -143,6 +149,7 @@ class GicpEngine:
         points, off = self._prep(points, offsets)
         self._keep[which] = points  # the library reads the caller's array later (covariance stage)
         self._n[which] = (points.shape[0], len(off) - 1)
+        self._pairs = None
         fn = self.lib.gicpSetTarget if which == TARGET else self.lib.gicpSetSource
         _lib.check(fn(self._h, _ptr(points), off.ctypes.data_as(C.POINTER(C.c_int64)), len(off) - 1, self._stream()))
 
@@ -163,6 +170,7 @@ class GicpEngine:
             raise ValueError("source and target need the same number of clouds")
         self._keep[TARGET], self._keep[SOURCE] = tp, sp
         self._n[TARGET], self._n[SOURCE] = (tp.shape[0], len(toff) - 1), (sp.shape[0], len(soff) - 1)
+        self._pairs = None
         i64p = C.POINTER(C.c_int64)
         _lib.check(self.lib.gicpSetPair(self._h, _ptr(tp), toff.ctypes.data_as(i64p), _ptr(sp), soff.ctypes.data_as(i64p),
                                         len(toff) - 1, self._stream()))
@@ -174,10 +182,41 @@ class GicpEngine:
         self._keep[SOURCE] = self._keep.pop(TARGET, None)
         self._n[SOURCE] = self._n[TARGET]
         self._n[TARGET] = (0, 0)
+        self._pairs = None
+
+    def set_pair_list(self, source_cloud, target_cloud, source_set=SOURCE):
+        """Register a list of pairs over the set-up clouds (gicpSetPairList; semantics in include/gicp_b200.h): pair p
+        registers cloud ``source_cloud[p]`` of the source set (``source_set=SOURCE``) or of the target set itself
+        (``source_set=TARGET``: one set-up of N clouds serves every pair among them) onto cloud ``target_cloud[p]`` of
+        the target set.  Afterwards register, evaluate, correspond, normal_equations, robust_scales and
+        source_covariances_at work on the pairs, with pair p's per-point rows at [offsets[p], offsets[p+1]).  Returns
+        the offsets, (P+1,) int64 numpy.  Every later set-up of a side and set_params return the engine to cloud i
+        against cloud i; a refused list leaves the previous one."""
+        s = np.ascontiguousarray(np.asarray(source_cloud, dtype=np.int64).reshape(-1))
+        t = np.ascontiguousarray(np.asarray(target_cloud, dtype=np.int64).reshape(-1))
+        if s.shape != t.shape:
+            raise ValueError(f"source_cloud and target_cloud differ in length ({s.size} and {t.size})")
+        lim = np.iinfo(np.int32)
+        if s.size and (min(s.min(), t.min()) < lim.min or max(s.max(), t.max()) > lim.max):
+            raise ValueError("a cloud index is out of range")
+        s32, t32 = s.astype(np.int32), t.astype(np.int32)
+        off = np.zeros(s.size + 1, dtype=np.int64)
+        i32p = C.POINTER(C.c_int32)
+        try:
+            _lib.check(self.lib.gicpSetPairList(self._h, int(s.size), s32.ctypes.data_as(i32p),
+                                                t32.ctypes.data_as(i32p), int(source_set),
+                                                off.ctypes.data_as(C.POINTER(C.c_int64)), self._stream()))
+        except RuntimeError as e:
+            # a refusal keeps the previous list; any other failure leaves the handle one-to-one
+            if "gicpSetPairList refused" not in str(e):
+                self._pairs = None
+            raise
+        self._pairs = (int(off[-1]), int(s.size))
+        return off
 
     # ---- the loop ----
     def register(self, T0=None, history=True) -> RegistrationResult:
-        n_pairs = self._n[SOURCE][1]
+        n_pairs = self._loop_n()[1]
         d1 = self.dim + 1
         mi = int(self.params.max_iterations)
         dev = self.device
@@ -200,7 +239,7 @@ class GicpEngine:
         RMSE, loss, information matrix H and vector b, as device tensors.  Stream-ordered, no synchronisation: a
         contiguous float64 T on the engine's device (e.g. ``register().T``) is read in place, anything else is copied
         there first."""
-        n_pairs = self._n[SOURCE][1]
+        n_pairs = self._loop_n()[1]
         d1, npar = self.dim + 1, 6 if self.dim == 3 else 3
         if not (isinstance(T, torch.Tensor) and T.device == self.device and T.dtype == torch.float64
                 and T.is_contiguous()):
@@ -246,6 +285,7 @@ class GicpEngine:
         base, row_bytes = self._pp_dev.data_ptr(), d * self._pp_dev.element_size()
         self._keep[TARGET] = self._keep[SOURCE] = self._pp_dev
         self._n[TARGET], self._n[SOURCE] = (n_t, 1), (n_s, 1)
+        self._pairs = None
         _lib.check(self.lib.gicpSetPair(self._h, vp(base + pad_s * row_bytes), (C.c_int64 * 2)(0, n_t), vp(base),
                                         (C.c_int64 * 2)(0, n_s), 1, st))
         # outputs: [T | loss_hist | T_hist | src_cov | tgt_cov] (f64) followed by [n_outer | converged | inliers] (i32)
@@ -311,6 +351,7 @@ class GicpEngine:
             self.promote_target_to_source()
         self._keep[TARGET] = self._sc_dev[slot]
         self._n[TARGET] = (n, 1)
+        self._pairs = None
         _lib.check(self.lib.gicpSetTarget(self._h, vp(self._sc_dev[slot].data_ptr()), (C.c_int64 * 2)(0, n), 1, st))
         if not have_previous:
             return None
@@ -431,6 +472,7 @@ class GicpEngine:
         m = int(out_off[-1])
         self._keep[which] = out     # the side's point array: the library reads it in every later call
         self._n[which] = (m, nc)
+        self._pairs = None
         return out[:m], out_off
 
     def set_target_voxelized(self, points, offsets=None, *, voxel_size, min_points=1):
@@ -466,13 +508,13 @@ class GicpEngine:
         return out
 
     def _T_arg(self, T, lead=()):
-        n_pairs = self._n[SOURCE][1]
+        n_pairs = self._loop_n()[1]
         d1 = self.dim + 1
         T = np.ascontiguousarray(np.asarray(T, dtype=np.float64).reshape(*lead, n_pairs, d1, d1))
         return T, T.ctypes.data_as(C.POINTER(C.c_double))
 
     def correspond(self, T, with_W=True):
-        n = self._n[SOURCE][0]
+        n = self._loop_n()[0]
         T, tp = self._T_arg(T)
         idx = torch.empty((n,), dtype=torch.int32, device=self.device)
         dist = torch.empty((n,), dtype=torch.float64, device=self.device)
@@ -481,7 +523,7 @@ class GicpEngine:
         return idx, dist, W
 
     def normal_equations(self, T):
-        n_pairs = self._n[SOURCE][1]
+        n_pairs = self._loop_n()[1]
         T, tp = self._T_arg(T)
         nred = 80 if self.dim == 3 else 32
         out = np.zeros((n_pairs, nred), dtype=np.float64)
@@ -492,7 +534,7 @@ class GicpEngine:
         Ts = np.asarray(Ts, dtype=np.float64)
         n_T = Ts.shape[0]
         T, tp = self._T_arg(Ts, lead=(n_T,))
-        n = self._n[SOURCE][0]
+        n = self._loop_n()[0]
         out = torch.empty((n_T, n, self.dim, self.dim), dtype=torch.float64, device=self.device)
         _lib.check(self.lib.gicpSourceCovariancesAt(self._h, tp, n_T, _ptr(out), self._stream()))
         return out
@@ -506,6 +548,7 @@ class GicpEngine:
 
     def comm_init(self, n_ranks, rank, unique_id: bytes):
         _lib.check(self.lib.gicpCommInit(self._h, n_ranks, rank, C.create_string_buffer(unique_id, 128)))
+        self._pairs = None
 
     def comm_destroy(self):
         _lib.check(self.lib.gicpCommDestroy(self._h))

@@ -68,6 +68,44 @@ CONFIG5 = dict(n=16_777_216, n_patches=1024, cube=400.0, patch=30.0, sigma=0.02,
 CONFIG5_PARAMS = dict(k=20, max_distance_nearest_neighbors=1.8, max_distance_correspondence=2.5, tolerance=1e-6)
 
 
+def patches3d_sequence(n_clouds, n=32_768, n_patches=16, cube=40.0, patch=30.0, sigma=0.02, max_rot_deg=2.0,
+                       max_trans=0.5, seed=0):
+    """A scan sequence of one planar-patch scene: ``n_clouds`` clouds of ``n`` points, each drawn independently from
+    the same patches (config-4 density and noise by default) and expressed in the frame of its own pose.  The poses
+    are a random walk: pose k is pose k-1 followed by a rotation of up to ``max_rot_deg`` about the cube centre and a
+    translation of up to ``max_trans``.  Returns ``(clouds, poses)``: a list of float32 (n, 3) arrays and (n_clouds,
+    4, 4) float64 poses mapping each cloud's frame to the scene's, so cloud i registers onto cloud j under
+    :func:`relative_pose` ``(poses, i, j)``."""
+    rng = np.random.default_rng(seed)
+    centres = rng.uniform(0.25 * cube, 0.75 * cube, size=(n_patches, 3))
+    frames = np.stack([np.linalg.qr(rng.normal(size=(3, 3)))[0] for _ in range(n_patches)])
+    c = np.full(3, cube / 2)
+    poses = np.empty((n_clouds, 4, 4))
+    pose = np.eye(4)
+    clouds = []
+    for k in range(n_clouds):
+        if k:
+            step = np.eye(4)
+            R = _rand_rotation(rng, max_rot_deg)
+            tdir = rng.normal(size=3)
+            step[:3, :3] = R
+            step[:3, 3] = c - R @ c + tdir / np.linalg.norm(tdir) * rng.uniform(0, max_trans)
+            pose = pose @ step
+        poses[k] = pose
+        which = rng.integers(0, n_patches, size=n)
+        ab = rng.uniform(-patch / 2, patch / 2, size=(n, 2))
+        p = centres[which] + ab[:, :1] * frames[which, :, 0] + ab[:, 1:] * frames[which, :, 1]
+        p += rng.normal(0, sigma, size=(n, 3))
+        inv = np.linalg.inv(pose)                      # scene -> cloud k's frame
+        clouds.append((p @ inv[:3, :3].T + inv[:3, 3]).astype(np.float32))
+    return clouds, poses
+
+
+def relative_pose(poses, i, j):
+    """The transform that maps cloud i of :func:`patches3d_sequence` onto cloud j: inv(pose_j) @ pose_i."""
+    return np.linalg.inv(poses[j]) @ poses[i]
+
+
 def patches3d_batch_device(n_pairs, n=32_768, n_patches=16, cube=40.0, patch=30.0, sigma=0.02,
                            max_rot_deg=2.0, max_trans=0.5, seed=0, device="cuda", chunk=256, first_pair=0):
     """Config-4 batch generated in HBM: (src, tgt) float32 (n_pairs*n, 3), CSR

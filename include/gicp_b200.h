@@ -24,7 +24,7 @@
  *  - clouds come as BATCHES: `n_clouds` clouds concatenated into one (n_total,
  *    dim) row-major array, with h_offsets[n_clouds+1] giving each cloud's row
  *    range.  A single pair is a batch of one.  Source cloud i is registered
- *    against target cloud i.
+ *    against target cloud i, unless a pair list is set (gicpSetPairList).
  *  - point indices reported by the library are cloud-local (0-based row within
  *    the cloud), -1 meaning "none".
  */
@@ -136,6 +136,53 @@ int gicpSetPair(gicpHandle h, const void* d_target_points, const int64_t* h_targ
  * being rebuilt (the reference recomputes both on every call, gicp.py:104,111).  After this call
  * the handle's source is the former target; set a new target with gicpSetTarget.             */
 int gicpPromoteTargetToSource(gicpHandle h);
+
+/* ---- pairs over set-up clouds (multi-frame odometry, loop-closure candidates, the edges of a pose graph) ---------
+ * Pair p registers cloud h_source_cloud[p] of the source set onto cloud h_target_cloud[p] of the target set.
+ * source_set = GICP_SOURCE: the source indices refer to the handle's source set (gicpSetSource / gicpSetPair /
+ * gicpSetVoxelized(GICP_SOURCE)); source_set = GICP_TARGET: they refer to the TARGET set, so one set-up of N clouds
+ * serves every pair among them and no source set-up is needed.  h_pair_offsets (n_pairs+1, host, may be NULL)
+ * receives the row range of every pair in the per-source-point outputs.
+ *  - After the call every pair-indexed entry point works on the n_pairs pairs instead of cloud i against cloud i:
+ *    gicpRegister, gicpCorrespond, gicpNormalEquations, gicpRobustScales, gicpEvaluate and gicpSourceCovariancesAt.
+ *    Their n_clouds becomes n_pairs: h_T0, d_T, the histories, the quality rows, H and b are per pair.  The
+ *    per-source-point outputs (d_idx, d_dist, d_W, d_out) are laid out pair after pair: pair p holds rows
+ *    [h_pair_offsets[p], h_pair_offsets[p+1]), in its source cloud's input order.
+ *  - Pair p gives exactly what a one-to-one batch gives whose p-th source is that source cloud and p-th target that
+ *    target cloud, bit for bit, whenever every set-up involved (the list's sets and the batch's two sides) makes the
+ *    same two set-up choices, which depend on the whole set, not on the cloud alone:
+ *      - the same cells per cloud: always with max_cells_per_cloud set; with the automatic budget when the largest
+ *        cloud of every set-up rounds up to the same power of two and budget x clouds stays within 2^30 (the budget
+ *        can enlarge a cloud's cell edge, and with it the grid order);
+ *      - the same k-NN estimator of the covariances: a set-up whose largest cloud has <= 2048 points and whose total
+ *        is <= 65536 points takes the latency path (the mean first, then centred sums over the sorted k nearest);
+ *        any other set-up with k <= 24 (float32 storage) or k <= 13 (float64) takes the histogram kernel (moments
+ *        about the query point, in candidate order).  The two round differently.  So a list over 100 scans of 360
+ *        points (36000 points, latency path) is bitwise equal to one-to-one batches of at most 65536 points per side,
+ *        not to one batch of all its pairs (the histogram path).
+ *    Otherwise the covariances or the grid order differ in the last bits and the results agree to the tolerances the
+ *    loop is held to.  Sides whose covariances no k-NN search estimates (covariance_model 1 / 2 sources, model 1
+ *    targets, voxelized sides) do not depend on the second choice.
+ *  - With source_set = GICP_TARGET and covariance_model 1 or 2 the sources' covariances are 0, as a source set-up
+ *    gives them (a target set-up holds I or the estimated ones).
+ *  - Self-pairs, repeated pairs, (i, j) together with (j, i) and pairs with empty clouds are allowed.
+ *  - gicpKnn and gicpCovariances stay per side and are unaffected.
+ *  - The sources are copied into pair order once, by this call (sum over the pairs' sources of 40 B per point in
+ *    float32 3-D, 80 B in float64), so later calls read neither the source set's arrays nor the caller's.
+ *  - The list is discarded, and the handle returns to one-to-one, by every call that sets up or unsets a side
+ *    (gicpSetSource, gicpSetTarget, gicpSetPair, gicpSetVoxelized once its input is accepted,
+ *    gicpPromoteTargetToSource), by a successful gicpSetParams and by gicpCommInit.  gicpSetRobustKernel and
+ *    gicpSetRobustKernelAdaptive keep it, as they keep the clouds.
+ *  - Fails, leaving the handle as it was (its previous list or none), on n_pairs outside [1, 65535], an index out of
+ *    range, a source_set other than the two above, the referenced set not being set up (both sides for GICP_SOURCE,
+ *    the target for GICP_TARGET), >= 2^31 - 1024 points summed over the pairs' sources, or a handle with a
+ *    communicator (gicpCommInit).  These refusals' messages begin "gicpSetPairList refused".  Any other failure (a
+ *    CUDA error while the list is gathered) leaves the handle one-to-one.
+ * Stream-ordered, no synchronisation: the offsets come from the host-side cloud sizes.
+ * gicpVersion() stays 106 with this entry point (a test of the 106 interface pins that value); a caller detects pair
+ * lists by the exported symbol gicpSetPairList.                             */
+int gicpSetPairList(gicpHandle h, int32_t n_pairs, const int32_t* h_source_cloud, const int32_t* h_target_cloud,
+                    int source_set, int64_t* h_pair_offsets, void* stream);
 
 /* ---- the registration loop (replaces gicp.py:107-174) ------------------------------------
  * Runs all pairs to convergence / max_iterations on the device.
